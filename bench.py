@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W              # our B200 path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (oracle port)
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also save what the last timed step computed
 
 Workload (BASELINE.json configs[1]): one data-parallel training step of NCameraCNN on a synthetic 2-view batch of
 256 image pairs per GPU at 256x256 — uint8 images -> GPU augmentation -> forward (bf16, fp32 accumulate) ->
@@ -32,6 +33,8 @@ FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustain
 # pairs per CPU step in BOTH CPU legs (`cpu_baseline` of our line and `--impl reference`): the largest sample of the
 # 256-pair workload that keeps `--steps 20 --warmup 5` within a few minutes on the box's host cores (~8 pairs/s)
 CPU_SAMPLE_PAIRS = 32
+# --dump-outputs keeps this many positions of each 25.9 M-element arena (parameters, gradients): 16 MiB apiece in fp32
+DUMP_SAMPLE = 1 << 22
 
 
 def load_peaks():
@@ -109,6 +112,25 @@ def synthetic_batch(B: int, n_cams: int, H: int, W: int, seed: int):
     q = torch.randn(B, 4, generator=g)
     targets = torch.cat([torch.randn(B, 3, generator=g), q / q.norm(dim=-1, keepdim=True)], -1)
     return images, targets
+
+
+def dump_step_outputs(directory: str, model, engine, loss) -> None:
+    """Saves what the last training step handed its caller, as float32 .npy files: the mean loss it returned, the
+    gradient norm before clipping, and the state the next step starts from (the updated parameters and the batch-norm
+    running statistics) together with the gradients of the step. Parameters and gradients are the same fixed, seeded
+    sample of DUMP_SAMPLE positions, so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+
+    params = model.flat_params
+    idx = torch.randperm(params.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    idx = idx.to(params.device)
+    arrays = {"loss": loss.reshape(1), "grad_norm": engine.last_grad_norm.reshape(1), "params_sample": params[idx],
+              "grads_sample": model.flat_grads[idx], "bn_running_stats": model._flat_buffers}
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(out / f"{name}.npy", t.detach().float().cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -230,6 +252,8 @@ def run_ours(args) -> None:
     ms_total = float(t.item())
     value = world * B * args.steps / (ms_total / 1e3)
     final_loss = float(loss.item())
+    if args.dump_outputs and rank == 0:
+        dump_step_outputs(args.dump_outputs, model, engine, loss)   # before the passes below change the model
     if trace is not None and rank == 0:
         print("LOSS_TRACE " + " ".join(repr(float(x)) for x in trace), file=sys.stderr, flush=True)
         if os.environ.get("ARGUS_BENCH_TRACE") == "2":
@@ -695,7 +719,13 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-inference", action="store_true")
     ap.add_argument("--no-torch-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, about 34 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
