@@ -213,6 +213,14 @@ int argus_conv2d_wgrad(const void* dy, const void* x, float* dw, int N, int H, i
   ARGUS_API_END
 }
 
+int argus_stem_dgrad(const void* dy, const void* w, float* dx, int N, int H, int W, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  stem_dgrad(static_cast<const __nv_bfloat16*>(dy), static_cast<const __nv_bfloat16*>(w), dx, N, H, W,
+             static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
 int argus_bn_finalize(const float* partial, int slots, double count, const float* gamma, const float* beta,
                       float* running_mean, float* running_var, float momentum, float eps, float* scale, float* shift,
                       float* save_mean, float* save_invstd, int C, void* stream) {
@@ -553,6 +561,13 @@ int argus_model_backward(argus_model* m, const float* d_out, int stage_begin, in
   ARGUS_CHECK(m != nullptr, "null model");
   ARGUS_CHECK(0 <= stage_begin && stage_begin <= stage_end && stage_end <= 4, "bad stage range");
   m->impl.backward(d_out, stage_begin, stage_end, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+int argus_model_input_grad(argus_model* m, float* dx, void* stream) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(m != nullptr, "null model");
+  ARGUS_CHECK(dx != nullptr, "null gradient buffer");
+  m->impl.input_grad(dx, static_cast<cudaStream_t>(stream));
   ARGUS_API_END
 }
 int argus_model_stage_range(argus_model* m, int stage, int64_t* begin, int64_t* end) {

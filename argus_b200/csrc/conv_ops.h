@@ -96,6 +96,10 @@ WgradLaunch plan_conv_wgrad_gram(const ConvShape& s, const __nv_bfloat16* dy, co
 // stride 2): the Gram matrix from which the batch statistics of the convolution's OUTPUT follow without computing it.
 WgradLaunch plan_gram(const ConvShape& s, const __nv_bfloat16* x, float* g);
 
+// Input gradient of the stem (stem_dgrad.cu): dy (N, H/2, W/2, 64) bf16 NHWC, w the [64][256] packed stem weight of the
+// forward, dx (N, 3, H, W) fp32 NCHW, fully overwritten. H, W powers of two >= 32, W <= 1024. Deterministic.
+void stem_dgrad(const __nv_bfloat16* dy, const __nv_bfloat16* w, float* dx, int N, int H, int W, cudaStream_t stream);
+
 void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream);
 int choose_epilogue_groups(const ConvGemmParams& p, int block_n);
 // number of statistic slots launch_conv writes for this launch (one per epilogue group per CTA)

@@ -225,6 +225,17 @@ __global__ void nchw_to_nhwc3_kernel(const float* __restrict__ x, float* __restr
     y[i] = x[(n * 3 + c) * HW + pix];
   }
 }
+// inverse of nchw_to_nhwc3_kernel: the input gradient (n, H, W, 3) NHWC -> (n, 3, H, W) NCHW
+__global__ void nhwc3_to_nchw_kernel(const float* __restrict__ x, float* __restrict__ y, int n_images, int HW) {
+  pdl_prologue();
+  const int64_t total = static_cast<int64_t>(n_images) * HW * 3;
+  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int64_t pix = i % HW;
+    const int64_t t = i / HW;   // n * 3 + c
+    y[i] = x[((t / 3) * HW + pix) * 3 + t % 3];
+  }
+}
 __global__ void u8_to_f32_kernel(const uint8_t* __restrict__ x, float* __restrict__ y, int64_t n) {
   pdl_prologue();
   for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
@@ -235,6 +246,12 @@ void pack_input_nhwc_f32(const float* x_nchw, float* y_nhwc, int n_images, int H
   const int64_t total = static_cast<int64_t>(n_images) * H * W * 3;
   launch_kernel(nchw_to_nhwc3_kernel, static_cast<int>(std::min<int64_t>((total + 255) / 256, 8192)), 256, 0, s, x_nchw, y_nhwc,
                                                                                                       n_images, H * W);
+  ARGUS_CUDA(cudaGetLastError());
+}
+void unpack_input_grad_nhwc_f32(const float* dx_nhwc, float* dx_nchw, int n_images, int H, int W, cudaStream_t s) {
+  const int64_t total = static_cast<int64_t>(n_images) * H * W * 3;
+  launch_kernel(nhwc3_to_nchw_kernel, static_cast<int>(std::min<int64_t>((total + 255) / 256, 8192)), 256, 0, s, dx_nhwc,
+                dx_nchw, n_images, H * W);
   ARGUS_CUDA(cudaGetLastError());
 }
 void pack_input_u8_f32(const uint8_t* x_hwc, float* y_nhwc, int n_images, int H, int W, cudaStream_t s) {

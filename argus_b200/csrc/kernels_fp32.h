@@ -38,6 +38,8 @@ void conv_f32_wgrad(const ConvShapeF32& s, const float* dy, const float* x, floa
 // (B, 3*n_cams, H, W) NCHW == (B*n_cams, 3, H, W) -> NHWC; u8 HWC images -> fp32 / 255
 void pack_input_nhwc_f32(const float* x_nchw, float* y_nhwc, int n_images, int H, int W, cudaStream_t s);
 void pack_input_u8_f32(const uint8_t* x_hwc, float* y_nhwc, int n_images, int H, int W, cudaStream_t s);
+// the inverse of pack_input_nhwc_f32, for the input gradient: (n, H, W, 3) NHWC -> (B, 3*n_cams, H, W) NCHW
+void unpack_input_grad_nhwc_f32(const float* dx_nhwc, float* dx_nchw, int n_images, int H, int W, cudaStream_t s);
 
 constexpr int kBnF32MaxBlocks = 1024;   // scratch: kBnF32MaxBlocks * 2 * C doubles
 // batch statistics (fp64 sums) -> scale/shift/mean/invstd + running-stat update (torch.nn.BatchNorm2d semantics)

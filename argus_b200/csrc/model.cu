@@ -58,6 +58,7 @@ void Model::set_precision(int mode) {
   ARGUS_CHECK(mode == 0 || mode == 1, "precision mode must be 0 (bf16 tensor cores) or 1 (fp32)");
   precision_ = mode;
   last_train_plan_ = nullptr;
+  stem_grad_ready_ = false;
   last_plan_ = nullptr;
   staged_plan_ = nullptr;
   eval_fold_dirty_ = true;
@@ -645,6 +646,8 @@ void Model::forward(const void* x, bool is_u8, int B, int H, int W, bool trainin
   ARGUS_CHECK(B > 0, "empty batch");
   ARGUS_CHECK(!training || B * n_cams_ * (H / 32) * (W / 32) > 1,
               "train-mode batch norm needs more than one value per channel");
+  stem_grad_ready_ = false;
+  if (training) train_input_f32_ = (x != nullptr && !is_u8);
   if (precision_ == 1) {
     forward_fp32(x, is_u8, B, H, W, training, out, s);
     return;
@@ -974,6 +977,7 @@ void Model::backward(const float* d_out, int stage_begin, int stage_end, cudaStr
                               grads_dev_ + stem_.bn.beta_off, p.g_raw0, N, p.H / 2, p.W / 2, 64, bn_bwd_scratch_, s);
       }
       run_wgrad(p.stem.wgrad, s);
+      stem_grad_ready_ = true;   // p.g_raw0 now holds d loss / d (stem convolution output) for input_grad()
     }
     join_wgrad(s);
     // packed 3x3 / stem gradients of this stage -> PyTorch layout in the gradient arena
@@ -987,6 +991,23 @@ void Model::backward(const float* d_out, int stage_begin, int stage_end, cudaStr
       if (lo >= 0) unpack_wgrads(gpacked_, grads_dev_, pack_table_dev_ + lo, hi - lo, s);
     }
   }
+}
+
+void Model::check_input_grad_ready(bool have_train_forward) const {
+  ARGUS_CHECK(have_train_forward, "input_grad() needs a preceding training forward()");
+  ARGUS_CHECK(train_input_f32_, "the last training forward consumed a staged / uint8 input, which has no input gradient");
+  ARGUS_CHECK(stem_grad_ready_, "input_grad() needs backward() stage 3 to have run since the last forward()");
+}
+
+void Model::input_grad(float* dx, cudaStream_t s) {
+  if (precision_ == 1) {
+    input_grad_fp32(dx, s);
+    return;
+  }
+  check_input_grad_ready(last_train_plan_ != nullptr);
+  const Plan& p = *last_train_plan_;
+  // the forward rounded x to bf16 (pack_input_f32); its gradient passes straight through that rounding
+  stem_dgrad(p.g_raw0, packed_ + stem_.packed_off, dx, p.N, p.H, p.W, s);
 }
 
 }  // namespace argus

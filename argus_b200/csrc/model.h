@@ -140,6 +140,9 @@ class Model {
   // gradient arena for stages [stage_begin, stage_end); stages must be run in increasing order 0..3.
   void backward(const float* d_out, int stage_begin, int stage_end, cudaStream_t s);
   void zero_grads(cudaStream_t s);
+  // d loss / d x of the last training forward (whose input was the fp32 tensor x) once backward() has run stage 3:
+  // dx (B, 3*n_cams, H, W) fp32, overwritten. Throws without such a forward / backward, or for a staged / u8 input.
+  void input_grad(float* dx, cudaStream_t s);
   // overlap the weight-gradient GEMMs with the rest of the backward pass on a side stream (default on)
   void set_wgrad_overlap(bool on) { overlap_wgrad_ = on; }
   // Debug / test probe: copies an activation of the LAST forward (bf16 NHWC rows x C) into dst.
@@ -192,6 +195,8 @@ class Model {
   Fp32State& fp32_state(int B, int H, int W, bool training);
   void forward_fp32(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s);
   void backward_fp32(const float* d_out, int stage_begin, int stage_end, cudaStream_t s);
+  void input_grad_fp32(float* dx, cudaStream_t s);
+  void check_input_grad_ready(bool have_train_forward) const;
   int precision_ = 0;
   Fp32State* f32_ = nullptr;
 
@@ -245,6 +250,8 @@ class Model {
   Plan* last_plan_ = nullptr;
   uint64_t arena_epoch_ = 1;   // bumped whenever another plan (they share the arena) runs a forward pass
   Plan* staged_plan_ = nullptr;
+  bool train_input_f32_ = false;   // the last training forward read an fp32 image tensor (not u8 / a staged batch)
+  bool stem_grad_ready_ = false;   // backward() stage 3 ran after the last forward(): the stem's output gradient is live
   // stem input double buffer (see Plan): [n][H/2][W/2 + 4][16] bf16 each; cur_in_ = the buffer the last forward consumed
   bf16* stem_in_[2] = {nullptr, nullptr};
   size_t stem_in_elems_ = 0;

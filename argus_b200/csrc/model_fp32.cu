@@ -40,6 +40,8 @@ struct Fp32State {
   float *d_out = nullptr, *d_a2 = nullptr, *d_a1 = nullptr, *d_z0 = nullptr, *d_feat = nullptr, *d_pooled = nullptr;
   float* G[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
   float* cur_grad = nullptr;   // gradient wrt the current block output while walking backwards
+  float* stem_graw = nullptr;  // after backward stage 3: gradient wrt the stem convolution output (N, H/2, W/2, 64)
+  float* stem_gx = nullptr;    // a free gradient buffer of the same stage: the NHWC input gradient goes there
   float* wscratch = nullptr;
   double* bn_partial = nullptr;
   float* bn_sums = nullptr;
@@ -282,8 +284,19 @@ void Model::backward_fp32(const float* d_out, int stage_begin, int stage_end, cu
       maxpool_f32_bwd(Pg, st.idx0, others[0], N, H1, W1, 64, s);
       bn_bwd(stem_, others[0], st.stem.raw, st.stem.act, others[1], nullptr, static_cast<int64_t>(N) * H1 * W1);
       conv_bwd(stem_, others[1], st.x_nhwc, nullptr, N, st.H, st.W);
+      st.stem_graw = others[1];
+      st.stem_gx = others[0];
+      stem_grad_ready_ = true;
     }
   }
+}
+
+void Model::input_grad_fp32(float* dx, cudaStream_t s) {
+  check_input_grad_ready(f32_ != nullptr && f32_->have_train_forward);
+  Fp32State& st = *f32_;
+  // transposed stem convolution into NHWC (others[0] of stage 3 holds N*H*W*16 floats, more than the N*H*W*3 needed)
+  conv_f32_dgrad(shape_of(stem_, st.N, st.H, st.W), st.stem_graw, params_dev_ + stem_.w_off, st.stem_gx, s);
+  unpack_input_grad_nhwc_f32(st.stem_gx, dx, st.N, st.H, st.W, s);
 }
 
 }  // namespace argus

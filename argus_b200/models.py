@@ -7,6 +7,10 @@ Differences that are deliberate and documented in DESIGN.md:
   * the forward pass runs in bf16 with fp32 accumulation on the tensor cores and only exists on CUDA
     (no CPU fallback: calling the module with CPU tensors raises);
   * H and W must be powers of two >= 32 (the reference's default 256x256 and its 128x128 crop test both are).
+
+Gradients flow to the parameters and to the input images of a train-mode forward, as with the reference: with
+`x.requires_grad_()`, `loss.backward()` fills `x.grad` (the stem's transposed convolution runs on the tensor cores,
+argus_model_input_grad), also when every parameter is frozen. An eval-mode forward builds no graph.
 """
 from __future__ import annotations
 
@@ -89,7 +93,8 @@ class _ModelHandle:
 
 
 class _NCameraCNNFunction(torch.autograd.Function):
-    """Whole-network autograd node: forward = argus_model_forward, backward = argus_model_backward."""
+    """Whole-network autograd node: forward = argus_model_forward, backward = argus_model_backward (+
+    argus_model_input_grad when x requires grad)."""
 
     @staticmethod
     def forward(ctx, model: "NCameraCNN", x: torch.Tensor, *params: torch.Tensor) -> torch.Tensor:
@@ -98,6 +103,7 @@ class _NCameraCNNFunction(torch.autograd.Function):
         ctx.model = model
         ctx.is_train_forward = training
         ctx.n_params = len(params)
+        ctx.x_shape, ctx.x_dtype = x.shape, x.dtype
         return out
 
     @staticmethod
@@ -105,8 +111,9 @@ class _NCameraCNNFunction(torch.autograd.Function):
         model = ctx.model
         if not ctx.is_train_forward:
             raise RuntimeError("argus_b200: gradients are only available for a forward pass made in train() mode")
-        grads = model._backward_impl(grad_out)
-        return (None, None) + tuple(grads)
+        grads = model._backward_impl(grad_out, ctx.needs_input_grad[2:])
+        dx = model._input_grad_impl(ctx.x_shape).to(ctx.x_dtype) if ctx.needs_input_grad[1] else None
+        return (None, dx) + tuple(grads)
 
 
 class NCameraCNN(nn.Module):
@@ -345,13 +352,24 @@ class NCameraCNN(nn.Module):
         self._flat_nbt += 1
         return out
 
-    def _backward_impl(self, grad_out: torch.Tensor) -> list[torch.Tensor]:
+    def _backward_impl(self, grad_out: torch.Tensor, needs_grad=None) -> list[Optional[torch.Tensor]]:
+        """Parameter gradients of the last training forward; None for parameters whose `needs_grad` entry is False."""
         g = grad_out.contiguous().to(torch.float32)
         with torch.cuda.device(g.device):
             _lib.call("argus_model_zero_grads", self._handle.ptr, _lib.stream_ptr())
             _lib.call("argus_model_backward", self._handle.ptr, g, 0, 4, _lib.stream_ptr())
         fg = self._flat_grads
-        return [fg[off:off + numel].view(shape).clone() for (_n, off, numel, shape) in self._param_infos]
+        if needs_grad is None:
+            needs_grad = [True] * len(self._param_infos)
+        return [fg[off:off + numel].view(shape).clone() if need else None
+                for need, (_n, off, numel, shape) in zip(needs_grad, self._param_infos)]
+
+    def _input_grad_impl(self, shape) -> torch.Tensor:
+        """d loss / d x (fp32, `shape` = the input's) of the last training forward, after _backward_impl."""
+        dx = torch.empty(shape, dtype=torch.float32, device=self._flat_params.device)
+        with torch.cuda.device(dx.device):
+            _lib.call("argus_model_input_grad", self._handle.ptr, dx, _lib.stream_ptr())
+        return dx
 
     def probe_activation(self, index: int) -> torch.Tensor:
         """Test probe: activation of the last forward as a (rows, C) bf16 tensor (NHWC rows).
@@ -380,6 +398,6 @@ class NCameraCNN(nn.Module):
         """
         assert len(x.shape) == 4 or x.dtype == torch.uint8, \
             "The input images must be of shape (B, C, H, W)! If B=1, add a dummy dimension."
-        if torch.is_grad_enabled() and self.training and any(p.requires_grad for p in self._param_list):
+        if torch.is_grad_enabled() and self.training and (x.requires_grad or any(p.requires_grad for p in self._param_list)):
             return _NCameraCNNFunction.apply(self, x, *self._param_list)
         return self._forward_impl(x, self.training)

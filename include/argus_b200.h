@@ -81,6 +81,11 @@ int argus_conv_bn_backward_algebraic(const void* g, const void* act, const void*
 /* dw[Cout][k*k*Cin] (fp32) += dy^T * im2col(x); the caller zero-fills dw. */
 int argus_conv2d_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int k,
                        int stride, int kind, void* stream);
+/* Input gradient of the stem (resnet.conv1: 7x7, stride 2, pad 3, 3 -> 64; argus/models.py:84).
+ * dy: (N, H/2, W/2, 64) bf16 NHWC; w: the [64][256] packed bf16 stem weight the forward used ([64][p 4][q 4][16],
+ * the argus_conv2d_forward kind-1 layout); dx: (N, 3, H, W) fp32 NCHW, overwritten. H, W powers of two >= 32
+ * (W <= 1024). fp32 accumulation and output; deterministic. */
+int argus_stem_dgrad(const void* dy, const void* w, float* dx, int N, int H, int W, void* stream);
 
 /* ---- batch norm / pooling primitives (torch.nn.BatchNorm2d, ReLU, MaxPool2d(3,2,1), AdaptiveAvgPool2d(1) inside
  *      torchvision resnet50, argus/models.py:84). x, y, dy, dx, res, out: bf16 NHWC viewed as (rows, C); C/8 a
@@ -235,6 +240,11 @@ int argus_model_zero_grads(argus_model* m, void* stream);
 /* Backward of the last training forward. d_out (B,6). Stages 0..3 (head+fc+layer4, layer3, layer2, layer1+stem)
  * must run in order; gradients are ADDED into the bound gradient arena. */
 int argus_model_backward(argus_model* m, const float* d_out, int stage_begin, int stage_end, void* stream);
+/* d loss / d x for the last training forward whose input was the fp32 tensor x (B, 3*n_cams, H, W); call after
+ * argus_model_backward has run stage 3. dx: (B, 3*n_cams, H, W) fp32, overwritten. Image n = b*n_cams + v is channels
+ * [3v, 3v+3) of sample b; the gradient passes straight through the bf16 rounding of the input. Errors (non-zero status,
+ * message): no training forward, backward stage 3 not run since it, or the forward consumed a staged / uint8 input. */
+int argus_model_input_grad(argus_model* m, float* dx, void* stream);
 /* Element range of the parameter arena whose gradients are final once `stage` has run (all-reduce buckets). */
 int argus_model_stage_range(argus_model* m, int stage, int64_t* begin, int64_t* end);
 int argus_model_arena_bytes(argus_model* m, int64_t* bytes);
