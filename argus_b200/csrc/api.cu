@@ -9,6 +9,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <vector>
 
 using namespace argus;
 
@@ -139,6 +140,157 @@ int argus_conv2d_dgrad_ex(const void* dy, const void* w, void* dx, int N, int H,
   e.stat_partial = stat_partial;
   ARGUS_CHECK(stat_partial == nullptr || stat_slot_capacity >= stat_slots(l), "statistics buffer has too few slots");
   launch_conv(l, e, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
+int argus_conv2d_forward_full(const void* x, const void* w, void* y, int N, int H, int W, int Cin, int Cout, int k,
+                              int stride, int kind, const float* scale, const float* shift, const void* residual,
+                              const float* res_scale, const float* res_shift, int relu, void* relu_bits_out,
+                              float* stat_partial, int stat_slot_capacity, int early_trigger, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ConvShape s = make_shape(N, H, W, Cin, Cout, k, stride, kind);
+  ConvLaunch l = plan_conv_forward(s, static_cast<const bf16*>(x), static_cast<const bf16*>(w), static_cast<bf16*>(y));
+  Epilogue e;
+  e.scale = scale; e.shift = shift; e.residual = static_cast<const bf16*>(residual);
+  e.res_scale = res_scale; e.res_shift = res_shift;
+  e.relu = relu; e.relu_bits_out = static_cast<uint8_t*>(relu_bits_out);
+  e.stat_partial = stat_partial;
+  e.early_trigger = early_trigger;
+  ARGUS_CHECK(relu_bits_out == nullptr || relu != 0, "the ReLU bit mask needs the ReLU");
+  ARGUS_CHECK(res_scale == nullptr || residual != nullptr, "residual scale / shift need a residual");
+  ARGUS_CHECK(stat_partial == nullptr || stat_slot_capacity >= stat_slots(l), "statistics buffer has too few slots");
+  launch_conv(l, e, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
+static ConvLaunch plan_bnred_dgrad(const ConvShape& s, const void* dy, const void* w, void* dx, const void* concat_a,
+                                   int concat_channels) {
+  ARGUS_CHECK(s.stride == 1, "the fused BN reduction exists for stride-1 dgrads");
+  if (concat_a != nullptr)
+    return plan_dgrad_concat(s, static_cast<const bf16*>(dy), static_cast<const bf16*>(concat_a), concat_channels,
+                             static_cast<const bf16*>(w), static_cast<bf16*>(dx));
+  auto ls = plan_conv_dgrad(s, static_cast<const bf16*>(dy), static_cast<const bf16*>(w), static_cast<bf16*>(dx));
+  ARGUS_CHECK(ls.size() == 1, "unexpected dgrad decomposition");
+  return ls[0];
+}
+
+int argus_conv2d_dgrad_bnred(const void* dy, const void* w, void* dx, int N, int H, int W, int Cin, int Cout, int k,
+                             int stride, const void* concat_a, int concat_channels, const float* bias,
+                             const void* bn_raw, const float* bn_scale, const float* bn_shift, float* stat_partial,
+                             int stat_slot_capacity, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(bn_raw != nullptr && bn_scale != nullptr && bn_shift != nullptr && stat_partial != nullptr,
+              "null argument");
+  ConvShape s = make_shape(N, H, W, Cin, Cout, k, stride, 0);
+  ConvLaunch l = plan_bnred_dgrad(s, dy, w, dx, concat_a, concat_channels);
+  Epilogue e;
+  e.shift = bias;
+  e.bn_raw = static_cast<const bf16*>(bn_raw);
+  e.bn_scale = bn_scale;
+  e.bn_shift = bn_shift;
+  e.stat_partial = stat_partial;
+  ARGUS_CHECK(stat_slot_capacity >= stat_slots(l), "statistics buffer has too few slots");
+  launch_conv(l, e, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
+int argus_conv2d_launch_info(int launch, int N, int H, int W, int Cin, int Cout, int k, int stride, int kind,
+                             int concat_channels, int flags, int* out, int cap, int* n_launches) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(out != nullptr && n_launches != nullptr, "null argument");
+  ARGUS_CUDA(cudaFree(nullptr));   // tensor-map encoding needs a current context, which nothing may have created yet
+  // Planning encodes tensor maps but reads no memory: any 1 KB-aligned address stands in for the operands.
+  static __align__(1024) char dummy[1024];
+  bf16* d = reinterpret_cast<bf16*>(dummy);
+  const float* f = reinterpret_cast<const float*>(dummy);
+  uint8_t* b = reinterpret_cast<uint8_t*>(dummy);
+  ConvShape s = make_shape(N, H, W, Cin, Cout, k, stride, kind);
+  std::vector<ConvLaunch> ls;
+  if (launch == 0) ls.push_back(plan_conv_forward(s, d, d, d));
+  else if (launch == 1 && (flags & ARGUS_EPI_BN_RAW)) ls.push_back(plan_bnred_dgrad(s, d, d, d, nullptr, 0));
+  else if (launch == 1) ls = plan_conv_dgrad(s, d, d, d);
+  else if (launch == 2 && (flags & ARGUS_EPI_BN_RAW))
+    ls.push_back(plan_bnred_dgrad(make_shape(N, H, W, Cin, Cout, 1, stride, 0), d, d, d, d, concat_channels));
+  else if (launch == 2) ls.push_back(plan_dgrad_concat(make_shape(N, H, W, Cin, Cout, 1, stride, 0), d, d, concat_channels, d, d));
+  else throw Error("unknown launch kind");
+  Epilogue e;
+  if (flags & ARGUS_EPI_SCALE) e.scale = f;
+  if (flags & ARGUS_EPI_SHIFT) e.shift = f;
+  if (flags & ARGUS_EPI_RESIDUAL) e.residual = d;
+  if (flags & ARGUS_EPI_RES_AFFINE) { e.res_scale = f; e.res_shift = f; }
+  if (flags & ARGUS_EPI_RELU) e.relu = 1;
+  if (flags & ARGUS_EPI_RELU_BITS_OUT) e.relu_bits_out = b;
+  if (flags & ARGUS_EPI_OUT_BITS) e.out_bits = b;
+  if (flags & ARGUS_EPI_RESIDUAL_BITS) e.residual_bits = b;
+  if (flags & ARGUS_EPI_STATS) e.stat_partial = const_cast<float*>(f);
+  if (flags & ARGUS_EPI_BN_RAW) { e.bn_raw = d; e.bn_scale = f; e.bn_shift = f; }
+  if (flags & ARGUS_EPI_EARLY_TRIGGER) e.early_trigger = 1;
+  *n_launches = static_cast<int>(ls.size());
+  ARGUS_CHECK(cap >= ARGUS_LAUNCH_INFO_INTS * *n_launches, "launch info buffer too small");
+  for (size_t i = 0; i < ls.size(); ++i) {
+    const ConvLaunchInfo li = conv_launch_info(ls[i], e);
+    const int v[ARGUS_LAUNCH_INFO_INTS] = {li.inst.block_n, li.inst.b_mn, li.inst.opt, li.halo, li.b_resident,
+                                           li.halo_stages, li.num_m_tiles, li.num_n_tiles, li.grid, li.stat_slots};
+    std::memcpy(out + i * ARGUS_LAUNCH_INFO_INTS, v, sizeof(v));
+  }
+  ARGUS_API_END
+}
+
+int argus_conv_instances_record(int on) {
+  ARGUS_API_BEGIN
+  conv_instances_record(on != 0);
+  ARGUS_API_END
+}
+int argus_conv_instances_get(int* keys, int cap, int* n) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(n != nullptr && (keys != nullptr || cap == 0), "null argument");
+  const auto rec = conv_instances_recorded();
+  *n = static_cast<int>(rec.size());
+  for (int i = 0; i < *n && 5 * (i + 1) <= cap; ++i) std::memcpy(keys + 5 * i, rec[i].data(), 5 * sizeof(int));
+  ARGUS_API_END
+}
+
+int argus_conv_instances_all(int* keys, int cap, int* n) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(n != nullptr && (keys != nullptr || cap == 0), "null argument");
+  const auto all = conv_instances_all();
+  *n = static_cast<int>(all.size());
+  for (int i = 0; i < *n && 3 * (i + 1) <= cap; ++i) std::memcpy(keys + 3 * i, all[i].data(), 3 * sizeof(int));
+  ARGUS_API_END
+}
+
+int argus_conv2d_gram(const void* x, float* g, int N, int H, int W, int Cin, int Cout, int stride, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ConvShape s = make_shape(N, H, W, Cin, Cout, 1, stride, 0);
+  validate_shape(s);
+  WgradLaunch l = plan_gram(s, static_cast<const bf16*>(x), g);
+  launch_wgrad(l, lib_scratch(wgrad_scratch_elems(l)), static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
+int argus_colsum_pixels(const void* x, int N, int H, int W, int C, int stride, float* scratch, float* out, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(x != nullptr && scratch != nullptr && out != nullptr, "null argument");
+  ARGUS_CHECK(N > 0 && H > 0 && W > 0 && (stride == 1 || stride == 2) && H % stride == 0 && W % stride == 0,
+              "colsum: bad shape");
+  colsum_pixels_bf16(static_cast<const bf16*>(x), N, H, W, C, stride, scratch, out, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
+int argus_bn_stats_from_gram(const void* W, const float* G, const float* s, double rows, const float* gamma,
+                             const float* beta, float* running_mean, float* running_var, float momentum, float eps,
+                             float* scale, float* shift, float* save_mean, float* save_invstd, float* scratch, int O,
+                             int C, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK((running_mean == nullptr) == (running_var == nullptr), "running mean and variance come together");
+  bn_stats_from_gram(static_cast<const bf16*>(W), G, s, rows, gamma, beta, running_mean, running_var, momentum, eps,
+                     scale, shift, save_mean, save_invstd, scratch, O, C, static_cast<cudaStream_t>(stream));
   ARGUS_API_END
 }
 

@@ -1,12 +1,14 @@
 #include "conv_ops.h"
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
+#include <set>
 
 namespace argus {
 
@@ -574,36 +576,43 @@ WgradLaunch plan_gram(const ConvShape& s, const __nv_bfloat16* x, float* g) {
 // ------------------------------------------------------------------------------------------------
 // launches
 // ------------------------------------------------------------------------------------------------
-template <int BN, int BMN, int EPI, int OPT = kOptAll>
-static void launch_conv_t(const ConvGemmParams& p, cudaStream_t stream) {
+// Final per-launch parameters of one kernel instance: the halo pipeline depth and the weights-resident choice depend
+// on the instance's shared-memory layout and on the grid.
+template <int BN, int BMN, int EPI, int OPT>
+static ConvGemmParams finish_params(const ConvGemmParams& p) {
+  using L = ConvGemmSmem<BN, EPI, conv_staging_buffers<BN, OPT, EPI>()>;
+  const int tiles = p.num_m_tiles * p.num_n_tiles;
+  const int grid = std::min(tiles, num_sms());
+  // weights-resident mode (see ConvGemmParams::b_resident)
+  ConvGemmParams q = p;
+  const int bres = p.num_taps * p.kblocks_per_tap * L::kBBytes;
+  const bool fixed_n = (tiles <= grid) || (grid % p.num_n_tiles == 0);
+  if (q.halo) {
+    const int halo_a = (q.halo_rows + 2) * q.halo_row_bytes;
+    const int stage = halo_a + 3 * L::kBBytes;
+    q.halo_stages = std::min(L::kMaxStages, L::kPipeBytes / stage);
+    if (q.halo_stages < 2) q.halo = 0;
+    // halo + weights resident: when the whole weight slab fits next to two activation boxes (layer1 3x3: 72 KB), the
+    // per-tile L2 -> SM traffic drops from 3 x (32 + 24) to 3 x 32 KB
+    if (q.halo && fixed_n && q.k2_blocks == 0 && bres + 2 * halo_a <= L::kPipeBytes) {
+      q.b_resident = 1;
+      q.halo_stages = std::min(L::kMaxStages, (L::kPipeBytes - bres) / halo_a);
+    }
+  }
+  // (a weights-resident mode for the non-halo launches was built and measured in round 1: no gain -- weights are
+  // served from L2 without cost -- and removed in round 2)
+  return q;
+}
+
+template <int BN, int BMN, int EPI, int OPT>
+static void launch_conv_t(const ConvGemmParams& q, cudaStream_t stream) {
   using L = ConvGemmSmem<BN, EPI, conv_staging_buffers<BN, OPT, EPI>()>;
   static bool configured = false;
   if (!configured) {
     ARGUS_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<BN, BMN, EPI, OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
     configured = true;
   }
-  const int tiles = p.num_m_tiles * p.num_n_tiles;
-  const int grid = std::min(tiles, num_sms());
-  // weights-resident mode (see ConvGemmParams::b_resident)
-  ConvGemmParams q = p;
-  {
-    const int bres = p.num_taps * p.kblocks_per_tap * L::kBBytes;
-    const bool fixed_n = (tiles <= grid) || (grid % p.num_n_tiles == 0);
-    if (q.halo) {
-      const int halo_a = (q.halo_rows + 2) * q.halo_row_bytes;
-      const int stage = halo_a + 3 * L::kBBytes;
-      q.halo_stages = std::min(L::kMaxStages, L::kPipeBytes / stage);
-      if (q.halo_stages < 2) q.halo = 0;
-      // halo + weights resident: when the whole weight slab fits next to two activation boxes (layer1 3x3: 72 KB), the
-      // per-tile L2 -> SM traffic drops from 3 x (32 + 24) to 3 x 32 KB
-      if (q.halo && fixed_n && q.k2_blocks == 0 && bres + 2 * halo_a <= L::kPipeBytes) {
-        q.b_resident = 1;
-        q.halo_stages = std::min(L::kMaxStages, (L::kPipeBytes - bres) / halo_a);
-      }
-    }
-    // (a weights-resident mode for the non-halo launches was built and measured in round 1: no gain -- weights are
-    // served from L2 without cost -- and removed in round 2)
-  }
+  const int grid = std::min(q.num_m_tiles * q.num_n_tiles, num_sms());
   launch_kernel(conv_gemm_kernel<BN, BMN, EPI, OPT>, grid, 64 + 128 * EPI, L::kTotal, stream, q);
   ARGUS_CUDA(cudaGetLastError());
 }
@@ -613,7 +622,51 @@ static void launch_conv_t(const ConvGemmParams& p, cudaStream_t stream) {
 // the epilogue's instruction rate; DESIGN.md section 4) and both were removed in round 2.
 int choose_epilogue_groups(const ConvGemmParams&, int) { return 2; }
 
-void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream) {
+namespace {
+// Every conv_gemm_kernel instance the library compiles, all with two epilogue groups.
+struct ConvInstanceEntry {
+  int block_n, b_mn, opt;
+  ConvGemmParams (*finish)(const ConvGemmParams&);
+  void (*launch)(const ConvGemmParams&, cudaStream_t);
+};
+template <int BN, int BMN, int OPT>
+constexpr ConvInstanceEntry conv_entry() {
+  return {BN, BMN, OPT, &finish_params<BN, BMN, 2, OPT>, &launch_conv_t<BN, BMN, 2, OPT>};
+}
+constexpr int kTail = kOptAffine | kOptRes | kOptRelu;   // fused forward block tail: BN + identity + ReLU (+ bits)
+const ConvInstanceEntry kConvInstances[] = {
+    // dgrad + fused batch-norm backward reduction: plain (3x3 / 1x1 dgrads) or with the bias of the K-concatenated dgrad
+    conv_entry<64, 1, kOptRes | kOptBnRed>(), conv_entry<128, 1, kOptRes | kOptBnRed>(),
+    conv_entry<256, 1, kOptRes | kOptBnRed>(), conv_entry<64, 1, kOptAffine | kOptRes | kOptBnRed>(),
+    conv_entry<128, 1, kOptAffine | kOptRes | kOptBnRed>(), conv_entry<256, 1, kOptAffine | kOptRes | kOptBnRed>(),
+    // folded batch norm without statistics
+    conv_entry<64, 0, kTail>(), conv_entry<128, 0, kTail>(), conv_entry<256, 0, kTail>(),
+    conv_entry<64, 0, kOptAffine | kOptRelu>(), conv_entry<128, 0, kOptAffine | kOptRelu>(),
+    conv_entry<256, 0, kOptAffine | kOptRelu>(), conv_entry<64, 0, kOptAffine>(), conv_entry<128, 0, kOptAffine>(),
+    conv_entry<256, 0, kOptAffine>(),
+    // plain: store the tile (+ statistics)
+    conv_entry<64, 0, 0>(), conv_entry<128, 0, 0>(), conv_entry<256, 0, 0>(), conv_entry<64, 1, 0>(),
+    conv_entry<128, 1, 0>(), conv_entry<256, 1, 0>(),
+    // dgrads: identity-branch gradient + ReLU bits of the previous block; K-concatenated dgrad with bias + bits
+    conv_entry<64, 1, kOptRes | kOptOutBits>(), conv_entry<128, 1, kOptRes | kOptOutBits>(),
+    conv_entry<256, 1, kOptRes | kOptOutBits>(), conv_entry<64, 1, kOptAffine | kOptOutBits>(),
+    conv_entry<128, 1, kOptAffine | kOptOutBits>(), conv_entry<256, 1, kOptAffine | kOptOutBits>(),
+    // the generic kernel
+    conv_entry<64, 0, kOptAll>(), conv_entry<128, 0, kOptAll>(), conv_entry<256, 0, kOptAll>(),
+    conv_entry<64, 1, kOptAll>(), conv_entry<128, 1, kOptAll>(), conv_entry<256, 1, kOptAll>(),
+};
+const ConvInstanceEntry& find_instance(const ConvInstance& c) {
+  for (const auto& e : kConvInstances)
+    if (e.block_n == c.block_n && e.b_mn == c.b_mn && e.opt == c.opt) return e;
+  throw Error("unsupported conv tile configuration");
+}
+
+std::mutex g_record_mu;
+std::atomic<bool> g_recording{false};
+std::set<std::array<int, 5>> g_recorded;
+}  // namespace
+
+ConvGemmParams epilogue_params(const ConvLaunch& l, const Epilogue& e) {
   ConvGemmParams p = l.p;
   p.scale = e.scale;
   p.shift = e.shift;
@@ -644,6 +697,69 @@ void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream) {
   p.relu_bits_out = e.relu_bits_out;
   ARGUS_CHECK((e.res_scale == nullptr) == (e.res_shift == nullptr), "residual scale and shift come together");
   p.stat_partial = e.stat_partial;
+  return p;
+}
+
+// Specialised epilogues for the option combinations the model launches; anything else runs the generic kernel.
+ConvInstance select_conv_instance(const ConvLaunch& l, const ConvGemmParams& p) {
+  ARGUS_CHECK(l.epi == 2, "two epilogue groups");
+  int need = 0;
+  if (p.scale || p.shift) need |= kOptAffine;
+  if (p.has_res) need |= kOptRes;
+  if (p.res_bits || p.res_scale) need |= kOptRes | kOptResExtra;
+  if (p.out_bits) need |= kOptOutBits;
+  if (p.relu || p.relu_bits_out) need |= kOptRelu;
+  if (p.bn_raw != nullptr) return {l.block_n, 1, kOptRes | kOptBnRed | (p.shift != nullptr ? kOptAffine : 0)};
+  // Folded batch norm without statistics (packed-fp32 epilogue, coefficients in shared memory): the fused forward block
+  // tail, its downsample branch, every eval-mode convolution. Needs BOTH coefficient vectors (a bias-only epilogue such as
+  // resnet.fc runs the generic kernel). Round 2 also tried loading the residual row segments straight from global memory
+  // into registers: one thread per row = 32 rows per load instruction, uncoalesced, 1.5-1.9 TB/s against 5.1-5.5 TB/s
+  // through TMA + staging (profiles/r2_direct_residual_ab.txt).
+  const bool folded_bn = p.scale && p.shift && !p.stat_partial && !p.res_bits && !p.res_scale && !p.out_bits;
+  if (l.b_mn == 0 && folded_bn && (need & kOptAffine) && !(need & ~kTail) && (p.relu || !p.relu_bits_out)) {
+    const int t = need & kTail;
+    if (t == kTail || t == (kOptAffine | kOptRelu) || t == kOptAffine) return {l.block_n, 0, t};
+    // e.g. identity + BN without ReLU: generic kernel
+  }
+  if (need == 0) return {l.block_n, l.b_mn, 0};
+  if (l.b_mn == 1 && (need & ~(kOptRes | kOptOutBits)) == 0) return {l.block_n, 1, kOptRes | kOptOutBits};
+  // K-concatenated dgrad of the algebraic BN backward: bias + output bits
+  if (l.b_mn == 1 && (need & ~(kOptAffine | kOptOutBits)) == 0) return {l.block_n, 1, kOptAffine | kOptOutBits};
+  return {l.block_n, l.b_mn, kOptAll};
+}
+
+ConvLaunchInfo conv_launch_info(const ConvLaunch& l, const Epilogue& e) {
+  const ConvGemmParams p = epilogue_params(l, e);
+  ConvLaunchInfo info;
+  info.inst = select_conv_instance(l, p);
+  const ConvGemmParams q = find_instance(info.inst).finish(p);
+  info.halo = q.halo;
+  info.b_resident = q.b_resident;
+  info.halo_stages = q.halo ? q.halo_stages : 0;
+  info.num_m_tiles = q.num_m_tiles;
+  info.num_n_tiles = q.num_n_tiles;
+  info.grid = std::min(q.num_m_tiles * q.num_n_tiles, num_sms());
+  info.stat_slots = stat_slots(l);
+  return info;
+}
+
+void conv_instances_record(bool on) {
+  std::lock_guard<std::mutex> lk(g_record_mu);
+  if (on) g_recorded.clear();
+  g_recording = on;
+}
+std::vector<std::array<int, 3>> conv_instances_all() {
+  std::vector<std::array<int, 3>> v;
+  for (const auto& e : kConvInstances) v.push_back({e.block_n, e.b_mn, e.opt});
+  return v;
+}
+std::vector<std::array<int, 5>> conv_instances_recorded() {
+  std::lock_guard<std::mutex> lk(g_record_mu);
+  return std::vector<std::array<int, 5>>(g_recorded.begin(), g_recorded.end());
+}
+
+void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream) {
+  const ConvGemmParams p = epilogue_params(l, e);
   const double flops = 2.0 * p.m_total * static_cast<double>(p.n_total) * (p.num_taps * p.kblocks_per_tap + p.k2_blocks) * kBlockK;
   std::string fam = l.b_mn ? "conv_dgrad" : "conv_fwd";
   if (g_profiling && profile_detailed())
@@ -662,90 +778,14 @@ void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream) {
     bytes += 2.0 * p.n_total * (p.num_taps * kc + p.k2_blocks * kBlockK);
   }
   ProfileScope prof(fam, stream, flops, bytes);
-  // specialised epilogues: the option combinations the model actually launches; anything else runs the generic kernel
-  constexpr bool special = true;
-  int need = 0;
-  if (p.scale || p.shift) need |= kOptAffine;
-  if (p.has_res) need |= kOptRes;
-  if (p.res_bits || p.res_scale) need |= kOptRes | kOptResExtra;
-  if (p.out_bits) need |= kOptOutBits;
-  if (p.relu || p.relu_bits_out) need |= kOptRelu;
-  constexpr int kTail = kOptAffine | kOptRes | kOptRelu;           // fused forward block tail: BN + identity + ReLU (+ bits)
-  const int epi2 = l.epi;
-  ARGUS_CHECK(epi2 == 2, "two epilogue groups");
-  if (p.bn_raw != nullptr) {
-    // dgrad + fused batch-norm backward reduction: plain (3x3 / 1x1 dgrads) or with the bias of the K-concatenated dgrad
-    ARGUS_CHECK(epi2 == 2, "fused BN reduction: two epilogue groups only");
-    const bool bias = (p.shift != nullptr);
-    switch (l.block_n * 2 + (bias ? 1 : 0)) {
-      case 64 * 2 + 0: launch_conv_t<64, 1, 2, kOptRes | kOptBnRed>(p, stream); return;
-      case 128 * 2 + 0: launch_conv_t<128, 1, 2, kOptRes | kOptBnRed>(p, stream); return;
-      case 256 * 2 + 0: launch_conv_t<256, 1, 2, kOptRes | kOptBnRed>(p, stream); return;
-      case 64 * 2 + 1: launch_conv_t<64, 1, 2, kOptAffine | kOptRes | kOptBnRed>(p, stream); return;
-      case 128 * 2 + 1: launch_conv_t<128, 1, 2, kOptAffine | kOptRes | kOptBnRed>(p, stream); return;
-      case 256 * 2 + 1: launch_conv_t<256, 1, 2, kOptAffine | kOptRes | kOptBnRed>(p, stream); return;
-      default: throw Error("unsupported conv tile configuration");
-    }
+  const ConvInstance inst = select_conv_instance(l, p);
+  const ConvInstanceEntry& entry = find_instance(inst);
+  const ConvGemmParams q = entry.finish(p);
+  if (g_recording) {
+    std::lock_guard<std::mutex> lk(g_record_mu);
+    g_recorded.insert({inst.block_n, inst.b_mn, inst.opt, q.halo, q.b_resident});
   }
-  // Folded batch norm without statistics (packed-fp32 epilogue, coefficients in shared memory): the fused forward block
-  // tail, its downsample branch, every eval-mode convolution. Needs BOTH coefficient vectors (a bias-only epilogue such as
-  // resnet.fc runs the generic kernel). Round 2 also tried loading the residual row segments straight from global memory
-  // into registers: one thread per row = 32 rows per load instruction, uncoalesced, 1.5-1.9 TB/s against 5.1-5.5 TB/s
-  // through TMA + staging (profiles/r2_direct_residual_ab.txt).
-  const bool folded_bn = p.scale && p.shift && !p.stat_partial && !p.res_bits && !p.res_scale && !p.out_bits;
-  if (special && epi2 == 2 && l.b_mn == 0 && folded_bn && (need & kOptAffine) && !(need & ~kTail) &&
-      (p.relu || !p.relu_bits_out)) {
-    switch (l.block_n * 16 + (need & kTail)) {
-      case 64 * 16 + kTail: launch_conv_t<64, 0, 2, kTail>(p, stream); return;
-      case 128 * 16 + kTail: launch_conv_t<128, 0, 2, kTail>(p, stream); return;
-      case 256 * 16 + kTail: launch_conv_t<256, 0, 2, kTail>(p, stream); return;
-      case 64 * 16 + (kOptAffine | kOptRelu): launch_conv_t<64, 0, 2, kOptAffine | kOptRelu>(p, stream); return;
-      case 128 * 16 + (kOptAffine | kOptRelu): launch_conv_t<128, 0, 2, kOptAffine | kOptRelu>(p, stream); return;
-      case 256 * 16 + (kOptAffine | kOptRelu): launch_conv_t<256, 0, 2, kOptAffine | kOptRelu>(p, stream); return;
-      case 64 * 16 + kOptAffine: launch_conv_t<64, 0, 2, kOptAffine>(p, stream); return;
-      case 128 * 16 + kOptAffine: launch_conv_t<128, 0, 2, kOptAffine>(p, stream); return;
-      case 256 * 16 + kOptAffine: launch_conv_t<256, 0, 2, kOptAffine>(p, stream); return;
-      default: break;   // e.g. identity + BN without ReLU: generic kernel
-    }
-  }
-  if (special && epi2 == 2 && need == 0) {
-    switch (l.block_n * 2 + l.b_mn) {
-      case 64 * 2 + 0: launch_conv_t<64, 0, 2, 0>(p, stream); return;
-      case 128 * 2 + 0: launch_conv_t<128, 0, 2, 0>(p, stream); return;
-      case 256 * 2 + 0: launch_conv_t<256, 0, 2, 0>(p, stream); return;
-      case 64 * 2 + 1: launch_conv_t<64, 1, 2, 0>(p, stream); return;
-      case 128 * 2 + 1: launch_conv_t<128, 1, 2, 0>(p, stream); return;
-      case 256 * 2 + 1: launch_conv_t<256, 1, 2, 0>(p, stream); return;
-      default: break;
-    }
-  }
-  if (special && epi2 == 2 && l.b_mn == 1 && (need & ~(kOptRes | kOptOutBits)) == 0) {
-    switch (l.block_n) {
-      case 64: launch_conv_t<64, 1, 2, kOptRes | kOptOutBits>(p, stream); return;
-      case 128: launch_conv_t<128, 1, 2, kOptRes | kOptOutBits>(p, stream); return;
-      case 256: launch_conv_t<256, 1, 2, kOptRes | kOptOutBits>(p, stream); return;
-      default: break;
-    }
-  }
-  if (special && epi2 == 2 && l.b_mn == 1 && (need & ~(kOptAffine | kOptOutBits)) == 0) {
-    // K-concatenated dgrad of the algebraic BN backward: bias + output bits
-    switch (l.block_n) {
-      case 64: launch_conv_t<64, 1, 2, kOptAffine | kOptOutBits>(p, stream); return;
-      case 128: launch_conv_t<128, 1, 2, kOptAffine | kOptOutBits>(p, stream); return;
-      case 256: launch_conv_t<256, 1, 2, kOptAffine | kOptOutBits>(p, stream); return;
-      default: break;
-    }
-  }
-  const int key = (l.block_n * 2 + l.b_mn) * 4 + epi2;
-  switch (key) {
-    case (64 * 2 + 0) * 4 + 2: launch_conv_t<64, 0, 2>(p, stream); break;
-    case (128 * 2 + 0) * 4 + 2: launch_conv_t<128, 0, 2>(p, stream); break;
-    case (256 * 2 + 0) * 4 + 2: launch_conv_t<256, 0, 2>(p, stream); break;
-    case (64 * 2 + 1) * 4 + 2: launch_conv_t<64, 1, 2>(p, stream); break;
-    case (128 * 2 + 1) * 4 + 2: launch_conv_t<128, 1, 2>(p, stream); break;
-    case (256 * 2 + 1) * 4 + 2: launch_conv_t<256, 1, 2>(p, stream); break;
-    default: throw Error("unsupported conv tile configuration");
-  }
+  entry.launch(q, stream);
 }
 
 int stat_slots(const ConvLaunch& l) {

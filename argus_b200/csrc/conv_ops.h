@@ -1,6 +1,9 @@
 // Host-side planning for the tcgen05 convolution kernels: turns a convolution shape plus device pointers into
 // kernel parameter blocks (TMA tensor maps, filter-tap tables, tile counts) once, so the hot path only launches.
 #pragma once
+#include <array>
+#include <vector>
+
 #include "conv_gemm.cuh"
 #include "runtime.h"
 
@@ -101,6 +104,29 @@ WgradLaunch plan_gram(const ConvShape& s, const __nv_bfloat16* x, float* g);
 void stem_dgrad(const __nv_bfloat16* dy, const __nv_bfloat16* w, float* dx, int N, int H, int W, cudaStream_t stream);
 
 void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream);
+
+// The conv_gemm_kernel<block_n, b_mn, 2, opt> instance a launch runs (opt = kOptAll for the generic kernel).
+struct ConvInstance {
+  int block_n = 0, b_mn = 0, opt = 0;
+};
+// Kernel parameters of launch l with epilogue e (residual / raw-tile tensor maps included); checks the combination.
+ConvGemmParams epilogue_params(const ConvLaunch& l, const Epilogue& e);
+// The instance launch_conv dispatches p to. Pure: the launcher and conv_launch_info both call it.
+ConvInstance select_conv_instance(const ConvLaunch& l, const ConvGemmParams& p);
+// Everything launch_conv decides for (l, e) without launching: the instance, the final halo / weights-resident mode,
+// the tile counts and the grid.
+struct ConvLaunchInfo {
+  ConvInstance inst;
+  int halo = 0, b_resident = 0, halo_stages = 0;
+  int num_m_tiles = 0, num_n_tiles = 0, grid = 0, stat_slots = 0;
+};
+ConvLaunchInfo conv_launch_info(const ConvLaunch& l, const Epilogue& e);
+// While recording is on, launch_conv adds the key (block_n, b_mn, opt, halo, b_resident) of every launch to a host-side
+// set; turning it on clears the set.
+void conv_instances_record(bool on);
+std::vector<std::array<int, 5>> conv_instances_recorded();
+// (block_n, b_mn, opt) of every kernel instance launch_conv can dispatch to
+std::vector<std::array<int, 3>> conv_instances_all();
 int choose_epilogue_groups(const ConvGemmParams& p, int block_n);
 // number of statistic slots launch_conv writes for this launch (one per epilogue group per CTA)
 int stat_slots(const ConvLaunch& l);

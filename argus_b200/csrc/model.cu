@@ -702,6 +702,8 @@ void Model::copy_activation(int index, void* dst, int64_t capacity_elems, int64_
     src = p.pooled0; r = static_cast<int64_t>(p.N) * (p.H / 4) * (p.W / 4); c = 64;
   } else if (index >= 0 && index < static_cast<int>(p.blocks.size())) {
     src = p.blocks[index].out; r = p.blocks[index].rows_out; c = blocks_[index].c3.shape.Cout;
+  } else if (index >= 100 && index < 100 + static_cast<int>(p.blocks.size())) {
+    src = p.blocks[index - 100].act2; r = p.blocks[index - 100].rows_out; c = blocks_[index - 100].c2.shape.Cout;
   } else if (index == 16) {
     src = p.pooled; r = p.N; c = 2048;
   } else if (index == 17) {

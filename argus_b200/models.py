@@ -373,7 +373,8 @@ class NCameraCNN(nn.Module):
 
     def probe_activation(self, index: int) -> torch.Tensor:
         """Test probe: activation of the last forward as a (rows, C) bf16 tensor (NHWC rows).
-        index -1: pooled stem output, 0..15: bottleneck outputs, 16: pooled features, 17: resnet.fc output."""
+        index -1: pooled stem output, 0..15: bottleneck outputs, 16: pooled features, 17: resnet.fc output,
+        100..115: act2 (the input of conv3) of each bottleneck."""
         self._ensure_bound()
         dev = self._flat_params.device
         cap = 1 << 28

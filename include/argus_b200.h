@@ -66,6 +66,60 @@ int argus_conv2d_dgrad_bits(const void* dy, const void* w, void* dx, int N, int 
 int argus_conv2d_dgrad_ex(const void* dy, const void* w, void* dx, int N, int H, int W, int Cin, int Cout, int stride,
                           const void* concat_a, int concat_channels, const float* bias, const void* residual,
                           const void* out_bits, float* stat_partial, int stat_slot_capacity, void* stream);
+/* Forward convolution with every field of the epilogue: y = [relu](acc * scale + shift [+ residual * res_scale +
+ * res_shift]); scale, shift, residual, res_scale / res_shift (both or neither) are nullable. relu_bits_out (nullable,
+ * needs relu): [rows][Cout/8] bytes, bit = (value before the ReLU > 0). stat_partial as for argus_conv2d_forward.
+ * early_trigger: let the next kernel of the stream start its prologue while this one runs (the eval-mode chain). */
+int argus_conv2d_forward_full(const void* x, const void* w, void* y, int N, int H, int W, int Cin, int Cout, int k,
+                              int stride, int kind, const float* scale, const float* shift, const void* residual,
+                              const float* res_scale, const float* res_shift, int relu, void* relu_bits_out,
+                              float* stat_partial, int stat_slot_capacity, int early_trigger, void* stream);
+/* Stride-1 dgrad with the batch-norm backward reduction fused into its epilogue: g = conv_transpose(dy, w) [+ bias] is
+ * stored masked by (bn_raw * bn_scale + bn_shift > 0), and the zero-filled stat_partial [slots][2][Cin] receives
+ * sum(g) and sum(g * bn_raw) of the stored values. k = 1 or 3; with concat_a (k = 1 only) the K-concatenated form of
+ * argus_conv2d_dgrad_ex, where w is the stacked [(Cout + concat_channels)][Cin] matrix and bias is nullable. */
+int argus_conv2d_dgrad_bnred(const void* dy, const void* w, void* dx, int N, int H, int W, int Cin, int Cout, int k,
+                             int stride, const void* concat_a, int concat_channels, const float* bias,
+                             const void* bn_raw, const float* bn_scale, const float* bn_shift, float* stat_partial,
+                             int stat_slot_capacity, void* stream);
+/* Plans a convolution the way the calls above do and reports, without launching, what each of its launches would run.
+ * launch: 0 forward (kind as for argus_conv2d_forward), 1 dgrad, 2 K-concatenated 1x1 dgrad (concat_channels).
+ * flags: the epilogue fields that are present (ARGUS_EPI_*). Per launch, ARGUS_LAUNCH_INFO_INTS ints go to out:
+ * block_n, b_mn, opt (kernel option mask; 31 = the generic kernel), halo, b_resident, halo_stages, num_m_tiles,
+ * num_n_tiles, grid, stat_slots. */
+#define ARGUS_EPI_SCALE 1
+#define ARGUS_EPI_SHIFT 2
+#define ARGUS_EPI_RESIDUAL 4
+#define ARGUS_EPI_RES_AFFINE 8
+#define ARGUS_EPI_RELU 16
+#define ARGUS_EPI_RELU_BITS_OUT 32
+#define ARGUS_EPI_OUT_BITS 64
+#define ARGUS_EPI_RESIDUAL_BITS 128
+#define ARGUS_EPI_STATS 256
+#define ARGUS_EPI_BN_RAW 512
+#define ARGUS_EPI_EARLY_TRIGGER 1024
+#define ARGUS_LAUNCH_INFO_INTS 10
+int argus_conv2d_launch_info(int launch, int N, int H, int W, int Cin, int Cout, int k, int stride, int kind,
+                             int concat_channels, int flags, int* out, int cap, int* n_launches);
+/* Records the kernel instance of every convolution launch while on (turning it on clears the record); get copies up to
+ * cap keys of five ints (block_n, b_mn, opt, halo, b_resident) and sets *n to the number recorded. */
+int argus_conv_instances_record(int on);
+int argus_conv_instances_get(int* keys, int cap, int* n);
+/* Every kernel instance a convolution launch can run: up to cap keys of three ints (block_n, b_mn, opt); *n = count. */
+int argus_conv_instances_all(int* keys, int cap, int* n);
+/* g[Cin][Cin] (fp32, +=; the caller zero-fills) = x_s^T x_s over the pixels a 1x1 convolution of this shape reads (its
+ * even pixels at stride 2): the Gram matrix from which the statistics of the convolution's output follow. */
+int argus_conv2d_gram(const void* x, float* g, int N, int H, int W, int Cin, int Cout, int stride, void* stream);
+/* out[C] = column sums (fp32, deterministic) of the bf16 (N, H, W, C) tensor over the pixels a stride-`stride` 1x1
+ * convolution reads. C / 8 a power of two, C <= 2048; scratch: 4 * (SM count) * C floats. */
+int argus_colsum_pixels(const void* x, int N, int H, int W, int C, int stride, float* scratch, float* out, void* stream);
+/* Train-mode batch norm of y = x W^T from G = x^T x [C][C] and s = colsum(x) [C] over `rows` pixels, without y: the
+ * folded scale / shift, save_mean / save_invstd and (when running_mean is not null) the running statistics, as
+ * argus_bn_finalize computes them. W: bf16 [O][C], O % 16 == 0, C % 32 == 0; scratch: O * C / 16 floats. */
+int argus_bn_stats_from_gram(const void* W, const float* G, const float* s, double rows, const float* gamma,
+                             const float* beta, float* running_mean, float* running_var, float momentum, float eps,
+                             float* scale, float* shift, float* save_mean, float* save_invstd, float* scratch, int O,
+                             int C, void* stream);
 /* 1x1: dw[(Cout + Cin)][Cin] (fp32, +=): rows < Cout = dy^T x, rows Cout + j = x^T x (Gram matrix of the pixels the
  * convolution reads); Cout % 128 == 0. One launch, the x tiles are loaded once. */
 int argus_conv2d_wgrad_gram(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int stride,
@@ -250,7 +304,8 @@ int argus_model_stage_range(argus_model* m, int stage, int64_t* begin, int64_t* 
 int argus_model_arena_bytes(argus_model* m, int64_t* bytes);
 /* Test probe: copy an activation of the last forward pass (bf16, NHWC rows x C) into dst (device memory).
  * index -1: stem output after max pooling; 0..15: bottleneck outputs (torchvision layer1[0] .. layer4[2]);
- * 16: global-average-pooled features; 17: resnet.fc output. */
+ * 16: global-average-pooled features; 17: resnet.fc output; 100..115: act2 of each bottleneck (the input of conv3,
+ * relu(bn2(conv2)): what the fused block tail takes its Gram matrix of). */
 int argus_model_copy_activation(argus_model* m, int index, void* dst, int64_t capacity_elems, int64_t* rows, int* C,
                                 void* stream);
 
