@@ -404,6 +404,7 @@ int argus_bn_backward(void* dy, const void* x, const void* out, const float* sca
   ARGUS_API_BEGIN
   require_sm100();
   cudaStream_t s = static_cast<cudaStream_t>(stream);
+  bn_check_aligned(dy, x, out, dx);   // dx too: the reduce pass below already adds to dgamma / dbeta
   bn_bwd_reduce(static_cast<const bf16*>(dy), static_cast<const bf16*>(x), static_cast<const bf16*>(out), scale, shift,
                 mean, invstd, dgamma, dbeta, rows, C, mask_mode, lib_scratch(bn_bwd_scratch_elems()), s);
   bn_bwd_apply(static_cast<bf16*>(dy), static_cast<const bf16*>(x), static_cast<const bf16*>(out), scale, shift, mean,

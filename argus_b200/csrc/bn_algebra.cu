@@ -315,28 +315,6 @@ colsum_partial_kernel(const uint4* __restrict__ x, float* __restrict__ partial, 
     }
   }
 }
-// block = 8 channels x 32 lanes: lane sl adds blocks sl, sl+32, ... in order, lane 0 then adds the 32 lane sums in
-// order (bitwise reproducible, 32-way parallel; a single thread per channel took 80 us over 1184 partials)
-__global__ void __launch_bounds__(256)
-colsum_final_kernel(const float* __restrict__ partial, int blocks, float* __restrict__ out, int C) {
-  pdl_prologue();
-  __shared__ double red[32][8];
-  const int ch = threadIdx.x & 7, sl = threadIdx.x >> 3;
-  const int c = blockIdx.x * 8 + ch;
-  double acc = 0.0;
-  if (c < C)
-    for (int b = sl; b < blocks; b += 32) acc += static_cast<double>(partial[static_cast<size_t>(b) * C + c]);
-  red[sl][ch] = acc;
-  __syncthreads();
-  if (sl != 0 || c >= C) return;
-  acc = 0.0;
-  for (int k = 0; k < 32; ++k) acc += red[k][ch];
-  out[c] = static_cast<float>(acc);
-}
-void colsum_finalize(const float* partial, int blocks, float* out, int C, cudaStream_t st) {
-  launch_kernel(colsum_final_kernel, (C + 7) / 8, 256, 0, st, partial, blocks, out, C);
-  ARGUS_CUDA(cudaGetLastError());
-}
 void colsum_rows_bf16(const bf16* x, int64_t rows, int C, float* scratch, float* out, cudaStream_t st) {
   colsum_pixels_bf16(x, static_cast<int>(rows), 1, 1, C, 1, scratch, out, st);
 }
@@ -352,8 +330,7 @@ void colsum_pixels_bf16(const bf16* x, int N, int H, int W, int C, int stride, f
   launch_kernel(colsum_partial_kernel, blocks, 256, 0, st, reinterpret_cast<const uint4*>(x), scratch, rows, cvec, stride, W / stride,
                                                 (H / stride) * (W / stride), W, H * W);
   ARGUS_CUDA(cudaGetLastError());
-  launch_kernel(colsum_final_kernel, (C + 7) / 8, 256, 0, st, scratch, blocks, out, C);
-  ARGUS_CUDA(cudaGetLastError());
+  colsum_finalize(scratch, blocks, out, C, st);
 }
 
 int64_t bn_alg_matrix_scratch_elems(int C) { return static_cast<int64_t>(kSplitO) * (C + 1) * C; }

@@ -257,48 +257,62 @@ __device__ __forceinline__ float ldg_f32_issue(const float* p) {
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// batch norm: finalize / fold
+// batch norm: finalize / fold, and the ordered sum of per-block partials every finalize shares
 // ------------------------------------------------------------------------------------------------------------
-// block = 8 channels x 32 slot lanes: lane sl adds slots sl, sl+32, ... in order, then lane 0 adds the 32 lane sums in
-// order -> the statistics are bitwise reproducible and the slot loop is 32-way parallel.
+// Sums of the NS series of partial = [slots][NS][C] for channel c = blockIdx.x * 8 + (threadIdx.x & 7).
+// Block = 8 channels x 32 slot lanes: lane sl adds slots sl, sl+32, ... in order in fp64, then lane 0 adds the 32 lane
+// sums in order -> bitwise reproducible, and the slot loop is 32-way parallel (a single thread per channel took 80 us
+// over 1184 partials). The loads of eight slots are issued together (one L2 round trip instead of eight); missing
+// slots are skipped, so the additions are those of the plain loop.
+// Returns true in the one thread per channel (lane 0, c < C) that then holds the channel's totals in sum[].
+template <int NS>
+__device__ __forceinline__ bool ordered_slot_sum(const float* __restrict__ partial, int slots, int C, double (&sum)[NS]) {
+  __shared__ double red[NS][32][8];
+  const int ch = threadIdx.x & 7, sl = threadIdx.x >> 3;
+  const int c = blockIdx.x * 8 + ch;
+#pragma unroll
+  for (int j = 0; j < NS; ++j) sum[j] = 0.0;
+  if (c < C) {
+    for (int k = sl; k < slots; k += 32 * 8) {
+      float a[8][NS];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) {
+        const int kk = min(k + 32 * u, slots - 1);   // clamped: always a valid address, masked below
+#pragma unroll
+        for (int j = 0; j < NS; ++j) a[u][j] = ldg_f32_issue(partial + (static_cast<size_t>(kk) * NS + j) * C + c);
+      }
+#pragma unroll
+      for (int u = 0; u < 8; ++u) {
+        if (k + 32 * u < slots) {
+#pragma unroll
+          for (int j = 0; j < NS; ++j) sum[j] += static_cast<double>(a[u][j]);
+        }
+      }
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < NS; ++j) red[j][sl][ch] = sum[j];
+  __syncthreads();
+  if (sl != 0 || c >= C) return false;
+#pragma unroll
+  for (int j = 0; j < NS; ++j) sum[j] = 0.0;
+  for (int k = 0; k < 32; ++k) {
+#pragma unroll
+    for (int j = 0; j < NS; ++j) sum[j] += red[j][k][ch];
+  }
+  return true;
+}
+
 __global__ void __launch_bounds__(256)
 bn_finalize_kernel(const float* __restrict__ partial, int slots, double count, const float* gamma, const float* beta,
                    float* running_mean, float* running_var, float momentum, float eps, float* scale, float* shift,
                    float* save_mean, float* save_invstd, int C) {
   pdl_prologue();
-  __shared__ double red[2][32][8];
-  const int ch = threadIdx.x & 7, sl = threadIdx.x >> 3;
-  const int c = blockIdx.x * 8 + ch;
-  double sum = 0.0, sqsum = 0.0;
-  if (c < C) {
-    // eight slots per batch: the loads are issued together (one L2 round trip instead of eight), the additions keep
-    // the slot order (missing slots are skipped) -> same bits as the plain loop
-    for (int k = sl; k < slots; k += 32 * 8) {
-      float a[8], b[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int kk = min(k + 32 * u, slots - 1);   // clamped: always a valid address, masked below
-        a[u] = ldg_f32_issue(partial + (static_cast<size_t>(kk) * 2 + 0) * C + c);
-        b[u] = ldg_f32_issue(partial + (static_cast<size_t>(kk) * 2 + 1) * C + c);
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        if (k + 32 * u < slots) {
-          sum += static_cast<double>(a[u]);
-          sqsum += static_cast<double>(b[u]);
-        }
-      }
-    }
-  }
-  red[0][sl][ch] = sum;
-  red[1][sl][ch] = sqsum;
-  __syncthreads();
-  if (sl != 0 || c >= C) return;
-  sum = 0.0;
-  sqsum = 0.0;
-  for (int k = 0; k < 32; ++k) { sum += red[0][k][ch]; sqsum += red[1][k][ch]; }
-  const double mean = sum / count;
-  double var = sqsum / count - mean * mean;
+  double s[2];   // sum x, sum x^2
+  if (!ordered_slot_sum<2>(partial, slots, C, s)) return;
+  const int c = blockIdx.x * 8 + (threadIdx.x & 7);
+  const double mean = s[0] / count;
+  double var = s[1] / count - mean * mean;
   if (var < 0) var = 0;
   const float invstd = static_cast<float>(1.0 / sqrt(var + static_cast<double>(eps)));
   const float sc = gamma[c] * invstd;
@@ -336,289 +350,68 @@ void bn_fold_eval(const float* gamma, const float* beta, const float* running_me
   ARGUS_CUDA(cudaGetLastError());
 }
 
-// ------------------------------------------------------------------------------------------------------------
-// batch norm apply (+ residual, + ReLU)
-// ------------------------------------------------------------------------------------------------------------
-template <int RES, bool SUM>  // RES: 0 none, 1 plain residual, 2 residual with its own scale/shift (downsample branch)
-__global__ void __launch_bounds__(256)
-bn_apply_kernel(const uint4* __restrict__ x, const float* __restrict__ scale, const float* __restrict__ shift,
-                const uint4* __restrict__ res, const float* __restrict__ rscale, const float* __restrict__ rshift,
-                int relu, uint4* __restrict__ y, uint8_t* __restrict__ bits, float* __restrict__ colsum_partial,
-                int64_t nvec, int cvec) {
-  pdl_prologue();
-  // gridDim.x * 256 is a multiple of cvec (a power of two <= 256), so a thread always sees the same channel octet:
-  // the per-channel constants live in registers for the whole grid-stride loop.
-  const int64_t tid = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
-  const int c0 = static_cast<int>(tid & (cvec - 1)) * 8;
-  const F8 sc = load8f(scale + c0), sh = load8f(shift + c0);
-  F8 rs, rb;
-  if (RES == 2) { rs = load8f(rscale + c0); rb = load8f(rshift + c0); }
-  F8 acc;
-#pragma unroll
-  for (int k = 0; k < 8; ++k) acc.v[k] = 0.f;
-  auto one = [&](int64_t i, const uint4& xq, const uint4& rq) {
-    const F8 xv = unpack8(xq);
-    F8 o;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) o.v[k] = fmaf(xv.v[k], sc.v[k], sh.v[k]);
-    if (RES == 1) {
-      const F8 rv = unpack8(rq);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) o.v[k] += rv.v[k];
-    } else if (RES == 2) {
-      const F8 rv = unpack8(rq);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) o.v[k] += fmaf(rv.v[k], rs.v[k], rb.v[k]);
-    }
-    if (bits != nullptr) bits[i] = positive_bits(o);
-    if (relu) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) o.v[k] = fmaxf(o.v[k], 0.f);
-    }
-    const uint4 packed = pack8(o);
-    y[i] = packed;
-    if (SUM) {
-      const F8 r = unpack8(packed);   // sums of the STORED (bf16) values
-#pragma unroll
-      for (int k = 0; k < 8; ++k) acc.v[k] += r.v[k];
-    }
-  };
-  int64_t i = tid;
-  for (; i + stride < nvec; i += 2 * stride) {
-    const uint4 xa = ldg_stream(x + i), xb = ldg_stream(x + i + stride);
-    uint4 ra = make_uint4(0, 0, 0, 0), rbv = ra;
-    if (RES != 0) { ra = ldg_stream(res + i); rbv = ldg_stream(res + i + stride); }
-    one(i, xa, ra);
-    one(i + stride, xb, rbv);
-  }
-  for (; i < nvec; i += stride) {
-    uint4 ra = make_uint4(0, 0, 0, 0);
-    if (RES != 0) ra = ldg_stream(res + i);
-    one(i, ldg_stream(x + i), ra);
-  }
-  if (SUM) {
-    // per-block column sums of the output: threads t, t + cvec, ... of the block share a channel octet
-    __shared__ float red[8][256];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) red[k][threadIdx.x] = acc.v[k];
-    __syncthreads();
-    const int lanes = cvec < 256 ? cvec : 256;
-    if (threadIdx.x < lanes) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        float s0 = 0.f;
-        for (int r = threadIdx.x; r < 256; r += lanes) s0 += red[k][r];
-        colsum_partial[static_cast<size_t>(blockIdx.x) * (cvec * 8) + threadIdx.x * 8 + k] = s0;
-      }
-    }
-  }
-}
-// shared-memory ring version (defined below, next to the ring versions of the backward passes)
-static bool bn_ring_enabled();
-static int bn_ring_grid(int64_t nvec);
-static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-static void launch_bn_apply_ring(const uint4* x, const float* scale, const float* shift, const uint4* res,
-                                 const float* rscale, const float* rshift, int relu, uint4* y, uint8_t* bits,
-                                 float* colsum_partial, int64_t nvec, int cvec, cudaStream_t s);
-// number of per-block column-sum partials bn_apply writes (callers size and finalize the buffer with this)
-int bn_apply_grid(int64_t rows, int C) {
-  return bn_ring_enabled() ? bn_ring_grid(rows * (C / 8)) : grid_for(rows * (C / 8), 256);
-}
-void bn_apply(const bf16* x, const float* scale, const float* shift, const bf16* res, const float* rscale,
-              const float* rshift, int relu, bf16* y, uint8_t* relu_bits, float* colsum_partial, int64_t rows, int C,
-              cudaStream_t s) {
-  ProfileScope prof("bn_apply", s, 0, static_cast<double>(rows) * C * (2 * (res ? 3 : 2) + (relu_bits ? 0.125 : 0.0)));
-  ARGUS_CHECK(C % 8 == 0 && is_pow2(C / 8) && C <= 2048, "bn_apply: C/8 must be a power of two <= 256");
-  const int64_t nvec = rows * (C / 8);
-  const int grid = bn_apply_grid(rows, C);
-  auto X = reinterpret_cast<const uint4*>(x);
-  auto R = reinterpret_cast<const uint4*>(res);
-  auto Y = reinterpret_cast<uint4*>(y);
-  if (bn_ring_enabled()) {
-    ARGUS_CHECK(aligned16(x) && aligned16(res) && aligned16(y), "bn_apply: tensors must be 16-byte aligned");
-    ARGUS_CHECK(colsum_partial == nullptr || res == nullptr, "column sums are only produced by the plain (no residual) variant");
-    launch_bn_apply_ring(X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, colsum_partial, nvec, C / 8, s);
-    ARGUS_CUDA(cudaGetLastError());
-    return;
-  }
-  if (colsum_partial != nullptr) {
-    ARGUS_CHECK(res == nullptr, "column sums are only produced by the plain (no residual) variant");
-    launch_kernel(bn_apply_kernel<0, true>, grid, 256, 0, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, colsum_partial, nvec, C / 8);
-  } else if (res == nullptr) {
-    launch_kernel(bn_apply_kernel<0, false>, grid, 256, 0, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, nullptr, nvec, C / 8);
-  } else if (rscale == nullptr) {
-    launch_kernel(bn_apply_kernel<1, false>, grid, 256, 0, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, nullptr, nvec, C / 8);
-  } else {
-    launch_kernel(bn_apply_kernel<2, false>, grid, 256, 0, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, nullptr, nvec, C / 8);
-  }
-  ARGUS_CUDA(cudaGetLastError());
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// batch norm backward: per-channel reductions, then the elementwise input gradient
-// ------------------------------------------------------------------------------------------------------------
-template <int MASK>
-__global__ void __launch_bounds__(256)
-bn_bwd_reduce_kernel(const uint4* __restrict__ dy, const uint4* __restrict__ x, const uint4* __restrict__ out,
-                     const float* __restrict__ scale, const float* __restrict__ shift,
-                     const float* __restrict__ mean, const float* __restrict__ invstd, float* __restrict__ partial,
-                     int64_t rows, int cvec) {
-  pdl_prologue();
-  __shared__ float red[16][256];
-  const int lanes = cvec < 256 ? cvec : 256;   // threads along the channel dimension (cvec <= 256 for C <= 2048)
-  const int row_lanes = 256 / lanes;           // rows processed concurrently by one block
-  const int rl = threadIdx.x / lanes;
-  const int oc = threadIdx.x % lanes;
-  const int c0 = oc * 8;
-  const F8 sc = load8f(scale + c0), sh = load8f(shift + c0), mu = load8f(mean + c0), is = load8f(invstd + c0);
-  float a_dy[8], a_dyx[8];
-#pragma unroll
-  for (int k = 0; k < 8; ++k) a_dy[k] = a_dyx[k] = 0.f;
-  const uint8_t* bits = reinterpret_cast<const uint8_t*>(out);   // MASK == 3: one byte per channel octet
-  auto body = [&](const uint4& dyv, const uint4& xv4, const uint4& ov4) {
-    const F8 d = unpack8(dyv);
-    const F8 xv = unpack8(xv4);
-    F8 g = d;
-    if (MASK == 1) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) g.v[k] = fmaf(xv.v[k], sc.v[k], sh.v[k]) > 0.f ? d.v[k] : 0.f;
-    } else if (MASK == 2) {
-      const F8 o = unpack8(ov4);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) g.v[k] = o.v[k] > 0.f ? d.v[k] : 0.f;
-    } else if (MASK == 3) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) g.v[k] = ((ov4.x >> k) & 1u) ? d.v[k] : 0.f;
-    }
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      a_dy[k] += g.v[k];
-      a_dyx[k] = fmaf(g.v[k], xv.v[k], a_dyx[k]);   // sum g*x; centred and scaled by invstd once at the end
-    }
-  };
-  const int64_t rstride = static_cast<int64_t>(gridDim.x) * row_lanes;
-  int64_t row = static_cast<int64_t>(blockIdx.x) * row_lanes + rl;
-  for (; row + rstride < rows; row += 2 * rstride) {
-    const int64_t i0 = row * cvec + oc, i1 = (row + rstride) * cvec + oc;
-    const uint4 d0 = ldg_stream(dy + i0), d1 = ldg_stream(dy + i1);
-    const uint4 x0 = ldg_stream(x + i0), x1 = ldg_stream(x + i1);
-    uint4 o0 = make_uint4(0, 0, 0, 0), o1 = o0;
-    if (MASK == 2) { o0 = ldg_stream(out + i0); o1 = ldg_stream(out + i1); }
-    if (MASK == 3) { o0.x = __ldg(bits + i0); o1.x = __ldg(bits + i1); }
-    body(d0, x0, o0);
-    body(d1, x1, o1);
-  }
-  for (; row < rows; row += rstride) {
-    const int64_t i0 = row * cvec + oc;
-    uint4 o0 = make_uint4(0, 0, 0, 0);
-    if (MASK == 2) o0 = ldg_stream(out + i0);
-    if (MASK == 3) o0.x = __ldg(bits + i0);
-    body(ldg_stream(dy + i0), ldg_stream(x + i0), o0);
-  }
-#pragma unroll
-  for (int k = 0; k < 8; ++k) {
-    red[k][threadIdx.x] = a_dy[k];
-    red[8 + k][threadIdx.x] = (a_dyx[k] - mu.v[k] * a_dy[k]) * is.v[k];
-  }
-  __syncthreads();
-  if (rl == 0) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      float s0 = 0.f, s1 = 0.f;
-      for (int r = 0; r < row_lanes; ++r) {
-        s0 += red[k][r * lanes + oc];
-        s1 += red[8 + k][r * lanes + oc];
-      }
-      // partial[block][0][c] = sum g, partial[block][1][c] = sum g * xhat
-      partial[(static_cast<size_t>(blockIdx.x) * 2 + 0) * (cvec * 8) + c0 + k] = s0;
-      partial[(static_cast<size_t>(blockIdx.x) * 2 + 1) * (cvec * 8) + c0 + k] = s1;
-    }
-  }
-}
-
 __global__ void __launch_bounds__(256)
 bn_bwd_finalize_kernel(const float* __restrict__ partial, int blocks, float* dgamma, float* dbeta, int C,
                        const float* __restrict__ mean, const float* __restrict__ invstd) {
   pdl_prologue();
-  __shared__ double red[2][32][8];
-  const int ch = threadIdx.x & 7, sl = threadIdx.x >> 3;
-  const int c = blockIdx.x * 8 + ch;
-  double sb = 0.0, sg = 0.0;
-  if (c < C) {
-    for (int k = sl; k < blocks; k += 32 * 8) {   // batched loads, ordered additions (see bn_finalize_kernel)
-      float a[8], b[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int kk = min(k + 32 * u, blocks - 1);
-        a[u] = ldg_f32_issue(partial + (static_cast<size_t>(kk) * 2 + 0) * C + c);
-        b[u] = ldg_f32_issue(partial + (static_cast<size_t>(kk) * 2 + 1) * C + c);
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        if (k + 32 * u < blocks) {
-          sb += static_cast<double>(a[u]);
-          sg += static_cast<double>(b[u]);
-        }
-      }
-    }
-  }
-  red[0][sl][ch] = sb;
-  red[1][sl][ch] = sg;
-  __syncthreads();
-  if (sl != 0 || c >= C) return;
-  sb = 0.0;
-  sg = 0.0;
-  for (int k = 0; k < 32; ++k) { sb += red[0][k][ch]; sg += red[1][k][ch]; }
+  double s[2];   // sum g, sum g * xhat
+  if (!ordered_slot_sum<2>(partial, blocks, C, s)) return;
+  const int c = blockIdx.x * 8 + (threadIdx.x & 7);
   // mean != nullptr: the second sums are sum(g * x) of the RAW layer output (statistics slots of a dgrad epilogue,
   // bn_bwd_finalize_slots); centred and scaled here, once, in double
-  if (mean != nullptr) sg = (sg - static_cast<double>(mean[c]) * sb) * static_cast<double>(invstd[c]);
-  dbeta[c] += static_cast<float>(sb);
-  dgamma[c] += static_cast<float>(sg);
+  if (mean != nullptr) s[1] = (s[1] - static_cast<double>(mean[c]) * s[0]) * static_cast<double>(invstd[c]);
+  dbeta[c] += static_cast<float>(s[0]);
+  dgamma[c] += static_cast<float>(s[1]);
+}
+
+__global__ void __launch_bounds__(256)
+colsum_final_kernel(const float* __restrict__ partial, int blocks, float* __restrict__ out, int C) {
+  pdl_prologue();
+  double s[1];
+  if (ordered_slot_sum<1>(partial, blocks, C, s)) out[blockIdx.x * 8 + (threadIdx.x & 7)] = static_cast<float>(s[0]);
+}
+void colsum_finalize(const float* partial, int blocks, float* out, int C, cudaStream_t st) {
+  launch_kernel(colsum_final_kernel, (C + 7) / 8, 256, 0, st, partial, blocks, out, C);
+  ARGUS_CUDA(cudaGetLastError());
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// Shared-memory ring versions of the two batch-norm backward passes (default; ARGUS_BN_RING=0 selects the register
-// versions above). A producer warp streams 8 KB slices of dy / x (/ out or the bit mask) into a ring of stages with
-// 1-D bulk copies (TMA) that complete on mbarriers; eight consumer warps read their 16-byte vectors from the landed
-// stage, release it, and do the math. The bytes in flight per SM are set by the ring (2 CTAs x 6 stages x 16 KB)
-// instead of by the registers the loads of one loop iteration can hold (1024 threads x 64 B), which is what kept the
-// register versions at 55-70 % of the HBM copy bandwidth.
+// Batch-norm apply and backward passes through a shared-memory ring. A producer warp streams 8 KB slices of each input
+// tensor into a ring of stages with 1-D bulk copies (TMA) that complete on mbarriers; eight consumer warps read their
+// 16-byte vectors from the landed stage, release it, and do the math. The bytes in flight per SM are set by the ring
+// (2 CTAs x 5 stages x 16 KB) instead of by the registers the loads of one loop iteration can hold (1024 threads x
+// 64 B), which is what held earlier register-streaming kernels of these passes at 55-70 % of the HBM copy bandwidth
+// (DESIGN.md section 4). Bulk copies and 16-byte vectors need every tensor 16-byte aligned: bn_check_aligned rejects
+// anything else on the host.
 // ------------------------------------------------------------------------------------------------------------
-constexpr int kRingVec = 512;   // uint4 per tensor per stage: two per consumer thread
-template <int MASK>
-struct BnRing {
-  static constexpr int kTensorBytes = kRingVec * 16;
-  static constexpr int kExtraBytes = MASK == 2 ? kTensorBytes : (MASK == 3 ? kRingVec : 0);
-  static constexpr int kStageBytes = 2 * kTensorBytes + kExtraBytes;
-  // 2 CTAs x 5 stages x 16 KB in flight per SM is far more than HBM latency needs; stopping at ~80 KB per CTA leaves
-  // room for one CTA of the (ALU-bound, 41 KB) augmentation kernel of the next batch to share the SM
-  static constexpr int kStages = MASK == 2 ? 3 : 5;
+void bn_check_aligned(const void* a, const void* b, const void* c, const void* d) {
+  for (const void* p : {a, b, c, d})
+    ARGUS_CHECK((reinterpret_cast<uintptr_t>(p) & 15u) == 0, "batch norm: every tensor must be 16-byte aligned");
+}
+
+constexpr int kRingVec = 512;                 // vectors per tensor per stage: two per consumer thread
+constexpr int kRingTensor = kRingVec * 16;    // bytes of one bf16 tensor per stage
+constexpr int kRingThreads = 288;             // 8 consumer warps + 1 producer warp
+// A stage holds up to three tensors of B0, B1, B2 bytes (kRingTensor: bf16 vectors, kRingVec: a ReLU bit mask, one byte
+// per vector, 0: absent); the full / empty mbarriers of all stages follow the stages.
+template <int B0, int B1, int B2, int STAGES>
+struct Ring {
+  static constexpr int kBytes0 = B0, kBytes1 = B1, kBytes2 = B2;
+  static constexpr int kStages = STAGES;
+  static constexpr int kStageBytes = B0 + B1 + B2;
   static constexpr int kOffBars = kStages * kStageBytes;
   static constexpr int kTotal = kOffBars + 2 * kStages * 8;
-  static_assert(kStages * kStageBytes >= 16 * 256 * 4, "the block reduction reuses the ring memory");
+  static_assert(kOffBars >= 8 * 16 * 32 * 4, "the block reduction reuses the ring memory");
 };
-constexpr int kRingThreads = 288;   // 8 consumer warps + 1 producer warp
-
+// 2 CTAs x 5 stages x 16 KB in flight per SM is far more than HBM latency needs; stopping at ~80 KB per CTA leaves room
+// for one CTA of the (ALU-bound, 41 KB) augmentation kernel of the next batch to share the SM.
+// Backward: dy, x (+ the block output for MASK 2, + the ReLU bit mask for MASK 3).
 template <int MASK>
-__device__ __forceinline__ void bn_ring_producer(uint32_t sbase, const uint4* dy, const uint4* x, const uint4* out,
-                                                 int64_t nfull) {
-  using R = BnRing<MASK>;
-  int s = 0;
-  uint32_t ph = 0;
-  for (int64_t c = blockIdx.x; c < nfull; c += gridDim.x) {
-    const uint32_t full = sbase + R::kOffBars + 8u * s, empty = sbase + R::kOffBars + 8u * (R::kStages + s);
-    mbar_wait(empty, ph ^ 1);
-    mbar_arrive_expect_tx(full, R::kStageBytes);
-    const uint32_t dst = sbase + s * R::kStageBytes;
-    bulk_load_1d(dst, dy + c * kRingVec, R::kTensorBytes, full);
-    bulk_load_1d(dst + R::kTensorBytes, x + c * kRingVec, R::kTensorBytes, full);
-    if (MASK == 2) bulk_load_1d(dst + 2 * R::kTensorBytes, out + c * kRingVec, R::kTensorBytes, full);
-    if (MASK == 3)
-      bulk_load_1d(dst + 2 * R::kTensorBytes, reinterpret_cast<const uint8_t*>(out) + c * kRingVec, kRingVec, full);
-    if (++s == R::kStages) { s = 0; ph ^= 1; }
-  }
-}
+using BnRing = Ring<kRingTensor, kRingTensor, MASK == 2 ? kRingTensor : (MASK == 3 ? kRingVec : 0), MASK == 2 ? 3 : 5>;
+// Forward apply: x (+ residual).
+template <int RES>
+using ApplyRing = Ring<kRingTensor, RES ? kRingTensor : 0, 0, RES ? 5 : 10>;
+
 __device__ __forceinline__ void bn_ring_init(uint32_t sbase, int off_bars, int stages) {
   if (threadIdx.x == 0) {
     for (int s = 0; s < stages; ++s) {
@@ -629,7 +422,103 @@ __device__ __forceinline__ void bn_ring_init(uint32_t sbase, int off_bars, int s
   }
   __syncthreads();
 }
-// masked gradient of eight channels (see bn_bwd_reduce_kernel)
+// producer (one thread): the full stages c = blockIdx.x, blockIdx.x + gridDim.x, ... of tensors t0, t1, t2
+template <class R>
+__device__ __forceinline__ void ring_produce(uint32_t sbase, const void* t0, const void* t1, const void* t2,
+                                             int64_t nvec) {
+  const int64_t nfull = nvec / kRingVec;
+  int s = 0;
+  uint32_t ph = 0;
+  for (int64_t c = blockIdx.x; c < nfull; c += gridDim.x) {
+    const uint32_t full = sbase + R::kOffBars + 8u * s, empty = sbase + R::kOffBars + 8u * (R::kStages + s);
+    mbar_wait(empty, ph ^ 1);
+    mbar_arrive_expect_tx(full, R::kStageBytes);
+    const uint32_t dst = sbase + s * R::kStageBytes;
+    bulk_load_1d(dst, static_cast<const uint8_t*>(t0) + c * R::kBytes0, R::kBytes0, full);
+    if (R::kBytes1) bulk_load_1d(dst + R::kBytes0, static_cast<const uint8_t*>(t1) + c * R::kBytes1, R::kBytes1, full);
+    if (R::kBytes2)
+      bulk_load_1d(dst + R::kBytes0 + R::kBytes1, static_cast<const uint8_t*>(t2) + c * R::kBytes2, R::kBytes2, full);
+    if (++s == R::kStages) { s = 0; ph ^= 1; }
+  }
+}
+// vector i of a tensor with BYTES bytes per stage: 16 bytes, one bit-mask byte (in .x), or zeros when absent
+template <int BYTES>
+__device__ __forceinline__ uint4 ring_elem(const void* p, int64_t i) {
+  static_assert(BYTES == kRingTensor || BYTES == kRingVec || BYTES == 0, "ring tensors are bf16 vectors or bit masks");
+  uint4 v = make_uint4(0, 0, 0, 0);
+  if (BYTES == kRingTensor) v = static_cast<const uint4*>(p)[i];
+  if (BYTES == kRingVec) v.x = static_cast<const uint8_t*>(p)[i];
+  return v;
+}
+// consumers (threads 0..255): for each full stage of this block, wait until it has landed, take thread t's two vectors
+// of every tensor, release the stage, then body(i, v0, v1, v2) for i = c * kRingVec + t and i + 256. Block 0 then does
+// the ragged tail (< one stage) straight from global memory.
+template <class R, class Body>
+__device__ __forceinline__ void ring_consume(const uint8_t* smem, uint32_t sbase, const void* t0, const void* t1,
+                                             const void* t2, int64_t nvec, Body&& body) {
+  const int t = threadIdx.x;
+  const int64_t nfull = nvec / kRingVec;
+  int s = 0;
+  uint32_t ph = 0;
+  for (int64_t c = blockIdx.x; c < nfull; c += gridDim.x) {
+    mbar_wait(sbase + R::kOffBars + 8u * s, ph);
+    const uint8_t* s0 = smem + s * R::kStageBytes;
+    const uint8_t* s1 = s0 + R::kBytes0;
+    const uint8_t* s2 = s1 + R::kBytes1;
+    const uint4 a0 = ring_elem<R::kBytes0>(s0, t), a1 = ring_elem<R::kBytes0>(s0, t + 256);
+    const uint4 b0 = ring_elem<R::kBytes1>(s1, t), b1 = ring_elem<R::kBytes1>(s1, t + 256);
+    const uint4 e0 = ring_elem<R::kBytes2>(s2, t), e1 = ring_elem<R::kBytes2>(s2, t + 256);
+    __syncwarp();
+    if ((t & 31) == 0) mbar_arrive(sbase + R::kOffBars + 8u * (R::kStages + s));   // stage free: data is in registers
+    const int64_t i0 = c * kRingVec + t;
+    body(i0, a0, b0, e0);
+    body(i0 + 256, a1, b1, e1);
+    if (++s == R::kStages) { s = 0; ph ^= 1; }
+  }
+  if (blockIdx.x == 0) {
+    for (int64_t i = nfull * kRingVec + t; i < nvec; i += 256)
+      body(i, ring_elem<R::kBytes0>(t0, i), ring_elem<R::kBytes1>(t1, i), ring_elem<R::kBytes2>(t2, i));
+  }
+}
+// Per-block column sums of NV values per thread (NV / 8 series of the eight channels of octet t mod lanes) into
+// partial[blockIdx.x][NV / 8][C]: warp shuffles across the lanes of a warp that share an octet (lanes < 32), then one
+// pass over the eight consumer warps through [warp][value][lane] in the ring memory, which is free once every stage is
+// consumed. Fixed order -> deterministic. Called by all kRingThreads threads; the producer warp's values are ignored.
+template <int NV>
+__device__ __forceinline__ void ring_block_sums(float (&v)[NV], uint8_t* smem, int lanes, float* partial, int C) {
+  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  if (warp < 8) {
+    for (int o = 16; o >= lanes; o >>= 1) {
+#pragma unroll
+      for (int k = 0; k < NV; ++k) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
+    }
+  }
+  __syncthreads();
+  float (*red)[NV][32] = reinterpret_cast<float (*)[NV][32]>(smem);
+  if (warp < 8) {
+#pragma unroll
+    for (int k = 0; k < NV; ++k) red[warp][k][lane] = v[k];
+  }
+  __syncthreads();
+  // thread t < lanes owns octet t; the warps holding it are w = (t / 32) + j * (lanes / 32) for lanes >= 32, all eight
+  // warps (lane t) for lanes < 32
+  if (t < lanes) {
+    const int wstep = lanes >= 32 ? lanes / 32 : 1;
+    const int w0 = lanes >= 32 ? t / 32 : 0;
+    float sum[NV];
+#pragma unroll
+    for (int k = 0; k < NV; ++k) sum[k] = 0.f;
+    for (int w = w0; w < 8; w += wstep) {   // the NV sums are independent chains: their loads overlap
+#pragma unroll
+      for (int k = 0; k < NV; ++k) sum[k] += red[w][k][lane];
+    }
+#pragma unroll
+    for (int k = 0; k < NV; ++k) partial[(static_cast<size_t>(blockIdx.x) * (NV / 8) + k / 8) * C + t * 8 + k % 8] = sum[k];
+  }
+}
+
+// Masked gradient of eight channels. MASK 0: no ReLU after the batch norm; 1: ReLU right after it (mask recomputed from
+// x); 2: ReLU after a residual add (mask = block output > 0); 3: like 2, from the ReLU bit mask (byte in ov4.x).
 template <int MASK>
 __device__ __forceinline__ F8 bn_masked_grad(const F8& d, const F8& xv, const uint4& ov4, const F8& sc, const F8& sh) {
   F8 g = d;
@@ -646,206 +535,20 @@ __device__ __forceinline__ F8 bn_masked_grad(const F8& d, const F8& xv, const ui
   }
   return g;
 }
-
-template <int MASK>
-__global__ void __launch_bounds__(kRingThreads, 2)
-bn_bwd_reduce_ring_kernel(const uint4* __restrict__ dy, const uint4* __restrict__ x, const uint4* __restrict__ out,
-                          const float* __restrict__ scale, const float* __restrict__ shift,
-                          const float* __restrict__ mean, const float* __restrict__ invstd,
-                          float* __restrict__ partial, int64_t nvec, int cvec) {
-  pdl_prologue();
-  using R = BnRing<MASK>;
-  extern __shared__ __align__(128) uint8_t ring_smem[];
-  const uint32_t sbase = smem_u32(ring_smem);
-  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  bn_ring_init(sbase, R::kOffBars, R::kStages);
-  const int64_t nfull = nvec / kRingVec;
-  const int lanes = cvec < 256 ? cvec : 256;
-  const int oc = t & (lanes - 1);
-  const int c0 = oc * 8;
-  float a_dy[8], a_dyx[8];
+// dx = sc * (g - db/M - xhat * dg/M) with xhat = (x - mu) * is   ==   sc*g + k1*x + k0 (per-channel pointers at c0)
+__device__ __forceinline__ void bn_dx_coeffs(const F8& sc, const float* mean, const float* invstd, const float* dgamma,
+                                             const float* dbeta, float inv_rows, F8& k0, F8& k1) {
+  const F8 mu = load8f(mean), is = load8f(invstd), dg = load8f(dgamma), db = load8f(dbeta);
 #pragma unroll
-  for (int k = 0; k < 8; ++k) a_dy[k] = a_dyx[k] = 0.f;
-  if (warp == 8) {
-    if (lane == 0) bn_ring_producer<MASK>(sbase, dy, x, out, nfull);
-  } else {
-    F8 sc, sh;
-    if (MASK == 1) { sc = load8f(scale + c0); sh = load8f(shift + c0); }
-    auto body = [&](const uint4& dyv, const uint4& xv4, const uint4& ov4) {
-      const F8 d = unpack8(dyv);
-      const F8 xv = unpack8(xv4);
-      const F8 g = bn_masked_grad<MASK>(d, xv, ov4, sc, sh);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) {
-        a_dy[k] += g.v[k];
-        a_dyx[k] = fmaf(g.v[k], xv.v[k], a_dyx[k]);
-      }
-    };
-    int s = 0;
-    uint32_t ph = 0;
-    for (int64_t c = blockIdx.x; c < nfull; c += gridDim.x) {
-      mbar_wait(sbase + R::kOffBars + 8u * s, ph);
-      const uint8_t* st = ring_smem + s * R::kStageBytes;
-      const uint4* sd = reinterpret_cast<const uint4*>(st);
-      const uint4* sx = reinterpret_cast<const uint4*>(st + R::kTensorBytes);
-      const uint4 d0 = sd[t], d1 = sd[t + 256], x0 = sx[t], x1 = sx[t + 256];
-      uint4 o0 = make_uint4(0, 0, 0, 0), o1 = o0;
-      if (MASK == 2) {
-        const uint4* so = reinterpret_cast<const uint4*>(st + 2 * R::kTensorBytes);
-        o0 = so[t]; o1 = so[t + 256];
-      }
-      if (MASK == 3) {
-        const uint8_t* sb = st + 2 * R::kTensorBytes;
-        o0.x = sb[t]; o1.x = sb[t + 256];
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(sbase + R::kOffBars + 8u * (R::kStages + s));   // stage free: data is in registers
-      body(d0, x0, o0);
-      body(d1, x1, o1);
-      if (++s == R::kStages) { s = 0; ph ^= 1; }
-    }
-    if (blockIdx.x == 0) {
-      // ragged tail (< one stage): straight from global memory
-      const uint8_t* bits = reinterpret_cast<const uint8_t*>(out);
-      for (int64_t i = nfull * kRingVec + t; i < nvec; i += 256) {
-        uint4 o0 = make_uint4(0, 0, 0, 0);
-        if (MASK == 2) o0 = ldg_stream(out + i);
-        if (MASK == 3) o0.x = __ldg(bits + i);
-        body(ldg_stream(dy + i), ldg_stream(x + i), o0);
-      }
-    }
-  }
-  // Block reduction over the threads that share a channel octet (t = oc mod lanes): warp shuffles across the lanes of
-  // a warp that share it (lanes < 32), then one shared-memory pass across the eight warps. Fixed order -> deterministic.
-  float v[16];
-  {
-    F8 mu, is;
-    if (t < 256) { mu = load8f(mean + c0); is = load8f(invstd + c0); }
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      v[k] = a_dy[k];
-      v[8 + k] = t < 256 ? (a_dyx[k] - mu.v[k] * a_dy[k]) * is.v[k] : 0.f;
-    }
-  }
-  if (warp < 8) {
-    for (int o = 16; o >= lanes; o >>= 1) {
-#pragma unroll
-      for (int k = 0; k < 16; ++k) v[k] += __shfl_xor_sync(0xffffffffu, v[k], o);
-    }
-  }
-  __syncthreads();   // every stage has been consumed: the ring memory becomes the reduction scratch
-  float (*red)[16][32] = reinterpret_cast<float (*)[16][32]>(ring_smem);   // [warp][value][lane]
-  if (warp < 8) {
-#pragma unroll
-    for (int k = 0; k < 16; ++k) red[warp][k][lane] = v[k];
-  }
-  __syncthreads();
-  // thread t < lanes owns octet t; the warps holding it are w = (t / 32) + j * (lanes / 32) for lanes >= 32, all eight
-  // warps (lane t) for lanes < 32
-  if (t < lanes) {
-    const int wstep = lanes >= 32 ? lanes / 32 : 1;
-    const int w0 = lanes >= 32 ? t / 32 : 0;
-    const int ln = t & 31;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      float s0 = 0.f, s1 = 0.f;
-      for (int w = w0; w < 8; w += wstep) {
-        s0 += red[w][k][ln];
-        s1 += red[w][8 + k][ln];
-      }
-      partial[(static_cast<size_t>(blockIdx.x) * 2 + 0) * (cvec * 8) + c0 + k] = s0;
-      partial[(static_cast<size_t>(blockIdx.x) * 2 + 1) * (cvec * 8) + c0 + k] = s1;
-    }
+  for (int k = 0; k < 8; ++k) {
+    const float c2 = sc.v[k] * dg.v[k] * inv_rows * is.v[k];
+    k1.v[k] = -c2;
+    k0.v[k] = fmaf(c2, mu.v[k], -sc.v[k] * db.v[k] * inv_rows);
   }
 }
 
-template <int MASK>
-__global__ void __launch_bounds__(kRingThreads, 2)
-bn_bwd_apply_ring_kernel(uint4* __restrict__ dy, const uint4* __restrict__ x, const uint4* __restrict__ out,
-                         const float* __restrict__ scale, const float* __restrict__ shift,
-                         const float* __restrict__ mean, const float* __restrict__ invstd,
-                         const float* __restrict__ dgamma, const float* __restrict__ dbeta, uint4* __restrict__ dx,
-                         int64_t nvec, int cvec, float inv_rows) {
-  pdl_prologue();
-  using R = BnRing<MASK>;
-  extern __shared__ __align__(128) uint8_t ring_smem[];
-  const uint32_t sbase = smem_u32(ring_smem);
-  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  bn_ring_init(sbase, R::kOffBars, R::kStages);
-  const int64_t nfull = nvec / kRingVec;
-  if (warp == 8) {
-    if (lane == 0) bn_ring_producer<MASK>(sbase, dy, x, out, nfull);
-    return;
-  }
-  const int c0 = (t & ((cvec < 256 ? cvec : 256) - 1)) * 8;
-  const F8 sc = load8f(scale + c0);
-  F8 sh;
-  if (MASK == 1) sh = load8f(shift + c0);
-  F8 k0, k1;
-  {
-    const F8 mu = load8f(mean + c0), is = load8f(invstd + c0), dg = load8f(dgamma + c0), db = load8f(dbeta + c0);
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const float c2 = sc.v[k] * dg.v[k] * inv_rows * is.v[k];
-      k1.v[k] = -c2;
-      k0.v[k] = fmaf(c2, mu.v[k], -sc.v[k] * db.v[k] * inv_rows);
-    }
-  }
-  auto body = [&](int64_t i, const uint4& dyv, const uint4& xv4, const uint4& ov4) {
-    const F8 d = unpack8(dyv);
-    const F8 xv = unpack8(xv4);
-    const F8 g = bn_masked_grad<MASK>(d, xv, ov4, sc, sh);
-    F8 r;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) r.v[k] = fmaf(sc.v[k], g.v[k], fmaf(k1.v[k], xv.v[k], k0.v[k]));
-    dx[i] = pack8(r);
-    if (MASK == 2) dy[i] = pack8(g);
-  };
-  int s = 0;
-  uint32_t ph = 0;
-  for (int64_t c = blockIdx.x; c < nfull; c += gridDim.x) {
-    mbar_wait(sbase + R::kOffBars + 8u * s, ph);
-    const uint8_t* st = ring_smem + s * R::kStageBytes;
-    const uint4* sd = reinterpret_cast<const uint4*>(st);
-    const uint4* sx = reinterpret_cast<const uint4*>(st + R::kTensorBytes);
-    const uint4 d0 = sd[t], d1 = sd[t + 256], x0 = sx[t], x1 = sx[t + 256];
-    uint4 o0 = make_uint4(0, 0, 0, 0), o1 = o0;
-    if (MASK == 2) {
-      const uint4* so = reinterpret_cast<const uint4*>(st + 2 * R::kTensorBytes);
-      o0 = so[t]; o1 = so[t + 256];
-    }
-    if (MASK == 3) {
-      const uint8_t* sb = st + 2 * R::kTensorBytes;
-      o0.x = sb[t]; o1.x = sb[t + 256];
-    }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(sbase + R::kOffBars + 8u * (R::kStages + s));
-    const int64_t i0 = c * kRingVec + t;
-    body(i0, d0, x0, o0);
-    body(i0 + 256, d1, x1, o1);
-    if (++s == R::kStages) { s = 0; ph ^= 1; }
-  }
-  if (blockIdx.x == 0) {
-    const uint8_t* bits = reinterpret_cast<const uint8_t*>(out);
-    for (int64_t i = nfull * kRingVec + t; i < nvec; i += 256) {
-      uint4 o0 = make_uint4(0, 0, 0, 0);
-      if (MASK == 2) o0 = ldg_stream(out + i);
-      if (MASK == 3) o0.x = __ldg(bits + i);
-      body(i, dy[i], ldg_stream(x + i), o0);
-    }
-  }
-}
-
-// Forward batch-norm apply through the same ring: x (+ residual) stream in, y (+ ReLU bits, + per-block column sums) out.
-template <int RES>
-struct ApplyRing {
-  static constexpr int kTensorBytes = kRingVec * 16;
-  static constexpr int kStageBytes = RES ? 2 * kTensorBytes : kTensorBytes;
-  static constexpr int kStages = RES ? 5 : 10;   // ~80 KB per CTA (see BnRing)
-  static constexpr int kOffBars = kStages * kStageBytes;
-  static constexpr int kTotal = kOffBars + 2 * kStages * 8;
-  static_assert(kStages * kStageBytes >= 8 * 16 * 32 * 4, "the block reduction reuses the ring memory");
-};
+// y = [relu](x*scale+shift [+ res | + res*rscale+rshift]) (+ ReLU bits, + per-block column sums of the stored y).
+// RES: 0 none, 1 plain residual, 2 residual with its own scale/shift (downsample branch).
 template <int RES, bool SUM>
 __global__ void __launch_bounds__(kRingThreads, 2)
 bn_apply_ring_kernel(const uint4* __restrict__ x, const float* __restrict__ scale, const float* __restrict__ shift,
@@ -858,32 +561,19 @@ bn_apply_ring_kernel(const uint4* __restrict__ x, const float* __restrict__ scal
   const uint32_t sbase = smem_u32(ring_smem);
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   bn_ring_init(sbase, R::kOffBars, R::kStages);
-  const int64_t nfull = nvec / kRingVec;
   const int lanes = cvec < 256 ? cvec : 256;
   const int c0 = (t & (lanes - 1)) * 8;
   F8 acc;
 #pragma unroll
   for (int k = 0; k < 8; ++k) acc.v[k] = 0.f;
   if (warp == 8) {
-    if (lane == 0) {
-      int s = 0;
-      uint32_t ph = 0;
-      for (int64_t c = blockIdx.x; c < nfull; c += gridDim.x) {
-        const uint32_t full = sbase + R::kOffBars + 8u * s, empty = sbase + R::kOffBars + 8u * (R::kStages + s);
-        mbar_wait(empty, ph ^ 1);
-        mbar_arrive_expect_tx(full, R::kStageBytes);
-        const uint32_t dst = sbase + s * R::kStageBytes;
-        bulk_load_1d(dst, x + c * kRingVec, R::kTensorBytes, full);
-        if (RES) bulk_load_1d(dst + R::kTensorBytes, res + c * kRingVec, R::kTensorBytes, full);
-        if (++s == R::kStages) { s = 0; ph ^= 1; }
-      }
-    }
+    if (lane == 0) ring_produce<R>(sbase, x, res, nullptr, nvec);
     if (!SUM) return;
   } else {
     const F8 sc = load8f(scale + c0), sh = load8f(shift + c0);
     F8 rs, rb;
     if (RES == 2) { rs = load8f(rscale + c0); rb = load8f(rshift + c0); }
-    auto one = [&](int64_t i, const uint4& xq, const uint4& rq) {
+    auto one = [&](int64_t i, const uint4& xq, const uint4& rq, const uint4&) {
       const F8 xv = unpack8(xq);
       F8 o;
 #pragma unroll
@@ -910,116 +600,131 @@ bn_apply_ring_kernel(const uint4* __restrict__ x, const float* __restrict__ scal
         for (int k = 0; k < 8; ++k) acc.v[k] += r.v[k];
       }
     };
-    int s = 0;
-    uint32_t ph = 0;
-    for (int64_t c = blockIdx.x; c < nfull; c += gridDim.x) {
-      mbar_wait(sbase + R::kOffBars + 8u * s, ph);
-      const uint8_t* st = ring_smem + s * R::kStageBytes;
-      const uint4* sx = reinterpret_cast<const uint4*>(st);
-      const uint4 x0 = sx[t], x1 = sx[t + 256];
-      uint4 r0 = make_uint4(0, 0, 0, 0), r1 = r0;
-      if (RES) {
-        const uint4* sr = reinterpret_cast<const uint4*>(st + R::kTensorBytes);
-        r0 = sr[t]; r1 = sr[t + 256];
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(sbase + R::kOffBars + 8u * (R::kStages + s));
-      const int64_t i0 = c * kRingVec + t;
-      one(i0, x0, r0);
-      one(i0 + 256, x1, r1);
-      if (++s == R::kStages) { s = 0; ph ^= 1; }
-    }
-    if (blockIdx.x == 0) {
-      for (int64_t i = nfull * kRingVec + t; i < nvec; i += 256) {
-        uint4 r0 = make_uint4(0, 0, 0, 0);
-        if (RES) r0 = ldg_stream(res + i);
-        one(i, ldg_stream(x + i), r0);
-      }
-    }
+    ring_consume<R>(ring_smem, sbase, x, res, nullptr, nvec, one);
   }
-  if (SUM) {
-    // per-block column sums: same reduction scheme as bn_bwd_reduce_ring_kernel
-    if (warp < 8) {
-      for (int o = 16; o >= lanes; o >>= 1) {
+  if (SUM) ring_block_sums<8>(acc.v, ring_smem, lanes, colsum_partial, cvec * 8);
+}
+
+template <int MASK>
+__global__ void __launch_bounds__(kRingThreads, 2)
+bn_bwd_reduce_ring_kernel(const uint4* __restrict__ dy, const uint4* __restrict__ x, const uint4* __restrict__ out,
+                          const float* __restrict__ scale, const float* __restrict__ shift,
+                          const float* __restrict__ mean, const float* __restrict__ invstd,
+                          float* __restrict__ partial, int64_t nvec, int cvec) {
+  pdl_prologue();
+  using R = BnRing<MASK>;
+  extern __shared__ __align__(128) uint8_t ring_smem[];
+  const uint32_t sbase = smem_u32(ring_smem);
+  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  bn_ring_init(sbase, R::kOffBars, R::kStages);
+  const int lanes = cvec < 256 ? cvec : 256;
+  const int c0 = (t & (lanes - 1)) * 8;
+  float a_dy[8], a_dyx[8];
 #pragma unroll
-        for (int k = 0; k < 8; ++k) acc.v[k] += __shfl_xor_sync(0xffffffffu, acc.v[k], o);
-      }
-    }
-    __syncthreads();
-    float (*red)[8][32] = reinterpret_cast<float (*)[8][32]>(ring_smem);   // [warp][value][lane]
-    if (warp < 8) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) red[warp][k][lane] = acc.v[k];
-    }
-    __syncthreads();
-    if (t < lanes) {
-      const int wstep = lanes >= 32 ? lanes / 32 : 1;
-      const int w0 = lanes >= 32 ? t / 32 : 0;
-      const int ln = t & 31;
+  for (int k = 0; k < 8; ++k) a_dy[k] = a_dyx[k] = 0.f;
+  if (warp == 8) {
+    if (lane == 0) ring_produce<R>(sbase, dy, x, out, nvec);
+  } else {
+    F8 sc, sh;
+    if (MASK == 1) { sc = load8f(scale + c0); sh = load8f(shift + c0); }
+    auto body = [&](int64_t, const uint4& dyv, const uint4& xv4, const uint4& ov4) {
+      const F8 xv = unpack8(xv4);
+      const F8 g = bn_masked_grad<MASK>(unpack8(dyv), xv, ov4, sc, sh);
 #pragma unroll
       for (int k = 0; k < 8; ++k) {
-        float s0 = 0.f;
-        for (int w = w0; w < 8; w += wstep) s0 += red[w][k][ln];
-        colsum_partial[static_cast<size_t>(blockIdx.x) * (cvec * 8) + t * 8 + k] = s0;
+        a_dy[k] += g.v[k];
+        a_dyx[k] = fmaf(g.v[k], xv.v[k], a_dyx[k]);   // sum g*x; centred and scaled by invstd once at the end
       }
+    };
+    ring_consume<R>(ring_smem, sbase, dy, x, out, nvec, body);
+  }
+  // partial[block][0][c] = sum g, partial[block][1][c] = sum g * xhat
+  float v[16];
+  {
+    F8 mu, is;
+    if (t < 256) { mu = load8f(mean + c0); is = load8f(invstd + c0); }
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      v[k] = a_dy[k];
+      v[8 + k] = t < 256 ? (a_dyx[k] - mu.v[k] * a_dy[k]) * is.v[k] : 0.f;
     }
   }
+  ring_block_sums<16>(v, ring_smem, lanes, partial, cvec * 8);
 }
-template <int RES, bool SUM>
-static void launch_bn_apply_ring_t(const uint4* x, const float* scale, const float* shift, const uint4* res,
-                                   const float* rscale, const float* rshift, int relu, uint4* y, uint8_t* bits,
-                                   float* colsum_partial, int64_t nvec, int cvec, cudaStream_t s) {
+
+template <int MASK>
+__global__ void __launch_bounds__(kRingThreads, 2)
+bn_bwd_apply_ring_kernel(uint4* __restrict__ dy, const uint4* __restrict__ x, const uint4* __restrict__ out,
+                         const float* __restrict__ scale, const float* __restrict__ shift,
+                         const float* __restrict__ mean, const float* __restrict__ invstd,
+                         const float* __restrict__ dgamma, const float* __restrict__ dbeta, uint4* __restrict__ dx,
+                         int64_t nvec, int cvec, float inv_rows) {
+  pdl_prologue();
+  using R = BnRing<MASK>;
+  extern __shared__ __align__(128) uint8_t ring_smem[];
+  const uint32_t sbase = smem_u32(ring_smem);
+  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
+  bn_ring_init(sbase, R::kOffBars, R::kStages);
+  if (warp == 8) {
+    if (lane == 0) ring_produce<R>(sbase, dy, x, out, nvec);
+    return;
+  }
+  const int c0 = (t & ((cvec < 256 ? cvec : 256) - 1)) * 8;
+  const F8 sc = load8f(scale + c0);
+  F8 sh;
+  if (MASK == 1) sh = load8f(shift + c0);
+  F8 k0, k1;
+  bn_dx_coeffs(sc, mean + c0, invstd + c0, dgamma + c0, dbeta + c0, inv_rows, k0, k1);
+  auto body = [&](int64_t i, const uint4& dyv, const uint4& xv4, const uint4& ov4) {
+    const F8 xv = unpack8(xv4);
+    const F8 g = bn_masked_grad<MASK>(unpack8(dyv), xv, ov4, sc, sh);
+    F8 r;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) r.v[k] = fmaf(sc.v[k], g.v[k], fmaf(k1.v[k], xv.v[k], k0.v[k]));
+    dx[i] = pack8(r);
+    if (MASK == 2) dy[i] = pack8(g);
+  };
+  ring_consume<R>(ring_smem, sbase, dy, x, out, nvec, body);
+}
+
+// one ring kernel instance with R::kTotal bytes of dynamic shared memory (opted in on its first launch)
+template <auto kKernel, class R, class... Args>
+static void launch_ring(int grid, cudaStream_t s, Args&&... args) {
   static const bool once = [] {
-    ARGUS_CUDA(cudaFuncSetAttribute(bn_apply_ring_kernel<RES, SUM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    ApplyRing<RES>::kTotal));
+    ARGUS_CUDA(cudaFuncSetAttribute(kKernel, cudaFuncAttributeMaxDynamicSharedMemorySize, R::kTotal));
     return true;
   }();
   (void)once;
-  launch_kernel(bn_apply_ring_kernel<RES, SUM>, bn_ring_grid(nvec), kRingThreads, ApplyRing<RES>::kTotal, s, 
-      x, scale, shift, res, rscale, rshift, relu, y, bits, colsum_partial, nvec, cvec);
-}
-static void launch_bn_apply_ring(const uint4* x, const float* scale, const float* shift, const uint4* res,
-                                 const float* rscale, const float* rshift, int relu, uint4* y, uint8_t* bits,
-                                 float* colsum_partial, int64_t nvec, int cvec, cudaStream_t s) {
-  if (colsum_partial != nullptr) launch_bn_apply_ring_t<0, true>(x, scale, shift, res, rscale, rshift, relu, y, bits, colsum_partial, nvec, cvec, s);
-  else if (res == nullptr) launch_bn_apply_ring_t<0, false>(x, scale, shift, res, rscale, rshift, relu, y, bits, nullptr, nvec, cvec, s);
-  else if (rscale == nullptr) launch_bn_apply_ring_t<1, false>(x, scale, shift, res, rscale, rshift, relu, y, bits, nullptr, nvec, cvec, s);
-  else launch_bn_apply_ring_t<2, false>(x, scale, shift, res, rscale, rshift, relu, y, bits, nullptr, nvec, cvec, s);
-}
-
-static bool bn_ring_enabled() {
-  static const bool on = [] { const char* e = getenv("ARGUS_BN_RING"); return !(e && e[0] == '0'); }();
-  return on;
+  launch_kernel(kKernel, grid, kRingThreads, R::kTotal, s, std::forward<Args>(args)...);
+  ARGUS_CUDA(cudaGetLastError());
 }
 static int bn_ring_grid(int64_t nvec) {
   return static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(nvec / kRingVec, 2LL * num_sms())));
 }
-template <int MASK>
-static void launch_bn_bwd_reduce_ring(const uint4* dy, const uint4* x, const uint4* out, const float* scale,
-                                      const float* shift, const float* mean, const float* invstd, float* partial,
-                                      int64_t nvec, int cvec, int grid, cudaStream_t s) {
-  static const bool once = [] {
-    ARGUS_CUDA(cudaFuncSetAttribute(bn_bwd_reduce_ring_kernel<MASK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    BnRing<MASK>::kTotal));
-    return true;
-  }();
-  (void)once;
-  launch_kernel(bn_bwd_reduce_ring_kernel<MASK>, grid, kRingThreads, BnRing<MASK>::kTotal, s, dy, x, out, scale, shift, mean, invstd,
-                                                                                  partial, nvec, cvec);
-}
-template <int MASK>
-static void launch_bn_bwd_apply_ring(uint4* dy, const uint4* x, const uint4* out, const float* scale,
-                                     const float* shift, const float* mean, const float* invstd, const float* dgamma,
-                                     const float* dbeta, uint4* dx, int64_t nvec, int cvec, float inv_rows,
-                                     cudaStream_t s) {
-  static const bool once = [] {
-    ARGUS_CUDA(cudaFuncSetAttribute(bn_bwd_apply_ring_kernel<MASK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    BnRing<MASK>::kTotal));
-    return true;
-  }();
-  (void)once;
-  launch_kernel(bn_bwd_apply_ring_kernel<MASK>, bn_ring_grid(nvec), kRingThreads, BnRing<MASK>::kTotal, s, 
-      dy, x, out, scale, shift, mean, invstd, dgamma, dbeta, dx, nvec, cvec, inv_rows);
+
+// number of per-block column-sum partials bn_apply writes (callers size and finalize the buffer with this)
+int bn_apply_grid(int64_t rows, int C) { return bn_ring_grid(rows * (C / 8)); }
+void bn_apply(const bf16* x, const float* scale, const float* shift, const bf16* res, const float* rscale,
+              const float* rshift, int relu, bf16* y, uint8_t* relu_bits, float* colsum_partial, int64_t rows, int C,
+              cudaStream_t s) {
+  bn_check_aligned(x, res, y, relu_bits);
+  ProfileScope prof("bn_apply", s, 0, static_cast<double>(rows) * C * (2 * (res ? 3 : 2) + (relu_bits ? 0.125 : 0.0)));
+  ARGUS_CHECK(C % 8 == 0 && is_pow2(C / 8) && C <= 2048, "bn_apply: C/8 must be a power of two <= 256");
+  ARGUS_CHECK(colsum_partial == nullptr || res == nullptr, "column sums are only produced by the plain (no residual) variant");
+  const int cvec = C / 8;
+  const int64_t nvec = rows * cvec;
+  const int grid = bn_ring_grid(nvec);
+  auto X = reinterpret_cast<const uint4*>(x);
+  auto R = reinterpret_cast<const uint4*>(res);
+  auto Y = reinterpret_cast<uint4*>(y);
+  if (colsum_partial != nullptr)
+    launch_ring<bn_apply_ring_kernel<0, true>, ApplyRing<0>>(grid, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, colsum_partial, nvec, cvec);
+  else if (res == nullptr)
+    launch_ring<bn_apply_ring_kernel<0, false>, ApplyRing<0>>(grid, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, colsum_partial, nvec, cvec);
+  else if (rscale == nullptr)
+    launch_ring<bn_apply_ring_kernel<1, false>, ApplyRing<1>>(grid, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, colsum_partial, nvec, cvec);
+  else
+    launch_ring<bn_apply_ring_kernel<2, false>, ApplyRing<2>>(grid, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, colsum_partial, nvec, cvec);
 }
 
 int64_t bn_bwd_scratch_elems() { return 4LL * num_sms() * 2 * 2048; }
@@ -1027,54 +732,31 @@ int64_t bn_bwd_scratch_elems() { return 4LL * num_sms() * 2 * 2048; }
 void bn_bwd_reduce(const bf16* dy, const bf16* x, const bf16* out, const float* scale, const float* shift,
                    const float* mean, const float* invstd, float* dgamma, float* dbeta, int64_t rows, int C,
                    int mask_mode, float* scratch, cudaStream_t s) {
+  bn_check_aligned(dy, x, out);
   ARGUS_CHECK(scratch != nullptr, "bn_bwd_reduce needs a scratch buffer");
   std::string fam = "bn_bwd_reduce";
   if (profile_enabled() && profile_detailed()) fam += ":R" + std::to_string(rows) + "_C" + std::to_string(C) + "_m" + std::to_string(mask_mode);
   ProfileScope prof(fam, s, 0, static_cast<double>(rows) * C * (mask_mode == 2 ? 6.0 : (mask_mode == 3 ? 4.125 : 4.0)));
   ARGUS_CHECK(C % 8 == 0 && is_pow2(C / 8) && C <= 2048, "bn_bwd_reduce: C/8 must be a power of two <= 256");
   const int cvec = C / 8;
-  const int lanes = std::min(cvec, 256);
-  const int row_lanes = 256 / lanes;
-  const int64_t row_groups = (rows + row_lanes - 1) / row_lanes;
-  const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>(row_groups, 4LL * num_sms())));
+  const int64_t nvec = rows * cvec;
+  const int grid = bn_ring_grid(nvec);
   auto DY = reinterpret_cast<const uint4*>(dy);
   auto X = reinterpret_cast<const uint4*>(x);
   auto O = reinterpret_cast<const uint4*>(out);
-  if (bn_ring_enabled() && aligned16(dy) && aligned16(x) && aligned16(out)) {
-    const int64_t nvec = rows * cvec;
-    const int rgrid = bn_ring_grid(nvec);
-    switch (mask_mode) {
-      case 0: launch_bn_bwd_reduce_ring<0>(DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec, rgrid, s); break;
-      case 1: launch_bn_bwd_reduce_ring<1>(DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec, rgrid, s); break;
-      case 2:
-        ARGUS_CHECK(out != nullptr, "mask_mode 2 needs the block output");
-        launch_bn_bwd_reduce_ring<2>(DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec, rgrid, s);
-        break;
-      case 3:
-        ARGUS_CHECK(out != nullptr, "mask_mode 3 needs the ReLU bit mask");
-        launch_bn_bwd_reduce_ring<3>(DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec, rgrid, s);
-        break;
-      default: throw Error("bad mask_mode");
-    }
-    ARGUS_CUDA(cudaGetLastError());
-    launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, scratch, rgrid, dgamma, dbeta, C, nullptr, nullptr);
-    ARGUS_CUDA(cudaGetLastError());
-    return;
-  }
   switch (mask_mode) {
-    case 0: launch_kernel(bn_bwd_reduce_kernel<0>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, scratch, rows, cvec); break;
-    case 1: launch_kernel(bn_bwd_reduce_kernel<1>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, scratch, rows, cvec); break;
+    case 0: launch_ring<bn_bwd_reduce_ring_kernel<0>, BnRing<0>>(grid, s, DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec); break;
+    case 1: launch_ring<bn_bwd_reduce_ring_kernel<1>, BnRing<1>>(grid, s, DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec); break;
     case 2:
       ARGUS_CHECK(out != nullptr, "mask_mode 2 needs the block output");
-      launch_kernel(bn_bwd_reduce_kernel<2>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, scratch, rows, cvec);
+      launch_ring<bn_bwd_reduce_ring_kernel<2>, BnRing<2>>(grid, s, DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec);
       break;
     case 3:
       ARGUS_CHECK(out != nullptr, "mask_mode 3 needs the ReLU bit mask");
-      launch_kernel(bn_bwd_reduce_kernel<3>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, scratch, rows, cvec);
+      launch_ring<bn_bwd_reduce_ring_kernel<3>, BnRing<3>>(grid, s, DY, X, O, scale, shift, mean, invstd, scratch, nvec, cvec);
       break;
     default: throw Error("bad mask_mode");
   }
-  ARGUS_CUDA(cudaGetLastError());
   launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, scratch, grid, dgamma, dbeta, C, nullptr, nullptr);
   ARGUS_CUDA(cudaGetLastError());
 }
@@ -1086,101 +768,27 @@ void bn_bwd_finalize_slots(const float* partial, int slots, const float* mean, c
   ARGUS_CUDA(cudaGetLastError());
 }
 
-template <int MASK>
-__global__ void __launch_bounds__(256)
-bn_bwd_apply_kernel(uint4* __restrict__ dy, const uint4* __restrict__ x, const uint4* __restrict__ out,
-                    const float* __restrict__ scale, const float* __restrict__ shift,
-                    const float* __restrict__ mean, const float* __restrict__ invstd,
-                    const float* __restrict__ dgamma, const float* __restrict__ dbeta, uint4* __restrict__ dx,
-                    int64_t nvec, int cvec, float inv_rows) {
-  pdl_prologue();
-  const int64_t tid = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;   // multiple of cvec
-  const int c0 = static_cast<int>(tid & (cvec - 1)) * 8;
-  const F8 sc = load8f(scale + c0), sh = load8f(shift + c0);
-  // dx = sc * (g - db/M - xhat * dg/M) with xhat = (x - mu) * is   ==   sc*g + k1*x + k0
-  F8 k0, k1;
-  {
-    const F8 mu = load8f(mean + c0), is = load8f(invstd + c0), dg = load8f(dgamma + c0), db = load8f(dbeta + c0);
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const float c2 = sc.v[k] * dg.v[k] * inv_rows * is.v[k];
-      k1.v[k] = -c2;
-      k0.v[k] = fmaf(c2, mu.v[k], -sc.v[k] * db.v[k] * inv_rows);
-    }
-  }
-  const uint8_t* bits = reinterpret_cast<const uint8_t*>(out);   // MASK == 3: one byte per channel octet
-  auto body = [&](int64_t i, const uint4& dyv, const uint4& xv4, const uint4& ov4) {
-    const F8 d = unpack8(dyv);
-    const F8 xv = unpack8(xv4);
-    F8 g = d;
-    if (MASK == 1) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) g.v[k] = fmaf(xv.v[k], sc.v[k], sh.v[k]) > 0.f ? d.v[k] : 0.f;
-    } else if (MASK == 2) {
-      const F8 o = unpack8(ov4);
-#pragma unroll
-      for (int k = 0; k < 8; ++k) g.v[k] = o.v[k] > 0.f ? d.v[k] : 0.f;
-    } else if (MASK == 3) {
-#pragma unroll
-      for (int k = 0; k < 8; ++k) g.v[k] = ((ov4.x >> k) & 1u) ? d.v[k] : 0.f;
-    }
-    F8 r;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) r.v[k] = fmaf(sc.v[k], g.v[k], fmaf(k1.v[k], xv.v[k], k0.v[k]));
-    dx[i] = pack8(r);
-    if (MASK == 2) dy[i] = pack8(g);
-  };
-  int64_t i = tid;
-  for (; i + stride < nvec; i += 2 * stride) {
-    const uint4 da = dy[i], dbv = dy[i + stride];
-    const uint4 xa = ldg_stream(x + i), xb = ldg_stream(x + i + stride);
-    uint4 oa = make_uint4(0, 0, 0, 0), ob = oa;
-    if (MASK == 2) { oa = ldg_stream(out + i); ob = ldg_stream(out + i + stride); }
-    if (MASK == 3) { oa.x = __ldg(bits + i); ob.x = __ldg(bits + i + stride); }
-    body(i, da, xa, oa);
-    body(i + stride, dbv, xb, ob);
-  }
-  for (; i < nvec; i += stride) {
-    uint4 oa = make_uint4(0, 0, 0, 0);
-    if (MASK == 2) oa = ldg_stream(out + i);
-    if (MASK == 3) oa.x = __ldg(bits + i);
-    body(i, dy[i], ldg_stream(x + i), oa);
-  }
-}
-
 void bn_bwd_apply(bf16* dy, const bf16* x, const bf16* out, const float* scale, const float* shift,
                   const float* mean, const float* invstd, const float* dgamma, const float* dbeta, bf16* dx,
                   int64_t rows, int C, int mask_mode, cudaStream_t s) {
+  bn_check_aligned(dy, x, out, dx);
   ProfileScope prof("bn_bwd_apply", s, 0, static_cast<double>(rows) * C * (mask_mode == 2 ? 10.0 : (mask_mode == 3 ? 6.125 : 6.0)));
   ARGUS_CHECK(C % 8 == 0 && is_pow2(C / 8) && C <= 2048, "bn_bwd_apply: C/8 must be a power of two <= 256");
   const int cvec = C / 8;
   const int64_t nvec = rows * cvec;
-  const int grid = grid_for(nvec, 256);
+  const int grid = bn_ring_grid(nvec);
   const float inv_rows = static_cast<float>(1.0 / static_cast<double>(rows));
   auto DY = reinterpret_cast<uint4*>(dy);
   auto X = reinterpret_cast<const uint4*>(x);
   auto O = reinterpret_cast<const uint4*>(out);
   auto DX = reinterpret_cast<uint4*>(dx);
-  if (bn_ring_enabled() && aligned16(dy) && aligned16(x) && aligned16(out) && aligned16(dx)) {
-    switch (mask_mode) {
-      case 0: launch_bn_bwd_apply_ring<0>(DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows, s); break;
-      case 1: launch_bn_bwd_apply_ring<1>(DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows, s); break;
-      case 2: launch_bn_bwd_apply_ring<2>(DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows, s); break;
-      case 3: launch_bn_bwd_apply_ring<3>(DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows, s); break;
-      default: throw Error("bad mask_mode");
-    }
-    ARGUS_CUDA(cudaGetLastError());
-    return;
-  }
   switch (mask_mode) {
-    case 0: launch_kernel(bn_bwd_apply_kernel<0>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
-    case 1: launch_kernel(bn_bwd_apply_kernel<1>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
-    case 2: launch_kernel(bn_bwd_apply_kernel<2>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
-    case 3: launch_kernel(bn_bwd_apply_kernel<3>, grid, 256, 0, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
+    case 0: launch_ring<bn_bwd_apply_ring_kernel<0>, BnRing<0>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
+    case 1: launch_ring<bn_bwd_apply_ring_kernel<1>, BnRing<1>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
+    case 2: launch_ring<bn_bwd_apply_ring_kernel<2>, BnRing<2>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
+    case 3: launch_ring<bn_bwd_apply_ring_kernel<3>, BnRing<3>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
     default: throw Error("bad mask_mode");
   }
-  ARGUS_CUDA(cudaGetLastError());
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1375,15 +983,7 @@ stem_pool_bn_bwd_kernel(const uint4* __restrict__ dpool, const uint2* __restrict
   const int c0 = cv * 8;
   const F8 sc = load8f(scale + c0), sh = load8f(shift + c0);
   F8 k0, k1;
-  if (APPLY) {
-    const F8 mu = load8f(mean + c0), is = load8f(invstd + c0), dg = load8f(dgamma + c0), db = load8f(dbeta + c0);
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-      const float c2 = sc.v[k] * dg.v[k] * inv_rows * is.v[k];
-      k1.v[k] = -c2;
-      k0.v[k] = fmaf(c2, mu.v[k], -sc.v[k] * db.v[k] * inv_rows);
-    }
-  }
+  if (APPLY) bn_dx_coeffs(sc, mean + c0, invstd + c0, dgamma + c0, dbeta + c0, inv_rows, k0, k1);
   float a_dy[8], a_dyx[8];
 #pragma unroll
   for (int k = 0; k < 8; ++k) a_dy[k] = a_dyx[k] = 0.f;
@@ -1440,9 +1040,7 @@ stem_pool_bn_bwd_kernel(const uint4* __restrict__ dpool, const uint2* __restrict
             for (int k = 0; k < 8; ++k)
               if (code_of(wi[dy][dxx], k) == code) g.v[k] += wd[dy][dxx].v[k];
           }
-#pragma unroll
-        for (int k = 0; k < 8; ++k)
-          if (!(fmaf(xv.v[k], sc.v[k], sh.v[k]) > 0.f)) g.v[k] = 0.f;
+        g = bn_masked_grad<1>(g, xv, uint4{}, sc, sh);
         if (APPLY) {
           F8 r;
 #pragma unroll

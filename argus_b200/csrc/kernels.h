@@ -63,6 +63,11 @@ void bn_finalize(const float* partial, int slots, double count, const float* gam
 // eval: running statistics -> scale/shift
 void bn_fold_eval(const float* gamma, const float* beta, const float* running_mean, const float* running_var,
                   float eps, float* scale, float* shift, int C, cudaStream_t s);
+// bn_apply, bn_bwd_reduce and bn_bwd_apply stream their tensors with 16-byte vectors and bulk copies: every tensor
+// pointer they take (x, res, y, relu_bits; dy, x, out, dx) must be 16-byte aligned. They call this before launching
+// anything; it throws for a misaligned pointer (nullptr passes). A caller of several passes checks all their tensors
+// up front with it, so that none of the passes runs.
+void bn_check_aligned(const void* a, const void* b, const void* c, const void* d = nullptr);
 // y = [relu]( x*scale+shift  [+ res]  or  [+ res*rscale+rshift] )
 // relu_bits (optional): [rows][C/8] bytes, bit k of byte j = (pre-ReLU value of channel 8j+k > 0). The backward pass
 // reads this mask instead of the whole bf16 output (1/16 of the bytes).

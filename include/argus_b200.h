@@ -149,16 +149,19 @@ int argus_stem_dgrad(const void* dy, const void* w, float* dx, int N, int H, int
 int argus_bn_finalize(const float* partial, int slots, double count, const float* gamma, const float* beta,
                       float* running_mean, float* running_var, float momentum, float eps, float* scale, float* shift,
                       float* save_mean, float* save_invstd, int C, void* stream);
-/* y = [relu](x*scale+shift [+ res | + res*rscale+rshift]) */
+/* y = [relu](x*scale+shift [+ res | + res*rscale+rshift]). x, res and y must be 16-byte aligned: a misaligned pointer
+ * is an error, reported before anything runs. */
 int argus_bn_apply(const void* x, const float* scale, const float* shift, const void* res, const float* rscale,
                    const float* rshift, int relu, void* y, int64_t rows, int C, void* stream);
 /* same, and also writes the ReLU mask of the result: relu_bits[rows][C/8] bytes, bit k of byte j = (channel 8j+k of
- * the pre-ReLU value > 0). The backward pass reads these bits instead of the bf16 output (1/16 of the bytes). */
+ * the pre-ReLU value > 0). The backward pass reads these bits instead of the bf16 output (1/16 of the bytes).
+ * relu_bits must be 16-byte aligned too. */
 int argus_bn_apply_bits(const void* x, const float* scale, const float* shift, const void* res, const float* rscale,
                         const float* rshift, int relu, void* y, void* relu_bits, int64_t rows, int C, void* stream);
 /* BN (+ReLU) backward. mask_mode 0: no ReLU; 1: ReLU right after the BN; 2: ReLU after a residual add (mask = out > 0,
  * dy is overwritten with the masked gradient); 3: like 2 but `out` is the relu_bits mask of argus_bn_apply_bits and dy
- * is left untouched. dgamma / dbeta are ADDED to (caller zeroes); dx = d loss / d x. */
+ * is left untouched. dgamma / dbeta are ADDED to (caller zeroes); dx = d loss / d x. dy, x, out and dx must be 16-byte
+ * aligned: a misaligned pointer is an error, reported before dgamma / dbeta are touched. */
 int argus_bn_backward(void* dy, const void* x, const void* out, const float* scale, const float* shift,
                       const float* mean, const float* invstd, float* dgamma, float* dbeta, void* dx, int64_t rows,
                       int C, int mask_mode, void* stream);

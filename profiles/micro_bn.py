@@ -1,6 +1,6 @@
 """Micro-benchmark: batch-norm backward (reduce + apply) and the statistics-carrying wide 1x1 forward convolutions at
 the bench shapes (B=256 pairs -> 512 images), through the C ABI, per kernel family with the library's own CUDA-event
-profiler. A/B switches are environment variables read by the library (ARGUS_BN_RING=0 -> register versions).
+profiler. A/B: MICRO_LIB=path runs another build of the library (e.g. the parent commit's) instead of the in-tree one.
 Usage: python profiles/micro_bn.py [reps]"""
 import ctypes
 import json

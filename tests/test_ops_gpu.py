@@ -166,6 +166,73 @@ def test_bn_relu_bits_forward_backward(cuda_device, rows, C, ds):
     assert torch.equal(dy2, (dy.float() * (y.float() > 0)).bfloat16())       # mode 2 masks it in place
 
 
+def misaligned_copy(t):
+    """t's contents in a larger allocation, one element (2 bytes of bf16, 1 byte of a bit mask) past a 16-byte boundary:
+    valid device memory that is not 16-byte aligned."""
+    big = torch.empty(t.numel() + 16, dtype=t.dtype, device=t.device)
+    v = big[1:1 + t.numel()].view(t.shape)
+    v.copy_(t)
+    assert v.data_ptr() % 16 != 0
+    return v
+
+
+@pytest.mark.parametrize("op", ["apply", "apply_bits", "backward0", "backward1", "backward2", "backward3"])
+def test_bn_passes_reject_misaligned_tensors(cuda_device, op):
+    """The batch-norm passes stream every tensor with 16-byte vectors and bulk copies. A tensor that is not 16-byte
+    aligned is rejected on the host before anything runs: the call fails, and the outputs and the dgamma / dbeta
+    accumulators keep their sentinel values. For the backward this includes dx, which only its second pass uses."""
+    rows, C = 1000, 64
+    g = torch.Generator().manual_seed(11)
+    x, dy, res, blk_out = (torch.randn(rows, C, generator=g).to(cuda_device).bfloat16() for _ in range(4))
+    bits = torch.randint(0, 256, (rows, C // 8), generator=g, dtype=torch.uint8).to(cuda_device)
+    scale, invstd = ((torch.rand(C, generator=g) + 0.5).to(cuda_device) for _ in range(2))
+    shift, mean = (torch.randn(C, generator=g).to(cuda_device) for _ in range(2))
+    dgamma, dbeta = torch.full((C,), 7.0, device=cuda_device), torch.full((C,), 7.0, device=cuda_device)
+    lib = _lib.load()
+    P = _lib.ptr
+    if op.startswith("apply"):
+        with_bits = op == "apply_bits"
+        tensors = {"x": x, "res": res, "y": torch.full_like(x, 3.0)}
+        if with_bits:
+            tensors["bits"] = torch.full((rows, C // 8), 0xA5, dtype=torch.uint8, device=cuda_device)
+
+        def run(t):
+            if with_bits:
+                return lib.argus_bn_apply_bits(P(t["x"]), P(scale), P(shift), P(t["res"]), None, None, ctypes.c_int(1),
+                                               P(t["y"]), P(t["bits"]), ctypes.c_int64(rows), ctypes.c_int(C),
+                                               _lib.stream_ptr())
+            return lib.argus_bn_apply(P(t["x"]), P(scale), P(shift), P(t["res"]), None, None, ctypes.c_int(1), P(t["y"]),
+                                      ctypes.c_int64(rows), ctypes.c_int(C), _lib.stream_ptr())
+    else:
+        mask = int(op[-1])
+        tensors = {"dy": dy, "x": x, "dx": torch.full_like(x, 3.0)}
+        if mask in (2, 3):
+            tensors["out"] = blk_out if mask == 2 else bits
+
+        def run(t):
+            return lib.argus_bn_backward(P(t["dy"]), P(t["x"]), P(t.get("out")), P(scale), P(shift), P(mean), P(invstd),
+                                         P(dgamma), P(dbeta), P(t["dx"]), ctypes.c_int64(rows), ctypes.c_int(C),
+                                         ctypes.c_int(mask), _lib.stream_ptr())
+
+    for name in tensors:
+        t = dict(tensors, **{name: misaligned_copy(tensors[name])})
+        before = {k: v.clone() for k, v in t.items()}
+        status = run(t)
+        assert status != 0, name
+        assert "16-byte aligned" in lib.argus_last_error_string().decode(), name
+        torch.cuda.synchronize()
+        for k, v in t.items():
+            assert torch.equal(v, before[k]), (name, k)
+        assert torch.all(dgamma == 7.0) and torch.all(dbeta == 7.0), name
+    # the same call with every tensor aligned runs
+    assert run(tensors) == 0, lib.argus_last_error_string()
+    torch.cuda.synchronize()
+    if op.startswith("apply"):
+        assert not torch.all(tensors["y"] == 3.0)
+    else:
+        assert not torch.all(dbeta == 7.0)
+
+
 @pytest.mark.parametrize("N,H,W,Cin,Cout", [(2, 16, 16, 256, 64), (1, 8, 8, 512, 128), (3, 8, 16, 64, 64)])
 def test_dgrad_residual_bits(cuda_device, N, H, W, Cin, Cout):
     """1x1 dgrad whose residual is gated by the bit mask == dgrad with the pre-masked residual, bit for bit."""

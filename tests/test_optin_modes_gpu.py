@@ -33,8 +33,3 @@ def test_fused_bn_reduction_modes(cuda_device):
                                             "train_forward_backward or reproducible or prefetch"])
     _rerun({"ARGUS_FUSED_TAIL": "0"}, ["tests/test_model_gpu.py", "tests/test_train_gpu.py", "-k",
                                        "train_forward_backward or reproducible or prefetch"])
-
-
-def test_register_bn_kernels(cuda_device):
-    """ARGUS_BN_RING=0: the register versions of the batch-norm passes (fallback for unaligned tensors)."""
-    _rerun({"ARGUS_BN_RING": "0"}, ["tests/test_ops_gpu.py", "-k", "bn_"])
