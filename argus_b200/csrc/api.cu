@@ -365,6 +365,50 @@ int argus_conv2d_wgrad(const void* dy, const void* x, float* dw, int N, int H, i
   ARGUS_API_END
 }
 
+int argus_bn_frozen_finish(const void* W, const float* H, const float* stat_partial, int slots, int stat_stride,
+                           const float* scale, const float* mean, const float* invstd, float* dgamma, float* dbeta,
+                           float* dW, int accumulate, int O, int K, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  bn_frozen_finish(static_cast<const bf16*>(W), H, stat_partial, slots, stat_stride, scale, mean, invstd, dgamma, dbeta,
+                   dW, accumulate != 0, O, K, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+int argus_relu_bits_mask_colsum(void* g, const void* bits, int64_t rows, int C, float* out, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  relu_bits_mask_colsum(static_cast<bf16*>(g), static_cast<const uint8_t*>(bits), rows, C,
+                        lib_scratch(4LL * num_sms() * C), out, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+int argus_stem_unpool_relu(const void* dpool, const void* idx, const void* pooled, void* g0, int N, int H, int W,
+                           float* out, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  stem_unpool_relu(static_cast<const bf16*>(dpool), static_cast<const uint8_t*>(idx), static_cast<const bf16*>(pooled),
+                   static_cast<bf16*>(g0), N, H, W, lib_scratch(4LL * num_sms() * 64), out,
+                   static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+int argus_pack_weight_scaled(const float* w, const float* scale, void* packed, int Cout, int Cin, int k, int kind,
+                             void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(kind == 0 || (kind == 1 && Cout == 64 && Cin == 3 && k == 7), "kind 1 is the 64 x 3 x 7 x 7 stem");
+  WeightPackEntry e;
+  e.src_off = 0; e.dst_off = 0; e.cout = Cout; e.cin = Cin; e.kk = k * k; e.kind = kind;
+  const int64_t zero = 0;
+  // the one-entry table and its scale offset live at the start of the library scratch (synchronous copies: test entry)
+  float* dev = lib_scratch(static_cast<int64_t>((sizeof(WeightPackEntry) + sizeof(int64_t)) / sizeof(float) + 4));
+  auto* table = reinterpret_cast<WeightPackEntry*>(dev);
+  auto* off = reinterpret_cast<int64_t*>(reinterpret_cast<uint8_t*>(dev) + (sizeof(WeightPackEntry) + 7) / 8 * 8);
+  ARGUS_CUDA(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));
+  ARGUS_CUDA(cudaMemcpy(table, &e, sizeof(e), cudaMemcpyHostToDevice));
+  ARGUS_CUDA(cudaMemcpy(off, &zero, sizeof(zero), cudaMemcpyHostToDevice));
+  pack_weights_scaled(w, scale, off, static_cast<bf16*>(packed), table, 1, static_cast<cudaStream_t>(stream));
+  ARGUS_CUDA(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));
+  ARGUS_API_END
+}
 int argus_stem_dgrad(const void* dy, const void* w, float* dx, int N, int H, int W, void* stream) {
   ARGUS_API_BEGIN
   require_sm100();
@@ -680,6 +724,12 @@ int argus_model_forward(argus_model* m, const void* x, int is_u8, int B, int H, 
   ARGUS_API_BEGIN
   ARGUS_CHECK(m != nullptr, "null model");
   m->impl.forward(x, is_u8 != 0, B, H, W, training != 0, out, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+int argus_model_forward_frozen(argus_model* m, const void* x, int is_u8, int B, int H, int W, float* out, void* stream) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(m != nullptr, "null model");
+  m->impl.forward(x, is_u8 != 0, B, H, W, false, out, static_cast<cudaStream_t>(stream), true);
   ARGUS_API_END
 }
 int argus_model_stage_input_u8(argus_model* m, const void* images, const float* aug_params, const void* arc_mask,

@@ -335,4 +335,170 @@ void colsum_pixels_bf16(const bf16* x, int N, int H, int W, int C, int stride, f
 
 int64_t bn_alg_matrix_scratch_elems(int C) { return static_cast<int64_t>(kSplitO) * (C + 1) * C; }
 
+// ------------------------------------------------------------------------------------------------------------
+// Frozen-statistics backward (eval-mode forward made differentiable): the k1 = k0 = 0 case of the algebra above, for
+// every convolution. Nothing is subtracted from g, so dRaw = sc * g never needs to exist: dW = diag(sc) H with
+// H = g^T im2col(x), and the input gradient is the dgrad of g against diag(sc) W (pack_weights_scaled).
+// ------------------------------------------------------------------------------------------------------------
+// one warp per output channel o (H and dW deliberately not __restrict__: the 3x3 / stem finish scales H in place)
+__global__ void __launch_bounds__(256)
+bn_frozen_finish_kernel(const bf16* __restrict__ W, const float* H, const float* __restrict__ stat_partial, int slots,
+                        int stat_stride, const float* __restrict__ scale, const float* __restrict__ mean,
+                        const float* __restrict__ invstd, float* dgamma, float* dbeta, float* dW, int accumulate, int O,
+                        int K) {
+  pdl_prologue();
+  const int o = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (o >= O) return;
+  double db = 0.0, t = 0.0;
+  for (int k = lane; k < slots; k += 32) db += static_cast<double>(stat_partial[static_cast<size_t>(k) * stat_stride + o]);
+  const bf16* w = W + static_cast<size_t>(o) * K;
+  const float* h = H + static_cast<size_t>(o) * K;
+  for (int i = lane; i < K; i += 32) t += static_cast<double>(__bfloat162float(w[i])) * static_cast<double>(h[i]);
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {   // (also orders every lane's reads of H before the in-place writes below)
+    db += __shfl_xor_sync(0xffffffffu, db, off);
+    t += __shfl_xor_sync(0xffffffffu, t, off);
+  }
+  const float sc = scale[o];
+  if (lane == 0) {
+    dgamma[o] += static_cast<float>(static_cast<double>(invstd[o]) * (t - static_cast<double>(mean[o]) * db));
+    dbeta[o] += static_cast<float>(db);
+  }
+  float* d = dW + static_cast<size_t>(o) * K;
+  for (int i = lane; i < K; i += 32) d[i] = (accumulate ? d[i] : 0.f) + sc * h[i];
+}
+void bn_frozen_finish(const bf16* W, const float* H, const float* stat_partial, int slots, int stat_stride,
+                      const float* scale, const float* mean, const float* invstd, float* dgamma, float* dbeta, float* dW,
+                      bool accumulate, int O, int K, cudaStream_t st) {
+  ProfileScope prof("bn_frozen", st, 2.0 * O * static_cast<double>(K), 10.0 * O * static_cast<double>(K));
+  launch_kernel(bn_frozen_finish_kernel, (O * 32 + 255) / 256, 256, 0, st, W, H, stat_partial, slots, stat_stride, scale,
+                mean, invstd, dgamma, dbeta, dW, accumulate ? 1 : 0, O, K);
+  ARGUS_CUDA(cudaGetLastError());
+}
+
+// Block column sums shared by the two passes below: thread (rl, oc) holds the sums of channels 8 oc .. 8 oc + 7 over its
+// rows; the row lanes are added in order into partial[blockIdx.x][C].
+__device__ __forceinline__ void block_colsum_store(const float (&acc)[8], float (&red)[8][256], float* partial, int lanes,
+                                                   int row_lanes, int rl, int oc, int cvec) {
+#pragma unroll
+  for (int k = 0; k < 8; ++k) red[k][threadIdx.x] = acc[k];
+  __syncthreads();
+  if (rl == 0) {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      float s0 = 0.f;
+      for (int r = 0; r < row_lanes; ++r) s0 += red[k][r * lanes + oc];
+      partial[static_cast<size_t>(blockIdx.x) * (cvec * 8) + oc * 8 + k] = s0;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(256)
+relu_bits_mask_colsum_kernel(uint4* __restrict__ g, const uint8_t* __restrict__ bits, float* __restrict__ partial,
+                             int64_t rows, int cvec) {
+  pdl_prologue();
+  __shared__ float red[8][256];
+  const int lanes = cvec < 256 ? cvec : 256;
+  const int row_lanes = 256 / lanes;
+  const int rl = threadIdx.x / lanes, oc = threadIdx.x % lanes;
+  float acc[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) acc[k] = 0.f;
+  for (int64_t r = static_cast<int64_t>(blockIdx.x) * row_lanes + rl; r < rows; r += static_cast<int64_t>(gridDim.x) * row_lanes) {
+    const int64_t i = r * cvec + oc;
+    const uint4 u = g[i];
+    const unsigned b = bits[i];
+    uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const uint32_t keep = ((b >> (2 * j)) & 1u ? 0x0000ffffu : 0u) | ((b >> (2 * j + 1)) & 1u ? 0xffff0000u : 0u);
+      w[j] &= keep;
+      const float2 f = unpack_bf16x2(w[j]);
+      acc[2 * j] += f.x;
+      acc[2 * j + 1] += f.y;
+    }
+    g[i] = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+  block_colsum_store(acc, red, partial, lanes, row_lanes, rl, oc, cvec);
+}
+void relu_bits_mask_colsum(bf16* g, const uint8_t* bits, int64_t rows, int C, float* scratch, float* out,
+                           cudaStream_t st) {
+  ARGUS_CHECK(C % 8 == 0 && is_pow2(C / 8) && C <= 2048, "relu_bits_mask_colsum: C/8 must be a power of two <= 256");
+  ProfileScope prof("bn_frozen", st, 0, static_cast<double>(rows) * C * (4 + 0.125));
+  const int cvec = C / 8;
+  const int row_lanes = 256 / std::min(cvec, 256);
+  const int blocks = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((rows + row_lanes - 1) / row_lanes, 4LL * num_sms())));
+  launch_kernel(relu_bits_mask_colsum_kernel, blocks, 256, 0, st, reinterpret_cast<uint4*>(g), bits, scratch, rows, cvec);
+  ARGUS_CUDA(cudaGetLastError());
+  colsum_finalize(scratch, blocks, out, C, st);
+}
+
+// thread = one stem pixel x 8 channels; the 3x3 stride-2 pad-1 windows holding pixel (h, w) are ph in {h/2, (h+1)/2},
+// pw likewise (maxpool_bwd's order), tap code (h - 2 ph + 1) * 3 + (w - 2 pw + 1)
+__global__ void __launch_bounds__(256)
+stem_unpool_relu_kernel(const uint4* __restrict__ dpool, const uint2* __restrict__ idx, const uint4* __restrict__ pooled,
+                        uint4* __restrict__ g0, float* __restrict__ partial, int N, int H, int W) {
+  pdl_prologue();
+  constexpr int cvec = 8;   // C = 64
+  __shared__ float red[8][256];
+  const int rl = threadIdx.x / cvec, oc = threadIdx.x % cvec;
+  const int Ho = H >> 1, Wo = W >> 1;
+  const int64_t pixels = static_cast<int64_t>(N) * H * W;
+  float acc[8];
+#pragma unroll
+  for (int k = 0; k < 8; ++k) acc[k] = 0.f;
+  for (int64_t r = static_cast<int64_t>(blockIdx.x) * 32 + rl; r < pixels; r += static_cast<int64_t>(gridDim.x) * 32) {
+    const int w = static_cast<int>(r % W);
+    const int64_t t = r / W;
+    const int h = static_cast<int>(t % H);
+    const int n = static_cast<int>(t / H);
+    float v[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) v[k] = 0.f;
+    for (int ph = h >> 1; ph <= ((h + 1) >> 1) && ph < Ho; ++ph) {
+      for (int pw = w >> 1; pw <= ((w + 1) >> 1) && pw < Wo; ++pw) {
+        const uint32_t code = static_cast<uint32_t>((h - 2 * ph + 1) * 3 + (w - 2 * pw + 1));
+        const int64_t j = ((static_cast<int64_t>(n) * Ho + ph) * Wo + pw) * cvec + oc;
+        const uint2 id = __ldg(idx + j);
+        const uint4 d = __ldg(dpool + j), pv = __ldg(pooled + j);
+        const uint32_t dw[4] = {d.x, d.y, d.z, d.w}, pw4[4] = {pv.x, pv.y, pv.z, pv.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const float2 df = unpack_bf16x2(dw[q]), pf = unpack_bf16x2(pw4[q]);
+          const uint32_t word = q < 2 ? id.x : id.y;
+          const uint32_t b0 = (word >> (16 * (q & 1))) & 0xffu, b1 = (word >> (16 * (q & 1) + 8)) & 0xffu;
+          if (b0 == code && pf.x > 0.f) v[2 * q] += df.x;
+          if (b1 == code && pf.y > 0.f) v[2 * q + 1] += df.y;
+        }
+      }
+    }
+    uint4 o;
+    o.x = pack_bf16x2(v[0], v[1]); o.y = pack_bf16x2(v[2], v[3]);
+    o.z = pack_bf16x2(v[4], v[5]); o.w = pack_bf16x2(v[6], v[7]);
+    g0[r * cvec + oc] = o;
+    const uint32_t ow[4] = {o.x, o.y, o.z, o.w};
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const float2 f = unpack_bf16x2(ow[q]);
+      acc[2 * q] += f.x;
+      acc[2 * q + 1] += f.y;
+    }
+  }
+  block_colsum_store(acc, red, partial, cvec, 32, rl, oc, cvec);
+}
+void stem_unpool_relu(const bf16* dpool, const uint8_t* idx, const bf16* pooled, bf16* g0, int N, int H, int W,
+                      float* scratch, float* out, cudaStream_t st) {
+  ARGUS_CHECK(H % 2 == 0 && W % 2 == 0, "stem_unpool_relu: H and W must be even");
+  const int64_t pixels = static_cast<int64_t>(N) * H * W;
+  // HBM model: the pooled gradient, pooled values and arg-max bytes once (a quarter of the pixels), g0 written once
+  ProfileScope prof("bn_frozen", st, 0, pixels * 64 * (2.0 + 0.25 * (2 + 2 + 1)));
+  const int blocks = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((pixels + 31) / 32, 4LL * num_sms())));
+  launch_kernel(stem_unpool_relu_kernel, blocks, 256, 0, st, reinterpret_cast<const uint4*>(dpool),
+                reinterpret_cast<const uint2*>(idx), reinterpret_cast<const uint4*>(pooled), reinterpret_cast<uint4*>(g0),
+                scratch, N, H, W);
+  ARGUS_CUDA(cudaGetLastError());
+  colsum_finalize(scratch, blocks, out, 64, st);
+}
+
 }  // namespace argus

@@ -247,6 +247,30 @@ void unpack_wgrads(const float* packed_grads, float* grads, const WeightPackEntr
   launch_kernel(unpack_wgrads_kernel, dim3(256, n_entries), 256, 0, s, packed_grads, grads, table_dev);
   ARGUS_CUDA(cudaGetLastError());
 }
+// diag(scale) W in the packed layout: every element is rounded once, bf16_rn(scale[co] * w). Runs once per refresh of the
+// eval-mode fold, so it keeps the plain per-element index map of the stem branch above for every entry.
+__global__ void __launch_bounds__(256)
+pack_weights_scaled_kernel(const float* __restrict__ params, const float* __restrict__ scales,
+                           const int64_t* __restrict__ scale_off, bf16* __restrict__ packed,
+                           const WeightPackEntry* __restrict__ table) {
+  pdl_prologue();
+  const WeightPackEntry e = table[blockIdx.y];
+  const float* sc = scales + scale_off[blockIdx.y];
+  const int64_t n = packed_count(e);
+  const int64_t row = n / e.cout;   // packed row of one output channel (stem: 256)
+  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n;
+       i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int64_t src = packed_to_torch(e, i);
+    packed[e.dst_off + i] = __float2bfloat16(src >= 0 ? sc[i / row] * params[e.src_off + src] : 0.f);
+  }
+}
+void pack_weights_scaled(const float* params, const float* scales, const int64_t* scale_off_dev, bf16* packed,
+                         const WeightPackEntry* table_dev, int n_entries, cudaStream_t s) {
+  ProfileScope prof("pack_weights", s, 0, 0);
+  launch_kernel(pack_weights_scaled_kernel, dim3(256, n_entries), 256, 0, s, params, scales, scale_off_dev, packed,
+                table_dev);
+  ARGUS_CUDA(cudaGetLastError());
+}
 
 // plain 4-byte global load as a volatile asm statement: a run of these is issued back to back (the compiler keeps
 // their order and cannot fold the consumers in between), so N partial sums cost one memory round trip, not N
@@ -335,18 +359,24 @@ void bn_finalize(const float* partial, int slots, double count, const float* gam
   ARGUS_CUDA(cudaGetLastError());
 }
 __global__ void bn_fold_eval_kernel(const float* gamma, const float* beta, const float* rm, const float* rv, float eps,
-                                    float* scale, float* shift, int C) {
+                                    float* scale, float* shift, float* mean, float* invstd, int C) {
   pdl_prologue();
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= C) return;
-  const float sc = gamma[c] * rsqrtf(rv[c] + eps);
+  const float is = rsqrtf(rv[c] + eps);
+  const float sc = gamma[c] * is;
   scale[c] = sc;
   shift[c] = beta[c] - rm[c] * sc;
+  if (mean != nullptr) {
+    mean[c] = rm[c];
+    invstd[c] = is;
+  }
 }
 void bn_fold_eval(const float* gamma, const float* beta, const float* running_mean, const float* running_var,
-                  float eps, float* scale, float* shift, int C, cudaStream_t s) {
+                  float eps, float* scale, float* shift, int C, cudaStream_t s, float* mean, float* invstd) {
   ProfileScope prof("bn_finalize", s, 0, 24.0 * C);
-  launch_kernel(bn_fold_eval_kernel, (C + 127) / 128, 128, 0, s, gamma, beta, running_mean, running_var, eps, scale, shift, C);
+  launch_kernel(bn_fold_eval_kernel, (C + 127) / 128, 128, 0, s, gamma, beta, running_mean, running_var, eps, scale, shift,
+                mean, invstd, C);
   ARGUS_CUDA(cudaGetLastError());
 }
 

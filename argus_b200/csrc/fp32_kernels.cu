@@ -412,7 +412,7 @@ __global__ void bn_bwd_apply_f32_kernel(const float* __restrict__ dy, const floa
 }
 void bn_f32_backward(const float* dy, const float* x, const float* out, const float* scale, const float* mean,
                      const float* invstd, float* dgamma, float* dbeta, float* dx, float* g_out, int64_t rows, int C,
-                     double* scratch, float* sums, cudaStream_t s) {
+                     double* scratch, float* sums, cudaStream_t s, bool frozen_stats) {
   ProfileScope prof("fp32_bn", s, 0, 20.0 * rows * C);
   const int blocks = bn_blocks(rows, C);
   launch_kernel(bn_sums_f32_kernel<1>, blocks, 256, 0, s, x, dy, out, mean, invstd, scratch, rows, C);
@@ -422,7 +422,7 @@ void bn_f32_backward(const float* dy, const float* x, const float* out, const fl
   const int64_t n = rows * C;
   launch_kernel(bn_bwd_apply_f32_kernel, static_cast<int>(std::min<int64_t>((n + 255) / 256, 16384)), 256, 0, s, 
       dy, x, out, scale, mean, invstd, sums, sums + C, dx, g_out, n, C,
-      static_cast<float>(1.0 / static_cast<double>(rows)));
+      frozen_stats ? 0.f : static_cast<float>(1.0 / static_cast<double>(rows)));
   ARGUS_CUDA(cudaGetLastError());
 }
 

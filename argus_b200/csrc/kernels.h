@@ -27,6 +27,10 @@ void pack_weights(const float* params, bf16* packed, const WeightPackEntry* tabl
 // fp32 packed-layout weight gradients -> PyTorch-layout gradient arena (only entries with kk > 1 or kind 1)
 void unpack_wgrads(const float* packed_grads, float* grads, const WeightPackEntry* table_dev, int n_entries,
                    cudaStream_t s);
+// diag(scale) W -> bf16 packed (same layout and offsets as pack_weights), bf16_rn(scale[co] * w) per element. Entry j
+// scales its output channels by scales[scale_off_dev[j] + co] (the frozen-statistics backward's dgrad operands).
+void pack_weights_scaled(const float* params, const float* scales, const int64_t* scale_off_dev, bf16* packed,
+                         const WeightPackEntry* table_dev, int n_entries, cudaStream_t s);
 
 // ---- augmentation (argus/data.py:41-103, 213-225) ---------------------------------------------------------------
 constexpr int kAugParams = 40;   // floats per image in the parameter table (layout: oracle/augment.py::sample_params)
@@ -60,9 +64,11 @@ void spaghetti_draw(const uint8_t* in, uint8_t* out, const float* arcs, uint32_t
 void bn_finalize(const float* partial, int slots, double count, const float* gamma, const float* beta,
                  float* running_mean, float* running_var, float momentum, float eps, float* scale, float* shift,
                  float* save_mean, float* save_invstd, int C, cudaStream_t s);
-// eval: running statistics -> scale/shift
+// eval: running statistics -> scale/shift (+ mean = running_mean, invstd = 1/sqrt(running_var + eps) when mean != nullptr:
+// the frozen-statistics backward reads them)
 void bn_fold_eval(const float* gamma, const float* beta, const float* running_mean, const float* running_var,
-                  float eps, float* scale, float* shift, int C, cudaStream_t s);
+                  float eps, float* scale, float* shift, int C, cudaStream_t s, float* mean = nullptr,
+                  float* invstd = nullptr);
 // bn_apply, bn_bwd_reduce and bn_bwd_apply stream their tensors with 16-byte vectors and bulk copies: every tensor
 // pointer they take (x, res, y, relu_bits; dy, x, out, dx) must be 16-byte aligned. They call this before launching
 // anything; it throws for a misaligned pointer (nullptr passes). A caller of several passes checks all their tensors
@@ -134,6 +140,28 @@ void bn_stats_from_gram(const bf16* W, const float* G, const float* s, double ro
                         const float* beta, float* running_mean, float* running_var, float momentum, float eps,
                         float* scale, float* shift, float* save_mean, float* save_invstd, float* scratch, int O, int C,
                         cudaStream_t st);
+// ---- frozen-statistics batch-norm backward (bn_algebra.cu) --------------------------------------------------------
+// With constant statistics the batch norm after a convolution is the per-channel affine map sc * raw + shift, so with g
+// the (ReLU-masked) gradient of its output and H = g^T im2col(x) the weight-gradient GEMM fed g:
+//   dW = diag(sc) H,  dgamma = invstd * (rowdot(W, H) - mean * sum g),  dbeta = sum g.
+// One warp per output channel o; W: bf16 [O][K] (the packed weight the forward used), H: fp32 [O][K] in the same layout.
+// sum g = the fp64 sum of stat_partial[k * stat_stride + o] over k < slots (a dgrad's statistics slots, or slots = 1 for
+// a finished vector). dgamma, dbeta += ; dW[o][:] = (accumulate ? dW[o][:] : 0) + scale[o] * H[o][:] (dW may be H).
+// Deterministic: fixed lane order and shuffle tree, fp64 sums.
+void bn_frozen_finish(const bf16* W, const float* H, const float* stat_partial, int slots, int stat_stride,
+                      const float* scale, const float* mean, const float* invstd, float* dgamma, float* dbeta, float* dW,
+                      bool accumulate, int O, int K, cudaStream_t st);
+// g[r][c] = bit(r, c) ? g[r][c] : 0 in place (bits: [rows][C/8], bit k of byte j = channel 8j + k) and out[c] = sum_r of
+// the stored values, deterministic. scratch: >= 4 * num_sms * C floats.
+void relu_bits_mask_colsum(bf16* g, const uint8_t* bits, int64_t rows, int C, float* scratch, float* out,
+                           cudaStream_t st);
+// Stem of the frozen-statistics backward: g0 = unpool(dpool) * [pooled > 0] -- the gradient wrt the stem's BN + ReLU
+// output (N, H, W, 64), written in full -- from the pooled gradient dpool and the pooled values (N, H/2, W/2, 64) and
+// the arg-max bytes of maxpool_fwd. A max of ReLU outputs is positive exactly where its arg-max element is. The up to
+// four windows that hold a pixel are added in fp32 in window order; out[c] = sum of the stored g0, deterministic.
+// scratch: >= 4 * num_sms * 64 floats.
+void stem_unpool_relu(const bf16* dpool, const uint8_t* idx, const bf16* pooled, bf16* g0, int N, int H, int W,
+                      float* scratch, float* out, cudaStream_t st);
 // out[c] = sum_r x[r][c], deterministic; scratch: >= 4 * num_sms * C floats
 void colsum_rows_bf16(const bf16* x, int64_t rows, int C, float* scratch, float* out, cudaStream_t st);
 // same over the pixels (stride*h, stride*w) of an (N, H, W, C) tensor (what a strided 1x1 convolution reads)

@@ -50,10 +50,11 @@ void bn_f32_train_stats(const float* x, int64_t rows, int C, const float* gamma,
 void bn_f32_apply(const float* x, const float* scale, const float* shift, const float* res, const float* rscale,
                   const float* rshift, int relu, float* y, int64_t rows, int C, cudaStream_t s);
 // g = dy masked by (out > 0) when out != nullptr; dgamma += sum g*xhat, dbeta += sum g; dx = BN input gradient;
-// g_out (optional) receives g. sums: 2*C floats of scratch.
+// g_out (optional) receives g. sums: 2*C floats of scratch. frozen_stats: mean / invstd are constants (eval-mode
+// statistics), so dx = scale * g (the batch-mean terms are multiplied by 0); dgamma / dbeta are the same sums.
 void bn_f32_backward(const float* dy, const float* x, const float* out, const float* scale, const float* mean,
                      const float* invstd, float* dgamma, float* dbeta, float* dx, float* g_out, int64_t rows, int C,
-                     double* scratch, float* sums, cudaStream_t s);
+                     double* scratch, float* sums, cudaStream_t s, bool frozen_stats = false);
 
 void maxpool_f32_fwd(const float* x, float* y, uint8_t* idx, int N, int H, int W, int C, cudaStream_t s);
 void maxpool_f32_bwd(const float* dy, const uint8_t* idx, float* dx, int N, int H, int W, int C, cudaStream_t s);

@@ -58,6 +58,9 @@ void Model::set_precision(int mode) {
   ARGUS_CHECK(mode == 0 || mode == 1, "precision mode must be 0 (bf16 tensor cores) or 1 (fp32)");
   precision_ = mode;
   last_train_plan_ = nullptr;
+  last_frozen_plan_ = nullptr;
+  last_grad_forward_ = 0;
+  last_forward_frozen_ = false;
   stem_grad_ready_ = false;
   last_plan_ = nullptr;
   staged_plan_ = nullptr;
@@ -80,6 +83,8 @@ Model::~Model() {
   cudaFree(bnred_stats_);
   cudaFree(wgrad_scratch_);
   cudaFree(pack_table_dev_);
+  cudaFree(packed_scaled_); cudaFree(scaled_table_dev_); cudaFree(scaled_scale_off_dev_);
+  cudaFree(frz_h_); cudaFree(frz_pstats_); cudaFree(frz_gstats_); cudaFree(frz_sums_); cudaFree(frz_partial_);
   cudaFree(stem_in_[0]);
   cudaFree(stem_in_[1]);
   cudaFree(arena_);
@@ -255,6 +260,8 @@ void Model::bind(float* params, float* grads, float* buffers) {
   }
   plans_.clear();
   last_train_plan_ = nullptr;
+  last_frozen_plan_ = nullptr;
+  last_grad_forward_ = 0;
   last_plan_ = nullptr;
   staged_plan_ = nullptr;
   eval_fold_dirty_ = true;
@@ -282,14 +289,14 @@ T* Model::arena_alloc(size_t count) {
   return reinterpret_cast<T*>(p);
 }
 
-void Model::reserve(int max_batch, int H, int W, bool training) {
+void Model::reserve(int max_batch, int H, int W, bool training, bool frozen) {
   ARGUS_CHECK(max_batch > 0, "batch must be positive");
   ARGUS_CHECK(is_pow2(H) && is_pow2(W) && H >= 32 && W >= 32, "H and W must be powers of two >= 32");
   // dry run to size the arena
   uint8_t* saved = arena_;
   arena_ = nullptr;
   Plan tmp;
-  tmp.B = max_batch; tmp.H = H; tmp.W = W; tmp.N = max_batch * n_cams_; tmp.training = training;
+  tmp.B = max_batch; tmp.H = H; tmp.W = W; tmp.N = max_batch * n_cams_; tmp.training = training; tmp.frozen = frozen;
   arena_used_ = 0;
   // build_plan only measures when arena_ == nullptr
   build_plan(tmp);
@@ -307,6 +314,8 @@ void Model::reserve(int max_batch, int H, int W, bool training) {
     stem_in_elems_ = stem_need;
     plans_.clear();
     last_train_plan_ = nullptr;
+    last_frozen_plan_ = nullptr;
+    last_grad_forward_ = 0;
     last_plan_ = nullptr;
     staged_plan_ = nullptr;
   }
@@ -317,6 +326,8 @@ void Model::reserve(int max_batch, int H, int W, bool training) {
     arena_bytes_ = need;
     plans_.clear();
     last_train_plan_ = nullptr;
+    last_frozen_plan_ = nullptr;
+    last_grad_forward_ = 0;
     last_plan_ = nullptr;
     staged_plan_ = nullptr;
   }
@@ -325,13 +336,14 @@ void Model::reserve(int max_batch, int H, int W, bool training) {
   reserved_training_ = reserved_training_ || training;
 }
 
-Plan& Model::get_plan(int B, int H, int W, bool training) {
-  auto key = std::make_tuple(B, H, W, training);
+Plan& Model::get_plan(int B, int H, int W, bool training, bool frozen) {
+  auto key = std::make_tuple(B, H, W, training, frozen);
   auto it = plans_.find(key);
   if (it != plans_.end()) return *it->second;
-  reserve(B, H, W, training);  // grows the arena if needed (and drops stale plans)
+  if (frozen) ensure_frozen_buffers();
+  reserve(B, H, W, training, frozen);  // grows the arena if needed (and drops stale plans)
   auto p = std::make_unique<Plan>();
-  p->B = B; p->H = H; p->W = W; p->N = B * n_cams_; p->training = training;
+  p->B = B; p->H = H; p->W = W; p->N = B * n_cams_; p->training = training; p->frozen = frozen;
   arena_used_ = 0;
   build_plan(*p);
   ARGUS_CHECK(arena_used_ <= arena_bytes_, "activation arena overflow");
@@ -344,6 +356,7 @@ void Model::build_plan(Plan& p) {
   const bool real = (arena_ != nullptr);  // dry runs only measure
   const int N = p.N, H = p.H, W = p.W;
   const bool tr = p.training;
+  const bool fz = p.frozen;   // eval layout + bit masks + backward scratch
   auto plan_conv = [&](ConvPlan& cp, ConvRef& c, int n, int h, int w, const bf16* in, bf16* out_raw,
                        bool want_dgrad) {
     c.shape.N = n; c.shape.H = h; c.shape.W = w;
@@ -358,7 +371,7 @@ void Model::build_plan(Plan& p) {
   const size_t stem_elems = static_cast<size_t>(N) * H1 * W1 * 64;
   if (tr) p.raw0 = arena_alloc<bf16>(stem_elems); else p.act0 = arena_alloc<bf16>(stem_elems);
   p.pooled0 = arena_alloc<bf16>(stem_elems / 4);
-  if (tr) p.idx0 = arena_alloc<uint8_t>(stem_elems / 4);
+  if (tr || fz) p.idx0 = arena_alloc<uint8_t>(stem_elems / 4);
   plan_conv(p.stem, stem_, N, H, W, tr ? stem_in_[0] : p.x_in, tr ? p.raw0 : p.act0, false);
   if (real) {
     ARGUS_CHECK(!tr || static_cast<size_t>(N) * (H / 2) * (W / 2 + 4) * 16 <= stem_in_elems_, "stem input buffers too small");
@@ -391,7 +404,11 @@ void Model::build_plan(Plan& p) {
     if (tr && !bp.fused_tail) bp.raw3 = arena_alloc<bf16>(e_out * oc);
     if (br.has_ds) bp.rawd = arena_alloc<bf16>(e_out * oc);  // eval / fused tail: holds the folded-BN identity branch
     bp.out = arena_alloc<bf16>(e_out * oc);
-    if (tr) bp.out_bits = arena_alloc<uint8_t>(e_out * oc / 8);
+    if (tr || fz) bp.out_bits = arena_alloc<uint8_t>(e_out * oc / 8);
+    if (fz) {
+      bp.act1_bits = arena_alloc<uint8_t>(e_in * wd / 8);
+      bp.act2_bits = arena_alloc<uint8_t>(e_out * wd / 8);
+    }
     if (tr && bn_algebra_ && wd <= 256)
       bp.act2_colsum = arena_alloc<float>(static_cast<size_t>(bn_apply_grid(static_cast<int64_t>(e_out), wd)) * wd);
     if (bp.fused_tail) {
@@ -428,7 +445,7 @@ void Model::build_plan(Plan& p) {
   p.h2 = arena_alloc<float>(static_cast<size_t>(B) * 128);
   p.a2 = arena_alloc<float>(static_cast<size_t>(B) * 128);
   p.out = arena_alloc<float>(static_cast<size_t>(B) * 8);
-  if (!tr) return;
+  if (!tr && !fz) return;
 
   // ---- backward scratch
   p.d_out = arena_alloc<float>(static_cast<size_t>(B) * 8);
@@ -443,6 +460,43 @@ void Model::build_plan(Plan& p) {
     p.fc.wgrad = plan_conv_wgrad(fc_.shape, p.d_feat, p.pooled, grads_dev_ + fc_.w_off);
     ensure_wgrad_scratch(p.fc.wgrad);
     p.fc.dgrad = plan_conv_dgrad(fc_.shape, p.d_feat, packed_ + fc_.packed_off, p.d_pooled);
+  }
+  if (fz) {
+    // Per block: P = the masked block-output gradient, Q = g2 (conv3 dgrad, masked by act2's bits), R = g1 (conv2 dgrad,
+    // masked by act1's bits), S = the block-input gradient (conv1 dgrad + identity branch), T = the downsample dgrad.
+    // Weight gradients: H = g^T x into frz_h_ (1x1) or the packed scratch (3x3, stem); dgrads against diag(sc) W.
+    bf16 *P = G[0], *Q = G[1], *R = G[2], *S = G[3], *T = G[4];
+    for (int i = static_cast<int>(blocks_.size()) - 1; i >= 0; --i) {
+      BlockRef& br = blocks_[i];
+      BlockPlan& bp = p.blocks[i];
+      bf16* Tb = (br.has_ds && br.ds.shape.stride == 2) ? arena_alloc<bf16>(bp.x_bytes / sizeof(bf16)) : T;
+      bp.g_out = P; bp.g_q = Q; bp.g_r = R; bp.g_t = Tb; bp.g_x = S;
+      if (real) {
+        auto Ws = [&](const ConvRef& c) { return packed_scaled_ + c.packed_off; };
+        bp.c3.wgrad = plan_conv_wgrad(br.c3.shape, P, bp.act2, frz_h_);
+        bp.c3.dgrad = plan_conv_dgrad(br.c3.shape, P, Ws(br.c3), Q);
+        if (br.has_ds) {
+          bp.ds.wgrad = plan_conv_wgrad(br.ds.shape, P, bp.x, frz_h_);
+          bp.ds.dgrad = plan_conv_dgrad(br.ds.shape, P, Ws(br.ds), Tb);
+          ensure_wgrad_scratch(bp.ds.wgrad);
+        }
+        bp.c2.wgrad = plan_conv_wgrad(br.c2.shape, Q, bp.act1, gpacked_ + br.c2.gpacked_off);
+        bp.c2.dgrad = plan_conv_dgrad(br.c2.shape, Q, Ws(br.c2), R);
+        bp.c1.wgrad = plan_conv_wgrad(br.c1.shape, R, bp.x, frz_h_);
+        bp.c1.dgrad = plan_conv_dgrad(br.c1.shape, R, Ws(br.c1), S);
+        ensure_wgrad_scratch(bp.c1.wgrad);
+        ensure_wgrad_scratch(bp.c2.wgrad);
+        ensure_wgrad_scratch(bp.c3.wgrad);
+      }
+      std::swap(P, S);
+    }
+    p.g_stem_in = P;
+    p.g_raw0 = Q;   // g0
+    if (real) {
+      p.stem.wgrad = plan_conv_wgrad(stem_.shape, Q, p.x_in, gpacked_ + stem_.gpacked_off);
+      ensure_wgrad_scratch(p.stem.wgrad);
+    }
+    return;
   }
   // rotate the five scratch buffers through the blocks in reverse order (see Model::backward)
   bf16 *P = G[0], *Q = G[1], *R = G[2], *S = G[3], *T = G[4];
@@ -510,7 +564,7 @@ void Model::fold_eval(cudaStream_t s) {
   auto fold = [&](const ConvRef& c) {
     float* sc = bn_scratch_ + c.bn.scratch_off;
     bn_fold_eval(params_dev_ + c.bn.gamma_off, params_dev_ + c.bn.beta_off, buffers_dev_ + c.bn.rm_off,
-                 buffers_dev_ + c.bn.rv_off, kBnEps, sc, sc + c.bn.C, c.bn.C, s);
+                 buffers_dev_ + c.bn.rv_off, kBnEps, sc, sc + c.bn.C, c.bn.C, s, sc + 2 * c.bn.C, sc + 3 * c.bn.C);
   };
   fold(stem_);
   for (auto& b : blocks_) {
@@ -518,6 +572,7 @@ void Model::fold_eval(cudaStream_t s) {
     if (b.has_ds) fold(b.ds);
   }
   eval_fold_dirty_ = false;
+  scaled_dirty_ = true;
 }
 
 void Model::run_conv_train(const ConvPlan& cp, const ConvRef& c, int64_t rows, cudaStream_t s) {
@@ -599,31 +654,39 @@ void Model::stats_from_gram(const ConvRef& c, const WgradLaunch& gram, float* G,
                      kBnEps, sc, sc + O, sc + 2 * O, sc + 3 * O, alg_mpartial_, O, C, s);
 }
 
+// Eval plans and frozen plans run the same launches; a frozen plan's epilogues also write the ReLU bit masks and its
+// max pooling the arg-max bytes (null pointers in an eval plan), which leaves every output bit as it is.
 void Model::forward_eval(Plan& p, cudaStream_t s) {
   if (eval_fold_dirty_) fold_eval(s);
+  if (p.frozen && scaled_dirty_) {
+    pack_weights_scaled(params_dev_, bn_scratch_, scaled_scale_off_dev_, packed_scaled_, scaled_table_dev_,
+                        n_scaled_entries_, s);
+    scaled_dirty_ = false;
+  }
   const int N = p.N;
-  auto EP = [&](const ConvRef& c, const bf16* res, int relu) {
+  auto EP = [&](const ConvRef& c, const bf16* res, int relu, uint8_t* bits) {
     Epilogue e;
     e.scale = bn_scratch_ + c.bn.scratch_off;
     e.shift = e.scale + c.bn.C;
     e.residual = res;
     e.relu = relu;
+    e.relu_bits_out = bits;
     e.early_trigger = 1;   // inference chain: the next convolution sets itself up while this one runs
     return e;
   };
-  launch_conv(p.stem.fwd, EP(stem_, nullptr, 1), s);
-  maxpool_fwd(p.act0, nullptr, nullptr, p.pooled0, nullptr, N, p.H / 2, p.W / 2, 64, s);
+  launch_conv(p.stem.fwd, EP(stem_, nullptr, 1, nullptr), s);
+  maxpool_fwd(p.act0, nullptr, nullptr, p.pooled0, p.idx0, N, p.H / 2, p.W / 2, 64, s);
   for (size_t i = 0; i < blocks_.size(); ++i) {
     BlockRef& br = blocks_[i];
     BlockPlan& bp = p.blocks[i];
-    launch_conv(bp.c1.fwd, EP(br.c1, nullptr, 1), s);
-    launch_conv(bp.c2.fwd, EP(br.c2, nullptr, 1), s);
+    launch_conv(bp.c1.fwd, EP(br.c1, nullptr, 1, bp.act1_bits), s);
+    launch_conv(bp.c2.fwd, EP(br.c2, nullptr, 1, bp.act2_bits), s);
     const bf16* identity = bp.x;
     if (br.has_ds) {
-      launch_conv(bp.ds.fwd, EP(br.ds, nullptr, 0), s);
+      launch_conv(bp.ds.fwd, EP(br.ds, nullptr, 0, nullptr), s);
       identity = bp.rawd;
     }
-    launch_conv(bp.c3.fwd, EP(br.c3, identity, 1), s);
+    launch_conv(bp.c3.fwd, EP(br.c3, identity, 1, bp.out_bits), s);
   }
 }
 
@@ -641,18 +704,29 @@ void Model::head_forward(Plan& p, float* out, cudaStream_t s) {
   ARGUS_CUDA(cudaMemcpyAsync(out, p.out, static_cast<size_t>(B) * 6 * sizeof(float), cudaMemcpyDeviceToDevice, s)); pdl_break(s, kPdlAfterMemop);
 }
 
-void Model::forward(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s) {
+void Model::forward(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s,
+                    bool frozen) {
   ARGUS_CHECK(params_dev_ != nullptr && buffers_dev_ != nullptr, "model is not bound");
   ARGUS_CHECK(B > 0, "empty batch");
   ARGUS_CHECK(!training || B * n_cams_ * (H / 32) * (W / 32) > 1,
               "train-mode batch norm needs more than one value per channel");
+  ARGUS_CHECK(!(training && frozen), "a frozen-statistics forward is an eval-mode forward");
+  ARGUS_CHECK(!frozen || x != nullptr, "the frozen-statistics forward needs the image tensor (no staged input)");
   stem_grad_ready_ = false;
-  if (training) train_input_f32_ = (x != nullptr && !is_u8);
+  if (training || frozen) train_input_f32_ = (x != nullptr && !is_u8);
+  // which forward backward() differentiates (set after get_plan(), whose arena growth forgets the previous plans)
+  auto note_kind = [&] {
+    if (training) last_grad_forward_ = 1;
+    if (frozen) last_grad_forward_ = 2;
+    last_forward_frozen_ = frozen;
+  };
   if (precision_ == 1) {
-    forward_fp32(x, is_u8, B, H, W, training, out, s);
+    note_kind();
+    forward_fp32(x, is_u8, B, H, W, training, frozen, out, s);
     return;
   }
-  Plan& p = get_plan(B, H, W, training);
+  Plan& p = get_plan(B, H, W, training, frozen);
+  note_kind();
   // every input is written to the alternate stem buffer, which then becomes the current one: a batch staged ahead of
   // time (stage_input_u8 on another stream) never touches the buffer the in-flight pass still reads
   if (x == nullptr) {
@@ -675,6 +749,7 @@ void Model::forward(const void* x, bool is_u8, int B, int H, int W, bool trainin
     last_train_plan_ = &p;
   } else {
     forward_eval(p, s);
+    if (frozen) last_frozen_plan_ = &p;
   }
   head_forward(p, out, s);
 }
@@ -865,57 +940,25 @@ void Model::zero_ds_gradient_once(BlockPlan& bp, const BlockRef& br, bf16* T, cu
 
 void Model::backward(const float* d_out, int stage_begin, int stage_end, cudaStream_t s) {
   ARGUS_CHECK(grads_dev_ != nullptr, "model is not bound to a gradient arena");
+  ARGUS_CHECK(last_grad_forward_ != 2 || last_forward_frozen_,
+              "backward(): another forward() ran after the frozen-statistics forward it would differentiate");
   if (precision_ == 1) {
     backward_fp32(d_out, stage_begin, stage_end, s);
     return;
   }
+  if (last_grad_forward_ == 2) {
+    backward_frozen(*last_frozen_plan_, stage_begin, stage_end, d_out, s);
+    return;
+  }
   ARGUS_CHECK(last_train_plan_ != nullptr, "backward() needs a preceding training forward()");
   Plan& p = *last_train_plan_;
-  const int N = p.N, B = p.B, F = n_cams_ * out_dim_;
+  const int N = p.N;
   const int n_blocks = static_cast<int>(blocks_.size());
   // block index ranges per stage: stage 0 = layer4, 1 = layer3, 2 = layer2, 3 = layer1
   const int first_block[4] = {13, 7, 3, 0};
   const int last_block[4] = {16, 13, 7, 3};
   for (int stage = stage_begin; stage < stage_end; ++stage) {
-    if (stage == 0) {
-      // ---- head
-      ARGUS_CUDA(cudaMemcpyAsync(p.d_out, d_out, static_cast<size_t>(B) * 6 * sizeof(float),
-                                 cudaMemcpyDeviceToDevice, s)); pdl_break(s, kPdlAfterMemop);
-      float* g = grads_dev_;
-      // The chain only needs the input gradients; the three weight gradients (the 2048-wide layer alone is 0.15 ms of
-      // latency-bound fp32 SIMT work) read the finished output gradients and run on the weight-gradient side stream,
-      // which is idle here. Same kernels, same summation order: the gradients keep their bits.
-      linear_bwd_input(p.d_out, nullptr, params_dev_ + head_w_off_[2], p.d_a2, B, 128, 6, s);
-      linear_bwd_input(p.d_a2, p.h2, params_dev_ + head_w_off_[1], p.d_a1, B, 128, 128, s);
-      linear_bwd_input(p.d_a1, p.h1, params_dev_ + head_w_off_[0], p.d_z0, B, F, 128, s);
-      {
-        const float *d2 = p.d_out, *d1 = p.d_a2, *d0 = p.d_a1, *x2 = p.a2, *x1 = p.a1, *x0 = p.z0;
-        float *w2 = g + head_w_off_[2], *b2 = g + head_b_off_[2], *w1 = g + head_w_off_[1], *b1 = g + head_b_off_[1],
-              *w0 = g + head_w_off_[0], *b0 = g + head_b_off_[0];
-        run_on_side(s, [=](cudaStream_t ss) {
-          linear_bwd_weights(d2, x2, w2, b2, B, 128, 6, ss);
-          linear_bwd_weights(d1, x1, w1, b1, B, 128, 128, ss);
-          linear_bwd_weights(d0, x0, w0, b0, B, F, 128, ss);
-        });
-      }
-      gelu_bwd_bf16(p.d_z0, p.feat, p.d_feat, static_cast<int64_t>(B) * F, s);
-      // ---- fc
-      { ProfileScope prof("head", s, 0, 2.0 * N * out_dim_); }
-      // (the fc bias gradient -- one block column walking all N rows, 38 us -- feeds nothing in the chain either)
-      {
-        const bf16* dfeat = p.d_feat;
-        float* dbias = g + fc_bias_off_;
-        const int od = out_dim_;
-        run_on_side(s, [=](cudaStream_t ss) {
-          launch_kernel(colsum_bf16_kernel, (od + 127) / 128, 128, 0, ss, dfeat, dbias, N, od);
-          ARGUS_CUDA(cudaGetLastError());
-        });
-      }
-      run_wgrad(p.fc.wgrad, s);
-      Epilogue e;
-      for (const auto& l : p.fc.dgrad) launch_conv(l, e, s);
-      avgpool_bwd(p.d_pooled, p.blocks.back().g_out, p.blocks.back().out_bits, N, p.final_hw, 2048, s);
-    }
+    if (stage == 0) head_backward(p, d_out, s);
     for (int i = last_block[stage] - 1; i >= first_block[stage]; --i) {
       ARGUS_CHECK(i < n_blocks, "block index");
       BlockRef& br = blocks_[i];
@@ -982,16 +1025,187 @@ void Model::backward(const float* d_out, int stage_begin, int stage_end, cudaStr
       stem_grad_ready_ = true;   // p.g_raw0 now holds d loss / d (stem convolution output) for input_grad()
     }
     join_wgrad(s);
-    // packed 3x3 / stem gradients of this stage -> PyTorch layout in the gradient arena
-    {
-      int lo = -1, hi = -1;
-      for (size_t i = 0; i < pack_table_.size(); ++i)
-        if (pack_table_stage_[i] == stage) {
-          if (lo < 0) lo = static_cast<int>(i);
-          hi = static_cast<int>(i) + 1;
-        }
-      if (lo >= 0) unpack_wgrads(gpacked_, grads_dev_, pack_table_dev_ + lo, hi - lo, s);
+    unpack_stage_wgrads(stage, s);
+  }
+}
+
+// head MLP, fc and the global average pooling backward: d_out -> the masked output gradient of the last block
+void Model::head_backward(Plan& p, const float* d_out, cudaStream_t s) {
+  const int N = p.N, B = p.B, F = n_cams_ * out_dim_;
+  // ---- head
+  ARGUS_CUDA(cudaMemcpyAsync(p.d_out, d_out, static_cast<size_t>(B) * 6 * sizeof(float),
+                             cudaMemcpyDeviceToDevice, s)); pdl_break(s, kPdlAfterMemop);
+  float* g = grads_dev_;
+  // The chain only needs the input gradients; the three weight gradients (the 2048-wide layer alone is 0.15 ms of
+  // latency-bound fp32 SIMT work) read the finished output gradients and run on the weight-gradient side stream,
+  // which is idle here. Same kernels, same summation order: the gradients keep their bits.
+  linear_bwd_input(p.d_out, nullptr, params_dev_ + head_w_off_[2], p.d_a2, B, 128, 6, s);
+  linear_bwd_input(p.d_a2, p.h2, params_dev_ + head_w_off_[1], p.d_a1, B, 128, 128, s);
+  linear_bwd_input(p.d_a1, p.h1, params_dev_ + head_w_off_[0], p.d_z0, B, F, 128, s);
+  {
+    const float *d2 = p.d_out, *d1 = p.d_a2, *d0 = p.d_a1, *x2 = p.a2, *x1 = p.a1, *x0 = p.z0;
+    float *w2 = g + head_w_off_[2], *b2 = g + head_b_off_[2], *w1 = g + head_w_off_[1], *b1 = g + head_b_off_[1],
+          *w0 = g + head_w_off_[0], *b0 = g + head_b_off_[0];
+    run_on_side(s, [=](cudaStream_t ss) {
+      linear_bwd_weights(d2, x2, w2, b2, B, 128, 6, ss);
+      linear_bwd_weights(d1, x1, w1, b1, B, 128, 128, ss);
+      linear_bwd_weights(d0, x0, w0, b0, B, F, 128, ss);
+    });
+  }
+  gelu_bwd_bf16(p.d_z0, p.feat, p.d_feat, static_cast<int64_t>(B) * F, s);
+  // ---- fc
+  { ProfileScope prof("head", s, 0, 2.0 * N * out_dim_); }
+  // (the fc bias gradient -- one block column walking all N rows, 38 us -- feeds nothing in the chain either)
+  {
+    const bf16* dfeat = p.d_feat;
+    float* dbias = g + fc_bias_off_;
+    const int od = out_dim_;
+    run_on_side(s, [=](cudaStream_t ss) {
+      launch_kernel(colsum_bf16_kernel, (od + 127) / 128, 128, 0, ss, dfeat, dbias, N, od);
+      ARGUS_CUDA(cudaGetLastError());
+    });
+  }
+  run_wgrad(p.fc.wgrad, s);
+  Epilogue e;
+  for (const auto& l : p.fc.dgrad) launch_conv(l, e, s);
+  avgpool_bwd(p.d_pooled, p.blocks.back().g_out, p.blocks.back().out_bits, N, p.final_hw, 2048, s);
+}
+
+// packed 3x3 / stem gradients of this stage -> PyTorch layout in the gradient arena
+void Model::unpack_stage_wgrads(int stage, cudaStream_t s) {
+  int lo = -1, hi = -1;
+  for (size_t i = 0; i < pack_table_.size(); ++i)
+    if (pack_table_stage_[i] == stage) {
+      if (lo < 0) lo = static_cast<int>(i);
+      hi = static_cast<int>(i) + 1;
     }
+  if (lo >= 0) unpack_wgrads(gpacked_, grads_dev_, pack_table_dev_ + lo, hi - lo, s);
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// backward of a frozen-statistics (eval-mode) forward: every batch norm is the constant affine map sc * raw + shift, so
+// each convolution's backward is its weight-gradient GEMM on the masked output gradient g (H = g^T im2col(x), finished
+// by bn_frozen_finish into dW = diag(sc) H, dgamma, dbeta) and its dgrad of g against diag(sc) W. No batch-norm pass
+// over an activation remains. All work runs on the caller's stream, in a fixed order: deterministic.
+// ------------------------------------------------------------------------------------------------------------
+void Model::ensure_frozen_buffers() {
+  if (packed_scaled_ != nullptr) return;
+  // (plan-build time only) every stream of this model is idle
+  ARGUS_CUDA(cudaMalloc(&packed_scaled_, n_packed_ * sizeof(bf16)));
+  std::vector<WeightPackEntry> table;
+  std::vector<int64_t> scale_off;
+  int64_t h_elems = 0;
+  auto add = [&](const ConvRef& c) {
+    for (const auto& e : pack_table_)
+      if (e.dst_off == c.packed_off) table.push_back(e);
+    scale_off.push_back(c.bn.scratch_off);
+    if (c.shape.kind == 0 && c.shape.k == 1) h_elems = std::max<int64_t>(h_elems, static_cast<int64_t>(c.shape.Cout) * c.shape.Cin);
+  };
+  add(stem_);
+  for (const auto& b : blocks_) {
+    add(b.c1); add(b.c2); add(b.c3);
+    if (b.has_ds) add(b.ds);
+  }
+  ARGUS_CHECK(table.size() == scale_off.size(), "frozen-statistics pack table");
+  n_scaled_entries_ = static_cast<int>(table.size());
+  ARGUS_CUDA(cudaMalloc(&scaled_table_dev_, table.size() * sizeof(WeightPackEntry)));
+  ARGUS_CUDA(cudaMemcpy(scaled_table_dev_, table.data(), table.size() * sizeof(WeightPackEntry), cudaMemcpyHostToDevice));
+  ARGUS_CUDA(cudaMalloc(&scaled_scale_off_dev_, scale_off.size() * sizeof(int64_t)));
+  ARGUS_CUDA(cudaMemcpy(scaled_scale_off_dev_, scale_off.data(), scale_off.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
+  ARGUS_CUDA(cudaMalloc(&frz_h_, h_elems * sizeof(float)));
+  ARGUS_CUDA(cudaMalloc(&frz_pstats_, static_cast<size_t>(max_stat_slots_) * 2 * 2048 * sizeof(float)));
+  ARGUS_CUDA(cudaMalloc(&frz_gstats_, static_cast<size_t>(max_stat_slots_) * 2 * 512 * sizeof(float)));
+  ARGUS_CUDA(cudaMalloc(&frz_sums_, 2 * 2048 * sizeof(float)));
+  ARGUS_CUDA(cudaMalloc(&frz_partial_, 4LL * num_sms() * 2048 * sizeof(float)));
+  scaled_dirty_ = true;
+}
+
+void Model::frozen_wgrad_finish(const ConvRef& c, const WgradLaunch& l, float* h, const float* sums, int slots,
+                                int stride, float* dW, bool accumulate, cudaStream_t s) {
+  const int O = c.shape.Cout, K = c.shape.Ktot();
+  ARGUS_CUDA(cudaMemsetAsync(h, 0, static_cast<size_t>(O) * K * sizeof(float), s)); pdl_break(s, kPdlAfterMemop);
+  launch_wgrad(l, wgrad_scratch_, s);
+  const float* sc = bn_scratch_ + c.bn.scratch_off;
+  bn_frozen_finish(packed_ + c.packed_off, h, sums, slots, stride, sc, sc + 2 * O, sc + 3 * O, grads_dev_ + c.bn.gamma_off,
+                   grads_dev_ + c.bn.beta_off, dW, accumulate, O, K, s);
+}
+
+void Model::backward_frozen(Plan& p, int stage_begin, int stage_end, const float* d_out, cudaStream_t s) {
+  const int N = p.N;
+  const int first_block[4] = {13, 7, 3, 0};
+  const int last_block[4] = {16, 13, 7, 3};
+  float* g1_sum = frz_sums_ + 2048;   // sum of g1 (block loop), of g0 (stem)
+  for (int stage = stage_begin; stage < stage_end; ++stage) {
+    if (stage == 0) {
+      head_backward(p, d_out, s);
+      join_wgrad(s);   // the weight-gradient GEMMs below share the split-K scratch with the fc's
+      const BlockPlan& last = p.blocks.back();
+      colsum_rows_bf16(last.g_out, last.rows_out, blocks_.back().c3.shape.Cout, frz_partial_, frz_sums_, s);
+      frz_p_sum_ = frz_sums_; frz_p_slots_ = 1; frz_p_stride_ = 0;
+    }
+    for (int i = last_block[stage] - 1; i >= first_block[stage]; --i) {
+      BlockRef& br = blocks_[i];
+      BlockPlan& bp = p.blocks[i];
+      bf16 *P = bp.g_out, *R = bp.g_r, *T = bp.g_t;
+      const int wd = br.c1.shape.Cout;
+      // conv3 / bn3 and the downsample branch: H = P^T act, dW += diag(sc) H, dgamma, dbeta = sum P
+      frozen_wgrad_finish(br.c3, bp.c3.wgrad, frz_h_, frz_p_sum_, frz_p_slots_, frz_p_stride_, grads_dev_ + br.c3.w_off,
+                          true, s);
+      if (br.has_ds)
+        frozen_wgrad_finish(br.ds, bp.ds.wgrad, frz_h_, frz_p_sum_, frz_p_slots_, frz_p_stride_,
+                            grads_dev_ + br.ds.w_off, true, s);
+      // g2 = (P diag(sc3) W3) masked by act2's bits, with its column sums in the statistics slots
+      {
+        Epilogue e;
+        e.out_bits = bp.act2_bits;
+        e.stat_partial = frz_gstats_;
+        ARGUS_CHECK(bp.c3.dgrad.size() == 1, "conv3 dgrad: one launch");
+        const int slots = stat_slots(bp.c3.dgrad[0]);
+        ARGUS_CUDA(cudaMemsetAsync(frz_gstats_, 0, static_cast<size_t>(slots) * 2 * wd * sizeof(float), s)); pdl_break(s, kPdlAfterMemop);
+        launch_conv(bp.c3.dgrad[0], e, s);
+        // conv2 / bn2: H2 = g2^T im2col(act1) in the packed layout, scaled in place (unpacked at the end of the stage)
+        frozen_wgrad_finish(br.c2, bp.c2.wgrad, gpacked_ + br.c2.gpacked_off, frz_gstats_, slots, 2 * wd,
+                            gpacked_ + br.c2.gpacked_off, false, s);
+      }
+      if (br.has_ds) {
+        zero_ds_gradient_once(bp, br, T, s);
+        Epilogue e;
+        for (const auto& l : bp.ds.dgrad) launch_conv(l, e, s);   // T = P diag(scd) Wd
+      }
+      {
+        // g1 = (g2 diag(sc2) W2) masked by act1's bits (a separate pass: the stride-2 dgrad is one launch per parity
+        // class, and the bit mask of a dense 3x3 dgrad would need an epilogue instance of its own)
+        Epilogue e;
+        for (const auto& l : bp.c2.dgrad) launch_conv(l, e, s);
+        relu_bits_mask_colsum(R, bp.act1_bits, bp.rows_in, wd, frz_partial_, g1_sum, s);
+      }
+      frozen_wgrad_finish(br.c1, bp.c1.wgrad, frz_h_, g1_sum, 1, 0, grads_dev_ + br.c1.w_off, true, s);
+      {
+        // block-input gradient = g1 diag(sc1) W1 + the identity branch, masked by the previous block's ReLU bits; its
+        // column sums are the sum of P of the previous block
+        Epilogue e;
+        e.residual = br.has_ds ? T : P;
+        e.out_bits = i > 0 ? p.blocks[i - 1].out_bits : nullptr;
+        ARGUS_CHECK(bp.c1.dgrad.size() == 1, "conv1 dgrad: one launch");
+        if (i > 0) {
+          const int C = br.c1.shape.Cin;
+          frz_p_slots_ = stat_slots(bp.c1.dgrad[0]);
+          frz_p_stride_ = 2 * C;
+          frz_p_sum_ = frz_pstats_;
+          ARGUS_CUDA(cudaMemsetAsync(frz_pstats_, 0, static_cast<size_t>(frz_p_slots_) * 2 * C * sizeof(float), s)); pdl_break(s, kPdlAfterMemop);
+          e.stat_partial = frz_pstats_;
+        }
+        launch_conv(bp.c1.dgrad[0], e, s);
+      }
+    }
+    if (stage == 3) {
+      // stem: g0 = unpool(g_pooled) masked by [pooled0 > 0], then H0 = g0^T x (packed), scaled in place
+      stem_unpool_relu(p.g_stem_in, p.idx0, p.pooled0, p.g_raw0, N, p.H / 2, p.W / 2, frz_partial_, g1_sum, s);
+      frozen_wgrad_finish(stem_, p.stem.wgrad, gpacked_ + stem_.gpacked_off, g1_sum, 1, 0, gpacked_ + stem_.gpacked_off,
+                          false, s);
+      stem_grad_ready_ = true;   // p.g_raw0 = g0: input_grad() runs its dgrad against diag(sc0) W0
+    }
+    unpack_stage_wgrads(stage, s);
   }
 }
 
@@ -1004,6 +1218,12 @@ void Model::check_input_grad_ready(bool have_train_forward) const {
 void Model::input_grad(float* dx, cudaStream_t s) {
   if (precision_ == 1) {
     input_grad_fp32(dx, s);
+    return;
+  }
+  if (last_grad_forward_ == 2) {
+    check_input_grad_ready(last_frozen_plan_ != nullptr);
+    const Plan& p = *last_frozen_plan_;
+    stem_dgrad(p.g_raw0, packed_scaled_ + stem_.packed_off, dx, p.N, p.H, p.W, s);   // dRaw0 = sc0 g0
     return;
   }
   check_input_grad_ready(last_train_plan_ != nullptr);

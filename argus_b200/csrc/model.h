@@ -58,7 +58,8 @@ struct BlockPlan {
   ConvPlan c1, c2, c3, ds;
   bf16 *x = nullptr, *raw1 = nullptr, *act1 = nullptr, *raw2 = nullptr, *act2 = nullptr, *raw3 = nullptr,
        *rawd = nullptr, *out = nullptr;
-  uint8_t* out_bits = nullptr;   // ReLU mask of `out` (training): [rows_out][Cout/8] bytes
+  uint8_t* out_bits = nullptr;   // ReLU mask of `out` (training, frozen): [rows_out][Cout/8] bytes
+  uint8_t *act1_bits = nullptr, *act2_bits = nullptr;   // frozen plans: ReLU masks of act1 / act2
   int64_t rows_in = 0, rows_mid = 0, rows_out = 0;
   // gradient scratch roles for this block
   bf16 *g_out = nullptr, *g_q = nullptr, *g_r = nullptr, *g_t = nullptr, *g_x = nullptr;
@@ -87,6 +88,9 @@ struct BlockPlan {
 struct Plan {
   int B = 0, H = 0, W = 0, N = 0;
   bool training = false;
+  // Frozen-statistics plan (a differentiable eval-mode forward): the eval layout plus the ReLU bit masks, the max-pool
+  // arg-max bytes and the backward scratch; no pre-BN tensors. Its backward is Model::backward_frozen.
+  bool frozen = false;
   ConvPlan stem;
   bf16 *raw0 = nullptr, *act0 = nullptr, *pooled0 = nullptr;
   // The stem input is double buffered so that the NEXT batch can be augmented / staged (on another stream) while the
@@ -107,7 +111,7 @@ struct Plan {
   float *d_out = nullptr, *d_a2 = nullptr, *d_a1 = nullptr, *d_z0 = nullptr;
   bf16 *d_feat = nullptr, *d_pooled = nullptr;
   bf16* g_stem_in = nullptr;   // gradient wrt the pooled stem output (= layer1.0 input gradient)
-  bf16 *g_act0 = nullptr, *g_raw0 = nullptr;
+  bf16 *g_act0 = nullptr, *g_raw0 = nullptr;   // (frozen plans: g_raw0 = g0, the gradient wrt the stem's BN output)
 };
 
 struct Fp32State;                        // fp32 parity mode (model_fp32.cu)
@@ -126,18 +130,22 @@ class Model {
   void stage_param_range(int stage, int64_t* begin, int64_t* end) const;
 
   void bind(float* params, float* grads, float* buffers);
-  void reserve(int max_batch, int H, int W, bool training);
+  void reserve(int max_batch, int H, int W, bool training, bool frozen = false);
   void sync_weights(cudaStream_t s);   // fp32 parameters -> packed bf16 (+ marks the eval BN fold dirty)
 
   // x: (B, 3*n_cams, H, W) fp32 NCHW in [0,1], or u8 (B*n_cams, H, W, 3) when is_u8. out: (B, 6) fp32.
-  void forward(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s);
+  // frozen (training == false): the eval-mode forward with the same output bits, made differentiable by backward() /
+  // input_grad() with the running statistics as constants; nothing the model keeps between passes changes.
+  void forward(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s,
+               bool frozen = false);
   // Augmentation fused with input staging: uint8 (B*n_cams, H, W, 3) images -> augmented bf16 stem input of the plan
   // for (B, H, W, training). A following forward() with x == nullptr consumes it.
   // arc_mask (nullable): spaghetti arcs as 1 bit per pixel; plasma_ws: workspace of B * n_cams * H * W / 8 bytes
   void stage_input_u8(const uint8_t* images, const float* aug_params, const uint32_t* arc_mask, uint32_t* plasma_ws, int B,
                       int H, int W, bool training, bool apply, cudaStream_t s);
   // d_out: (B, 6) gradient of the loss wrt forward()'s output. Accumulates parameter gradients (+=) into the bound
-  // gradient arena for stages [stage_begin, stage_end); stages must be run in increasing order 0..3.
+  // gradient arena for stages [stage_begin, stage_end); stages must be run in increasing order 0..3. Differentiates the
+  // last training or frozen forward, whichever ran last; a frozen one must still be the last forward of all.
   void backward(const float* d_out, int stage_begin, int stage_end, cudaStream_t s);
   void zero_grads(cudaStream_t s);
   // d loss / d x of the last training forward (whose input was the fp32 tensor x) once backward() has run stage 3:
@@ -159,12 +167,19 @@ class Model {
 
  private:
   void build_layout();
-  Plan& get_plan(int B, int H, int W, bool training);
+  Plan& get_plan(int B, int H, int W, bool training, bool frozen = false);
   void build_plan(Plan& p);
   void fold_eval(cudaStream_t s);
   void forward_train(Plan& p, cudaStream_t s);
   void forward_eval(Plan& p, cudaStream_t s);
   void head_forward(Plan& p, float* out, cudaStream_t s);
+  void head_backward(Plan& p, const float* d_out, cudaStream_t s);
+  void unpack_stage_wgrads(int stage, cudaStream_t s);
+  // frozen-statistics backward (see bn_algebra.cu): weight gradient H of c into h (zeroed here), then the finish
+  void frozen_wgrad_finish(const ConvRef& c, const WgradLaunch& l, float* h, const float* sums, int slots, int stride,
+                           float* dW, bool accumulate, cudaStream_t s);
+  void backward_frozen(Plan& p, int stage_begin, int stage_end, const float* d_out, cudaStream_t s);
+  void ensure_frozen_buffers();
   void run_conv_train(const ConvPlan& cp, const ConvRef& c, int64_t rows, cudaStream_t s);
   // batch statistics of the 1x1 convolution c from the Gram matrix of its input (gram launch + colsum) -> BN scratch
   void stats_from_gram(const ConvRef& c, const WgradLaunch& gram, float* G, const bf16* act, const float* colsum_partial,
@@ -193,7 +208,8 @@ class Model {
   // fp32 parity mode
   void plan_fp32(Fp32State& st, int B, int H, int W, bool training);
   Fp32State& fp32_state(int B, int H, int W, bool training);
-  void forward_fp32(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s);
+  void forward_fp32(const void* x, bool is_u8, int B, int H, int W, bool training, bool frozen, float* out,
+                    cudaStream_t s);
   void backward_fp32(const float* d_out, int stage_begin, int stage_end, cudaStream_t s);
   void input_grad_fp32(float* dx, cudaStream_t s);
   void check_input_grad_ready(bool have_train_forward) const;
@@ -240,17 +256,34 @@ class Model {
   std::vector<WeightPackEntry> pack_table_;
   std::vector<int> pack_table_stage_;
   bool eval_fold_dirty_ = true;
+  // frozen-statistics backward: diag(sc) W in the packed layout (refreshed after every eval fold), its pack table
+  // (every BN-followed convolution; scale offsets into bn_scratch_), and scratch
+  bf16* packed_scaled_ = nullptr;
+  WeightPackEntry* scaled_table_dev_ = nullptr;
+  int64_t* scaled_scale_off_dev_ = nullptr;
+  int n_scaled_entries_ = 0;
+  bool scaled_dirty_ = true;
+  float* frz_h_ = nullptr;        // H = g^T x of the 1x1 convolutions, [Cout][Cin]
+  float* frz_pstats_ = nullptr;   // [max_stat_slots_][2][2048] statistics slots of the conv1 dgrads: sum of P
+  float* frz_gstats_ = nullptr;   // [max_stat_slots_][2][512] statistics slots of the conv3 dgrads: sum of g2
+  float* frz_sums_ = nullptr;     // [2][2048] finished column sums: sum of P (last block), sum of g1 / g0
+  float* frz_partial_ = nullptr;  // per-block column-sum partials, 4 * num_sms * 2048 floats
+  const float* frz_p_sum_ = nullptr;   // where the sum of the current block's output gradient P lives
+  int frz_p_slots_ = 0, frz_p_stride_ = 0;
 
   uint8_t* arena_ = nullptr;
   size_t arena_bytes_ = 0, arena_used_ = 0;
   int reserved_batch_ = 0, reserved_h_ = 0, reserved_w_ = 0;
   bool reserved_training_ = false;
-  std::map<std::tuple<int, int, int, bool>, std::unique_ptr<Plan>> plans_;
+  std::map<std::tuple<int, int, int, bool, bool>, std::unique_ptr<Plan>> plans_;
   Plan* last_train_plan_ = nullptr;
+  Plan* last_frozen_plan_ = nullptr;
+  int last_grad_forward_ = 0;      // 0: none, 1: training, 2: frozen -- the forward backward() differentiates
+  bool last_forward_frozen_ = false;   // the most recent forward of any kind was a frozen one
   Plan* last_plan_ = nullptr;
   uint64_t arena_epoch_ = 1;   // bumped whenever another plan (they share the arena) runs a forward pass
   Plan* staged_plan_ = nullptr;
-  bool train_input_f32_ = false;   // the last training forward read an fp32 image tensor (not u8 / a staged batch)
+  bool train_input_f32_ = false;   // the last training / frozen forward read an fp32 image tensor (not u8 / staged)
   bool stem_grad_ready_ = false;   // backward() stage 3 ran after the last forward(): the stem's output gradient is live
   // stem input double buffer (see Plan): [n][H/2][W/2 + 4][16] bf16 each; cur_in_ = the buffer the last forward consumed
   bf16* stem_in_[2] = {nullptr, nullptr};

@@ -29,6 +29,7 @@ struct Fp32State {
   size_t arena_bytes = 0, used = 0;
   int B = 0, H = 0, W = 0, N = 0;
   bool training = false, planned = false, have_train_forward = false;
+  bool frozen = false;   // the last forward was a frozen-statistics (differentiable eval-mode) one
   float* x_nhwc = nullptr;
   UnitF32 stem;
   float* pooled0 = nullptr;
@@ -156,8 +157,10 @@ Fp32State& Model::fp32_state(int B, int H, int W, bool training) {
   return st;
 }
 
-void Model::forward_fp32(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s) {
-  Fp32State& st = fp32_state(B, H, W, training);
+// frozen: the eval-mode computation (running statistics folded), on a state that keeps the backward buffers
+void Model::forward_fp32(const void* x, bool is_u8, int B, int H, int W, bool training, bool frozen, float* out,
+                         cudaStream_t s) {
+  Fp32State& st = fp32_state(B, H, W, training || frozen);
   const int N = st.N;
   const float* P = params_dev_;
   float* BUF = buffers_dev_;
@@ -212,7 +215,8 @@ void Model::forward_fp32(const void* x, bool is_u8, int B, int H, int W, bool tr
   linear_fwd(st.a1, P + head_w_off_[1], P + head_b_off_[1], st.h2, st.a2, B, 128, 128, s);
   linear_fwd(st.a2, P + head_w_off_[2], P + head_b_off_[2], st.out, nullptr, B, 128, 6, s);
   ARGUS_CUDA(cudaMemcpyAsync(out, st.out, static_cast<size_t>(B) * 6 * sizeof(float), cudaMemcpyDeviceToDevice, s)); pdl_break(s, kPdlAfterMemop);
-  st.have_train_forward = training;
+  st.have_train_forward = training || frozen;
+  st.frozen = frozen;
 }
 
 void Model::backward_fp32(const float* d_out, int stage_begin, int stage_end, cudaStream_t s) {
@@ -226,8 +230,9 @@ void Model::backward_fp32(const float* d_out, int stage_begin, int stage_end, cu
                     int64_t rows) {
     const float* sc = SC(c);
     const int C = c.bn.C;
+    // (frozen: mean / invstd are the running statistics bn_fold_eval left in the scratch, and dx = sc * g)
     bn_f32_backward(dy, raw, out, sc, sc + 2 * C, sc + 3 * C, g + c.bn.gamma_off, g + c.bn.beta_off, dx, g_out, rows, C,
-                    st.bn_partial, st.bn_sums, s);
+                    st.bn_partial, st.bn_sums, s, st.frozen);
   };
   auto conv_bwd = [&](const ConvRef& c, const float* dy, const float* in, float* dx, int n, int h, int w) {
     const ConvShapeF32 cs = shape_of(c, n, h, w);

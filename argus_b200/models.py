@@ -8,9 +8,13 @@ Differences that are deliberate and documented in DESIGN.md:
     (no CPU fallback: calling the module with CPU tensors raises);
   * H and W must be powers of two >= 32 (the reference's default 256x256 and its 128x128 crop test both are).
 
-Gradients flow to the parameters and to the input images of a train-mode forward, as with the reference: with
-`x.requires_grad_()`, `loss.backward()` fills `x.grad` (the stem's transposed convolution runs on the tensor cores,
-argus_model_input_grad), also when every parameter is frozen. An eval-mode forward builds no graph.
+Gradients flow to the parameters and to the input images, as with the reference: with `x.requires_grad_()`,
+`loss.backward()` fills `x.grad` (the stem's transposed convolution runs on the tensor cores, argus_model_input_grad),
+also when every parameter is frozen. A train-mode forward uses batch statistics. An eval-mode forward made with grad
+enabled, while x or a parameter requires grad, is differentiable with the running statistics as constants
+(argus_model_forward_frozen): its output is bit for bit the no-grad eval output, and it updates no running statistic
+and no num_batches_tracked. This serves adversarial examples against the deployed network, fine-tuning with frozen
+batch norm (also at batch size 1) and saliency maps. Under torch.no_grad() an eval-mode forward builds no graph.
 """
 from __future__ import annotations
 
@@ -93,15 +97,14 @@ class _ModelHandle:
 
 
 class _NCameraCNNFunction(torch.autograd.Function):
-    """Whole-network autograd node: forward = argus_model_forward, backward = argus_model_backward (+
-    argus_model_input_grad when x requires grad)."""
+    """Whole-network autograd node: forward = argus_model_forward (train mode) or argus_model_forward_frozen (eval
+    mode), backward = argus_model_backward (+ argus_model_input_grad when x requires grad)."""
 
     @staticmethod
     def forward(ctx, model: "NCameraCNN", x: torch.Tensor, *params: torch.Tensor) -> torch.Tensor:
         training = model.training
-        out = model._forward_impl(x, training)
+        out = model._forward_impl(x, training, frozen=not training)
         ctx.model = model
-        ctx.is_train_forward = training
         ctx.n_params = len(params)
         ctx.x_shape, ctx.x_dtype = x.shape, x.dtype
         return out
@@ -109,8 +112,6 @@ class _NCameraCNNFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, grad_out: torch.Tensor):
         model = ctx.model
-        if not ctx.is_train_forward:
-            raise RuntimeError("argus_b200: gradients are only available for a forward pass made in train() mode")
         grads = model._backward_impl(grad_out, ctx.needs_input_grad[2:])
         dx = model._input_grad_impl(ctx.x_shape).to(ctx.x_dtype) if ctx.needs_input_grad[1] else None
         return (None, dx) + tuple(grads)
@@ -308,7 +309,8 @@ class NCameraCNN(nn.Module):
 
     def _forward_impl(self, x: torch.Tensor, training: bool, aug_params: Optional[torch.Tensor] = None,
                       augment: bool = False, arc_mask: Optional[torch.Tensor] = None,
-                      plasma_ws: Optional[torch.Tensor] = None) -> torch.Tensor:
+                      plasma_ws: Optional[torch.Tensor] = None, frozen: bool = False) -> torch.Tensor:
+        """frozen (eval mode only): the differentiable eval-mode forward, argus_model_forward_frozen."""
         self._ensure_bound()
         if x.device != self._flat_params.device:
             raise _lib.ArgusError(f"input is on {x.device} but the model is on {self._flat_params.device}")
@@ -326,7 +328,10 @@ class NCameraCNN(nn.Module):
         self.sync_weights()
         out = torch.empty((B, 6), dtype=torch.float32, device=x.device)
         with torch.cuda.device(x.device):
-            if is_u8 and (augment or arc_mask is not None):
+            if frozen:
+                _lib.call("argus_model_forward_frozen", self._handle.ptr, x, int(is_u8), int(B), int(H), int(W), out,
+                          _lib.stream_ptr())
+            elif is_u8 and (augment or arc_mask is not None):
                 # fused staging: arcs (bit mask) + augmentation (when `augment`) + /255 + bf16 space-to-depth packing
                 if augment and plasma_ws is None:
                     plasma_ws = torch.empty((B * self.n_cams, H, W // 32), dtype=torch.int32, device=x.device)
@@ -353,7 +358,8 @@ class NCameraCNN(nn.Module):
         return out
 
     def _backward_impl(self, grad_out: torch.Tensor, needs_grad=None) -> list[Optional[torch.Tensor]]:
-        """Parameter gradients of the last training forward; None for parameters whose `needs_grad` entry is False."""
+        """Parameter gradients of the last training or frozen forward; None for parameters whose `needs_grad` entry is
+        False."""
         g = grad_out.contiguous().to(torch.float32)
         with torch.cuda.device(g.device):
             _lib.call("argus_model_zero_grads", self._handle.ptr, _lib.stream_ptr())
@@ -365,7 +371,7 @@ class NCameraCNN(nn.Module):
                 for need, (_n, off, numel, shape) in zip(needs_grad, self._param_infos)]
 
     def _input_grad_impl(self, shape) -> torch.Tensor:
-        """d loss / d x (fp32, `shape` = the input's) of the last training forward, after _backward_impl."""
+        """d loss / d x (fp32, `shape` = the input's) of the last training or frozen forward, after _backward_impl."""
         dx = torch.empty(shape, dtype=torch.float32, device=self._flat_params.device)
         with torch.cuda.device(dx.device):
             _lib.call("argus_model_input_grad", self._handle.ptr, dx, _lib.stream_ptr())
@@ -399,6 +405,6 @@ class NCameraCNN(nn.Module):
         """
         assert len(x.shape) == 4 or x.dtype == torch.uint8, \
             "The input images must be of shape (B, C, H, W)! If B=1, add a dummy dimension."
-        if torch.is_grad_enabled() and self.training and (x.requires_grad or any(p.requires_grad for p in self._param_list)):
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self._param_list)):
             return _NCameraCNNFunction.apply(self, x, *self._param_list)
         return self._forward_impl(x, self.training)

@@ -42,7 +42,8 @@ def get_pose(images: torch.Tensor, model: torch.nn.Module) -> torch.Tensor:
         pose: The predicted pose as a 7d pose (x, y, z, qx, qy, qz, qw). The reference returns a pypose SE3
             LieTensor; pypose is not a dependency here, so a plain (B, 7) tensor with the same data is returned.
     """
-    return se3_exp(model(images))
+    with torch.no_grad():   # inference: se3_exp detaches anyway, and an eval-mode forward with grad builds a graph
+        return se3_exp(model(images))
 
 
 def time_torch_fn(fn: Callable[[], torch.Tensor]) -> tuple[torch.Tensor, float]:

@@ -278,6 +278,28 @@ int argus_model_sync_weights(argus_model* m, void* stream);
  * is_u8. training != 0 uses batch statistics and updates the running statistics. out is (B, 6) fp32. */
 int argus_model_forward(argus_model* m, const void* x, int is_u8, int B, int H, int W, int training, float* out,
                         void* stream);
+/* Frozen-statistics backward primitives (see argus_model_forward_frozen; exposed for tests):
+ * argus_bn_frozen_finish: one convolution's finish from H = g^T im2col(x) [O][K] fp32 and its bf16 weight W [O][K] in
+ *   the same layout: dgamma += invstd * (rowdot(W, H) - mean * sum g), dbeta += sum g, dW = (accumulate ? dW : 0) +
+ *   diag(scale) H (dW may be H). sum g = stat_partial summed over `slots` rows of stride stat_stride, in fp64.
+ * argus_relu_bits_mask_colsum: g (rows, C) bf16 masked in place by ReLU bits [rows][C/8]; out[c] = column sums.
+ * argus_stem_unpool_relu: g0 (N, H, W, 64) = max-unpooled dpool (N, H/2, W/2, 64) through the arg-max bytes, masked by
+ *   pooled > 0; out[64] = column sums of g0.
+ * argus_pack_weight_scaled: bf16_rn(scale[co] * w) of a PyTorch-layout fp32 weight in the packed layout of the
+ *   convolutions (kind 0: [Cout][k][k][Cin]; kind 1: the [64][256] stem). */
+int argus_bn_frozen_finish(const void* W, const float* H, const float* stat_partial, int slots, int stat_stride,
+                           const float* scale, const float* mean, const float* invstd, float* dgamma, float* dbeta,
+                           float* dW, int accumulate, int O, int K, void* stream);
+int argus_relu_bits_mask_colsum(void* g, const void* bits, int64_t rows, int C, float* out, void* stream);
+int argus_stem_unpool_relu(const void* dpool, const void* idx, const void* pooled, void* g0, int N, int H, int W,
+                           float* out, void* stream);
+int argus_pack_weight_scaled(const float* w, const float* scale, void* packed, int Cout, int Cin, int k, int kind,
+                             void* stream);
+/* Eval-mode forward that can be differentiated: the running statistics are constants, the output is bit for bit that of
+ * argus_model_forward(training = 0), and the running statistics, num_batches_tracked and the training input buffers
+ * are left as they are. argus_model_backward and argus_model_input_grad (fp32 x only) then differentiate it, as long as
+ * no other forward has run since. x as for argus_model_forward (no staged input). */
+int argus_model_forward_frozen(argus_model* m, const void* x, int is_u8, int B, int H, int W, float* out, void* stream);
 /* Fused augmentation + input staging: u8 (B*n_cams, H, W, 3) -> augmented stem input inside the model (training: one
  * of two model-owned staging buffers, so the NEXT batch -- of any size -- can be staged on another stream while the
  * current step runs). The next argus_model_forward call for the same (B, H, W, training) passes x = NULL.
@@ -294,10 +316,11 @@ int argus_model_set_precision(argus_model* m, int mode);
  * caller's stream (joined before the stage returns). on = 0 serialises them (used for per-kernel timing). */
 int argus_model_set_wgrad_overlap(argus_model* m, int on);
 int argus_model_zero_grads(argus_model* m, void* stream);
-/* Backward of the last training forward. d_out (B,6). Stages 0..3 (head+fc+layer4, layer3, layer2, layer1+stem)
+/* Backward of the last training or frozen-statistics forward (whichever ran later; an error when another forward ran
+ * after a frozen one). d_out (B,6). Stages 0..3 (head+fc+layer4, layer3, layer2, layer1+stem)
  * must run in order; gradients are ADDED into the bound gradient arena. */
 int argus_model_backward(argus_model* m, const float* d_out, int stage_begin, int stage_end, void* stream);
-/* d loss / d x for the last training forward whose input was the fp32 tensor x (B, 3*n_cams, H, W); call after
+/* d loss / d x for the last training (or frozen-statistics) forward whose input was the fp32 tensor x (B, 3*n_cams, H, W); call after
  * argus_model_backward has run stage 3. dx: (B, 3*n_cams, H, W) fp32, overwritten. Image n = b*n_cams + v is channels
  * [3v, 3v+3) of sample b; the gradient passes straight through the bf16 rounding of the input. Errors (non-zero status,
  * message): no training forward, backward stage 3 not run since it, or the forward consumed a staged / uint8 input. */
