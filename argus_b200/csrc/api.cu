@@ -83,7 +83,7 @@ int argus_conv2d_stat_slots(int N, int H, int W, int Cin, int Cout, int k, int s
   const int64_t m_tiles = (s.out_pixels() + kBlockM - 1) / kBlockM;
   // same tile choice as plan_conv_forward: an upper bound is enough for sizing
   const int64_t tiles = m_tiles * ((Cout + 63) / 64);
-  *slots = 4 * static_cast<int>(std::min<int64_t>(tiles, num_sms()));   // up to four epilogue groups per CTA
+  *slots = kEpiGroups * static_cast<int>(std::min<int64_t>(tiles, num_sms()));   // one per epilogue group per CTA
   ARGUS_API_END
 }
 

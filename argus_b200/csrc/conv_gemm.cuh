@@ -21,7 +21,8 @@ namespace argus {
 
 constexpr int kBlockM = 128;
 constexpr int kBlockK = 64;  // bf16 elements = 128 bytes = one swizzle atom row
-constexpr int kNumThreads = 320;       // conv kernel: TMA warp, MMA warp, 2 x 4 epilogue warps
+constexpr int kEpiGroups = 2;          // conv kernel: epilogue groups of four warps, one per TMEM accumulator stage
+constexpr int kNumThreads = 64 + 128 * kEpiGroups;   // conv kernel: TMA warp, MMA warp, the epilogue groups
 constexpr int kWgradThreads = 192;     // wgrad kernel: TMA warp, MMA warp, 4 epilogue warps
 constexpr int kMaxTaps = 16;
 
@@ -51,11 +52,10 @@ struct ConvGemmParams {
   const float* scale;            // per output channel multiplier (folded BN)
   const float* shift;            // per output channel offset (folded BN / bias)
   int has_res;                   // add the residual tile (TMA-loaded through res_map) before ReLU
-  // Weights resident in shared memory: when the whole [BLOCK_N x K] weight slab of the CTA's (fixed) N tile fits next
-  // to >= 3 activation stages, it is loaded once per CTA instead of once per M tile; the stage ring then carries the
-  // activation tiles only (res_stages of them). Cuts the L2 -> SM traffic of the small-K layers by 1/3 .. 2/3.
+  // Weights resident in shared memory (halo mode only, set by finish_params): when the CTA's N tile never changes and
+  // its whole [BLOCK_N x K] weight slab fits next to two halo boxes (layer1 3x3: 72 KB), the slab is loaded once per CTA
+  // instead of once per M tile and a halo stage carries the activation box only.
   int b_resident;
-  int res_stages;
   // Halo mode (3x3, stride 1, tile inside one image): instead of nine [128 x 64] activation boxes per 64-channel
   // block (one per tap, each re-read from L2), three boxes of (rows + 2) image rows are loaded -- one per horizontal
   // shift dw -- and the three vertical taps are row offsets into the same shared-memory box. Activation traffic from
@@ -96,37 +96,32 @@ struct ConvGemmParams {
 // NBUF = staging buffers per epilogue group. Two let the store of chunk i overlap the math of chunk i + 1 (and carry the
 // prefetched residual tile); a BLOCK_N = 64 tile has a single chunk, so without a residual one buffer is enough (the
 // group's next chunk is a whole tile later) and the 32 KB go to the operand pipeline (a third halo stage on layer1 3x3).
-// EPI = 4 is the split-tile mode (see conv_gemm_kernel): two groups share one 256-wide tile, each owns one buffer.
-template <int BLOCK_N, int OPT, int EPI = 2>
-constexpr int conv_staging_buffers() { return (EPI == 4 || (BLOCK_N == 64 && !(OPT & 2))) ? 1 : 2; }
+template <int BLOCK_N, int OPT>
+constexpr int conv_staging_buffers() { return (BLOCK_N == 64 && !(OPT & 2)) ? 1 : 2; }
 
-template <int BLOCK_N, int EPI = 2, int NBUF = 2>
+template <int BLOCK_N, int NBUF = 2>
 struct ConvGemmSmem {
   static constexpr int kABytes = kBlockM * kBlockK * 2;          // 16 KB
   static constexpr int kBBytes = BLOCK_N * kBlockK * 2;          // 8..32 KB
   static constexpr int kStageBytes = kABytes + kBBytes;
   static constexpr int kStagingBytes = kBlockM * 128;            // one 64-column bf16 chunk of the tile
-  static constexpr int kGroupCols = (EPI == 4) ? BLOCK_N / 2 : BLOCK_N;   // columns of a tile one epilogue group finishes
-  static constexpr int kStatsBytes = EPI * 4 * 2 * kGroupCols * 4;  // per group, per warp: sum[cols], sqsum[cols]
+  static constexpr int kStatsBytes = kEpiGroups * 4 * 2 * BLOCK_N * 4;  // per group, per warp: sum[cols], sqsum[cols]
   // operand pipeline region: everything the 227 KB of shared memory leave after staging, statistics and barriers
-  static constexpr int kPipeBytes = (232448 - 1024 - NBUF * EPI * kStagingBytes - kStatsBytes - 512) / 1024 * 1024;
+  static constexpr int kPipeBytes = (232448 - 1024 - NBUF * kEpiGroups * kStagingBytes - kStatsBytes - 512) / 1024 * 1024;
   static constexpr int kStagesRaw = kPipeBytes / kStageBytes;
   static constexpr int kStages = kStagesRaw > 6 ? 6 : kStagesRaw;
   static constexpr int kOffStaging = kPipeBytes;                 // NBUF staging buffers per epilogue group
-  static constexpr int kOffStats = kOffStaging + NBUF * EPI * kStagingBytes;
+  static constexpr int kOffStats = kOffStaging + NBUF * kEpiGroups * kStagingBytes;
   static constexpr int kOffBars = kOffStats + kStatsBytes;
-  static constexpr int kMaxStages = 8;               // stage ring length in weights-resident mode (<= kMaxStages)
-  // full/empty per stage, accumulator-full per epilogue GROUP, accumulator-empty per TMEM stage,
-  // residual x(EPI groups x 2 buffers), resident-weights barrier
-  static constexpr int kNumBars = 2 * kMaxStages + EPI + 2 + 2 * EPI + 1;
+  static constexpr int kMaxStages = 8;               // longest stage ring (halo mode; the streaming ring has kStages)
+  // full/empty per stage, accumulator-full and accumulator-empty per TMEM stage, residual x (groups x 2 buffers),
+  // resident-weights barrier
+  static constexpr int kNumBars = 2 * kMaxStages + kEpiGroups + 2 + 2 * kEpiGroups + 1;
   static constexpr int kOffTmemPtr = kOffBars + kNumBars * 8;
   static constexpr int kTotal = kOffTmemPtr + 16;
 };
 
-// EPI = number of epilogue groups (4 warps each): 2 for tensor-bound shapes (3 pipeline stages at N = 256), 3 for the
-// wide, shallow-K layers whose tile time is set by the epilogue (TMEM -> math -> smem -> TMA store + statistics), which
-// is latency-bound per warp: a third group raises the epilogue throughput by half. The two TMEM accumulator stages are
-// shared: CTA-local tile t uses stage t % 2 and is finished by group t % EPI.
+// Epilogue group g (four warps) finishes the CTA-local tiles g, g + 2, ..., all of which use TMEM accumulator stage g.
 // OPT = compile-time mask of the epilogue options a kernel instance can honour (kOptAll = the generic kernel). Options
 // outside the mask are compiled out, which removes their per-chunk flag tests (constant-bank loads + dependent branches)
 // and most of the instruction-cache footprint of the chunk loop. OPT = 0 ("plain": store the bf16 tile, optional
@@ -139,20 +134,13 @@ constexpr int kOptRelu = 8;      // ReLU, ReLU bit-mask output
 constexpr int kOptResExtra = 16; // bit mask on the residual, residual scale / shift (needs kOptRes)
 constexpr int kOptBnRed = 32;    // fused batch-norm backward reduction (needs kOptRes: the raw tile rides the residual path)
 constexpr int kOptAll = 31;      // the generic kernel (kOptBnRed only exists in specialised instances)
-template <int BLOCK_N, int B_MN, int EPI, int OPT = kOptAll>
-__global__ void __launch_bounds__(64 + 128 * EPI, 1)
+template <int BLOCK_N, int B_MN, int OPT = kOptAll>
+__global__ void __launch_bounds__(kNumThreads, 1)
 conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
   pdl_begin(p.early_trigger);
-  constexpr int NBUF = conv_staging_buffers<BLOCK_N, OPT, EPI>();
+  constexpr int NBUF = conv_staging_buffers<BLOCK_N, OPT>();
   static_assert(NBUF == 2 || !(OPT & kOptRes), "the residual prefetch needs two staging buffers");
-  // Split-tile mode (EPI == 4, BLOCK_N == 256): the two TMEM accumulator stages bound the tiles in flight, so instead of
-  // a third tile the four groups work in PAIRS on one tile -- groups 2t and 2t+1 finish the left / right 128 columns of
-  // the tile in accumulator stage t. Sixteen epilogue warps instead of eight on the layers whose tile time is set by the
-  // epilogue (wide, shallow-K, HBM-bound). One staging buffer per group (same 64 KB as two groups x two buffers).
-  constexpr bool SPLIT = (EPI == 4);
-  constexpr int kTileGroups = SPLIT ? 2 : EPI;   // tile epilogues in flight
-  static_assert(!SPLIT || (BLOCK_N == 256 && !(OPT & kOptRes)), "split-tile mode: 256-wide tiles without residual");
-  using L = ConvGemmSmem<BLOCK_N, EPI, NBUF>;
+  using L = ConvGemmSmem<BLOCK_N, NBUF>;
   constexpr int kStages = L::kStages;
   constexpr int kTmemCols = (2 * BLOCK_N) < 32 ? 32 : (2 * BLOCK_N);
   static_assert(BLOCK_N == 64 || BLOCK_N == 128 || BLOCK_N == 256, "BLOCK_N");
@@ -166,23 +154,21 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
   const uint32_t bar_base = smem_base + L::kOffBars;
   auto full_bar = [&](int s) { return bar_base + 8u * s; };
   auto empty_bar = [&](int s) { return bar_base + 8u * (kMaxStages + s); };
-  // "accumulator full" is signalled per epilogue GROUP (each group then sees strictly alternating phases of its own
-  // barrier; a per-stage barrier would let a group whose first tile is the stage's SECOND use pass its parity-1 wait
-  // at kernel start), "accumulator empty" per TMEM stage (single waiter: the MMA warp)
-  auto tfull_bar = [&](int g) { return bar_base + 8u * (2 * kMaxStages + g); };
-  auto tempty_bar = [&](int s) { return bar_base + 8u * (2 * kMaxStages + EPI + s); };
-  auto res_bar = [&](int g, int b) { return bar_base + 8u * (2 * kMaxStages + EPI + 2 + 2 * g + b); };
-  const uint32_t bres_bar = bar_base + 8u * (2 * kMaxStages + EPI + 2 + 2 * EPI);
+  // "accumulator full" (single waiter: the epilogue group of that stage) and "accumulator empty" (single waiter: the MMA
+  // warp) per TMEM stage
+  auto tfull_bar = [&](int s) { return bar_base + 8u * (2 * kMaxStages + s); };
+  auto tempty_bar = [&](int s) { return bar_base + 8u * (2 * kMaxStages + kEpiGroups + s); };
+  auto res_bar = [&](int g, int b) { return bar_base + 8u * (2 * kMaxStages + kEpiGroups + 2 + 2 * g + b); };
+  const uint32_t bres_bar = bar_base + 8u * (2 * kMaxStages + kEpiGroups + 2 + 2 * kEpiGroups);
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem + L::kOffTmemPtr);
   float* s_stats_all = reinterpret_cast<float*>(smem + L::kOffStats);
-  // pipeline geometry: streaming mode = kStages x (A | B); weights-resident mode = res_stages x A, then the B slab
+  // pipeline geometry: streaming mode = kStages x (A | B); halo mode = halo_stages x (box | 3 B), or with the weights
+  // resident (b_resident, halo mode only) halo_stages x box followed by the weight slab
   const bool resident = (p.b_resident != 0);
   const bool halo = (p.halo != 0);
   const uint32_t halo_a_bytes = static_cast<uint32_t>(p.halo_rows + 2) * p.halo_row_bytes;
-  const int nstages = halo ? p.halo_stages : (resident ? p.res_stages : kStages);
-  // halo + resident (layer1 3x3: the whole 72 KB weight slab stays in shared memory): a stage is the activation box only
-  const uint32_t stage_bytes = halo ? halo_a_bytes + (resident ? 0u : 3u * L::kBBytes)
-                                    : (resident ? L::kABytes : L::kStageBytes);
+  const int nstages = halo ? p.halo_stages : kStages;
+  const uint32_t stage_bytes = halo ? halo_a_bytes + (resident ? 0u : 3u * L::kBBytes) : L::kStageBytes;
   const uint32_t bres_base = smem_base + static_cast<uint32_t>(nstages) * stage_bytes;
 
   if (threadIdx.x == 0) {
@@ -192,8 +178,8 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
       mbar_init(empty_bar(s), 1);
     }
     mbar_init(bres_bar, 1);
-    for (int s = 0; s < 2; ++s) mbar_init(tempty_bar(s), SPLIT ? 8 : 4);  // one arrive per epilogue warp finishing the tile
-    for (int g = 0; g < EPI; ++g) {
+    for (int s = 0; s < 2; ++s) mbar_init(tempty_bar(s), 4);  // one arrive per epilogue warp finishing the tile
+    for (int g = 0; g < kEpiGroups; ++g) {
       mbar_init(tfull_bar(g), 1);
       mbar_init(res_bar(g, 0), 1);
       mbar_init(res_bar(g, 1), 1);
@@ -211,7 +197,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
     tmem_alloc(smem_u32(const_cast<uint32_t*>(tmem_ptr_smem)), kTmemCols);
     tmem_relinquish();
   }
-  for (int i = threadIdx.x; i < EPI * 8 * L::kGroupCols; i += blockDim.x) s_stats_all[i] = 0.f;
+  for (int i = threadIdx.x; i < kEpiGroups * 8 * BLOCK_N; i += blockDim.x) s_stats_all[i] = 0.f;
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -236,23 +222,17 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
         }
       };
       if (resident && blockIdx.x < num_tiles) {
-        // the N tile of this CTA never changes (gridDim.x is a multiple of num_n_tiles, or one tile per CTA)
+        // the N tile of this CTA never changes (gridDim.x is a multiple of num_n_tiles, or one tile per CTA); slab order
+        // = consumption order of the halo main loop: (k block, horizontal shift, vertical tap)
         const int n0 = (blockIdx.x % p.num_n_tiles) * BLOCK_N;
         mbar_arrive_expect_tx(bres_bar, static_cast<uint32_t>(num_kblocks) * L::kBBytes);
-        if (halo) {
-          // slab order = consumption order of the halo main loop: (k block, horizontal shift, vertical tap)
-          for (int kb = 0; kb < p.kblocks_per_tap; ++kb)
-            for (int dwi = 0; dwi < 3; ++dwi)
-              for (int dhi = 0; dhi < 3; ++dhi) {
-                Tap tap{};
-                tap.b_off = p.halo_boff[dwi][dhi];
-                load_b(bres_bar, bres_base + static_cast<uint32_t>((kb * 3 + dwi) * 3 + dhi) * L::kBBytes, tap, kb, n0);
-              }
-        } else {
-          for (int t = 0; t < p.num_taps; ++t)
-            for (int kb = 0; kb < p.kblocks_per_tap; ++kb)
-              load_b(bres_bar, bres_base + static_cast<uint32_t>(t * p.kblocks_per_tap + kb) * L::kBBytes, p.taps[t], kb, n0);
-        }
+        for (int kb = 0; kb < p.kblocks_per_tap; ++kb)
+          for (int dwi = 0; dwi < 3; ++dwi)
+            for (int dhi = 0; dhi < 3; ++dhi) {
+              Tap tap{};
+              tap.b_off = p.halo_boff[dwi][dhi];
+              load_b(bres_bar, bres_base + static_cast<uint32_t>((kb * 3 + dwi) * 3 + dhi) * L::kBBytes, tap, kb, n0);
+            }
       }
       int stage = 0;
       uint32_t phase = 0;
@@ -291,7 +271,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
             const uint32_t sa = smem_base + stage * stage_bytes;
             mbar_arrive_expect_tx(full_bar(stage), stage_bytes);
             tma_load_4d(&p.a_map[tap.map], full_bar(stage), sa, kb * kBlockK, w0 + tap.dw, h0 + tap.dh, img0);
-            if (!resident) load_b(full_bar(stage), sa + L::kABytes, tap, kb, n0);
+            load_b(full_bar(stage), sa + L::kABytes, tap, kb, n0);
             if (++stage == nstages) { stage = 0; phase ^= 1; }
           }
         }
@@ -315,7 +295,6 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      int tgrp = 0;   // epilogue group that finishes this tile (CTA-local tile index % EPI)
       if (resident && blockIdx.x < num_tiles) mbar_wait(bres_bar, 0);
       for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
         mbar_wait(tempty_bar(acc), acc_phase ^ 1);
@@ -341,18 +320,17 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
               }
             }
             umma_commit(empty_bar(stage));
-            if (st == nst - 1) umma_commit(tfull_bar(tgrp));
+            if (st == nst - 1) umma_commit(tfull_bar(acc));
             if (++stage == nstages) { stage = 0; phase ^= 1; }
           }
           if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-          if (++tgrp == kTileGroups) tgrp = 0;
           continue;
         }
         for (int kb = 0; kb < num_kblocks; ++kb) {
           mbar_wait(full_bar(stage), phase);
           tc_fence_after();
           const uint32_t sa = smem_base + stage * stage_bytes;
-          const uint32_t sb = resident ? bres_base + static_cast<uint32_t>(kb) * L::kBBytes : sa + L::kABytes;
+          const uint32_t sb = sa + L::kABytes;
 #pragma unroll
           for (int k = 0; k < kBlockK / 16; ++k) {
             const uint64_t da = make_smem_desc_sw128(sa + k * 32, 0, 1024);
@@ -361,30 +339,27 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
             umma_bf16(tmem_d, da, db, idesc, (kb | k) != 0);
           }
           umma_commit(empty_bar(stage));
-          if (kb == num_kblocks - 1) umma_commit(tfull_bar(tgrp));
+          if (kb == num_kblocks - 1) umma_commit(tfull_bar(acc));
           if (++stage == nstages) { stage = 0; phase ^= 1; }
         }
         if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        if (++tgrp == kTileGroups) tgrp = 0;
       }
     }
   } else {
-    // ===================== epilogue (warps 2..: EPI groups of four warps) =====================
-    // Tile group tg finishes the CTA-local tiles t = tg, tg + kTileGroups, ... (accumulator stage t % 2), so that many
-    // tile epilogues overlap each other and the main loop. Each group of four warps has its own staging buffer(s),
-    // statistics scratch, named barrier and TMA store queue; in split-tile mode two groups share a tile group.
+    // ===================== epilogue (warps 2..9: two groups of four warps) =====================
+    // Group grp finishes the CTA-local tiles grp, grp + 2, ... (accumulator stage grp), so the two tile epilogues overlap
+    // each other and the main loop. Each group has its own staging buffer(s), statistics scratch, named barrier and TMA
+    // store queue.
     const int ew = warp - 2;
     const int grp = ew >> 2;
-    const int tg = SPLIT ? (grp >> 1) : grp;
-    constexpr int GW = L::kGroupCols;                 // columns of the tile this group finishes
-    const int col_base = SPLIT ? (grp & 1) * GW : 0;  // first of them
+    const int acc = grp;                  // TMEM accumulator stage of every tile this group finishes
     const int wq = warp & 3;              // TMEM lane quarter this warp may access
     const int r = wq * 32 + lane;         // row of the tile owned by this thread
     const int et = (ew & 3) * 32 + lane;  // 0..127 inside the group
     const bool store_leader = (et == 0);
     const uint32_t bar_id = 1 + grp;
-    float* s_stats = s_stats_all + grp * 8 * GW;               // [warp 0..3][sum | sqsum][GW]
-    float* s_mine = s_stats + (ew & 3) * 2 * GW;               // this warp's private slot: no atomics, fixed order
+    float* s_stats = s_stats_all + grp * 8 * BLOCK_N;          // [warp 0..3][sum | sqsum][BLOCK_N]
+    float* s_mine = s_stats + (ew & 3) * 2 * BLOCK_N;          // this warp's private slot: no atomics, fixed order
     uint8_t* stg_base = smem + L::kOffStaging + grp * NBUF * L::kStagingBytes;
     uint32_t res_phase[2] = {0, 0};
     int buf = 0;
@@ -402,8 +377,8 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
     const bool ep_relu = (OPT & kOptRelu) ? (p.relu != 0) : false;
     constexpr bool BNRED = (OPT & kOptBnRed) != 0;
     static_assert(!BNRED || ((OPT & kOptRes) && !(OPT & (kOptResExtra | kOptRelu | kOptOutBits))), "kOptBnRed rides the residual path");
-    float* my_partial = do_stats ? p.stat_partial + static_cast<size_t>(EPI * blockIdx.x + grp) * 2 * p.n_total : nullptr;
-    constexpr int kChunks = GW / 64;
+    float* my_partial = do_stats ? p.stat_partial + static_cast<size_t>(kEpiGroups * blockIdx.x + grp) * 2 * p.n_total : nullptr;
+    constexpr int kChunks = BLOCK_N / 64;
     // Folded batch norm in the epilogue without statistics -- the fused forward block tail (BN + identity + ReLU + bit
     // mask), its downsample branch (BN only) and every eval-mode convolution (BN [+ identity] [+ ReLU]): scale / shift
     // of the CTA's current N tile live in the group's (otherwise unused) statistics scratch, the affine and the
@@ -411,20 +386,20 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
     // stalls on every FMUL / FADD, ncu: profiles/r2_ncu_fused_tail.txt) and spent ~1 000 instructions per 64-column
     // chunk. launch_conv only selects this instance when scale, shift, ReLU and a plain residual are all present and
     // no statistics are requested.
-    constexpr bool FAST_TAIL = (OPT & kOptAffine) && !(OPT & ~(kOptAffine | kOptRes | kOptRelu)) && EPI == 2;
-    float* s_aff = s_stats;   // [scale GW | shift GW]
+    constexpr bool FAST_TAIL = (OPT & kOptAffine) && !(OPT & ~(kOptAffine | kOptRes | kOptRelu));
+    float* s_aff = s_stats;   // [scale BLOCK_N | shift BLOCK_N]
     int cur_aff_n = -1;
 
     auto flush_stats = [&](int n_tile) {
       named_bar_sync(bar_id, 128);
-      for (int c = et; c < 2 * GW; c += 128) {
-        const int which = c / GW, col = c - which * GW;
-        const int gc = n_tile * BLOCK_N + col_base + col;
+      for (int c = et; c < 2 * BLOCK_N; c += 128) {
+        const int which = c / BLOCK_N, col = c - which * BLOCK_N;
+        const int gc = n_tile * BLOCK_N + col;
         float acc_s = 0.f;
 #pragma unroll
         for (int w = 0; w < 4; ++w) {
-          acc_s += s_stats[w * 2 * GW + c];
-          s_stats[w * 2 * GW + c] = 0.f;
+          acc_s += s_stats[w * 2 * BLOCK_N + c];
+          s_stats[w * 2 * BLOCK_N + c] = 0.f;
         }
         if (gc < p.n_total) my_partial[which * p.n_total + gc] += acc_s;   // only this thread ever touches this word
       }
@@ -442,13 +417,11 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
       tma_load_4d(&p.res_map, res_bar(grp, b), smem_u32(stg_base + b * L::kStagingBytes), n_tile * BLOCK_N + ch * 64,
                   rem & ((1 << p.log2_wo) - 1), rem >> p.log2_wo, img0);
     };
-    const int first_tile = blockIdx.x + tg * gridDim.x;
+    const int first_tile = blockIdx.x + grp * gridDim.x;
     if (has_res && store_leader && first_tile < num_tiles) issue_residual(first_tile, 0, 0);
 
-    int t_local = tg;
     uint32_t full_phase = 0;
-    for (int tile = first_tile; tile < num_tiles; tile += kTileGroups * gridDim.x, t_local += kTileGroups, full_phase ^= 1) {
-      const int acc = t_local & 1;   // TMEM accumulator stage of this tile
+    for (int tile = first_tile; tile < num_tiles; tile += kEpiGroups * gridDim.x, full_phase ^= 1) {
       const int m_tile = tile / p.num_n_tiles;
       const int n_tile = tile - m_tile * p.num_n_tiles;
       const int m0 = m_tile * kBlockM;
@@ -456,23 +429,23 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
       const int rem = m0 & ((1 << p.log2_howo) - 1);
       const int h0 = rem >> p.log2_wo;
       const int w0 = rem & ((1 << p.log2_wo) - 1);
-      const int n0 = n_tile * BLOCK_N + col_base;   // first output channel this group stores
+      const int n0 = n_tile * BLOCK_N;
       if (do_stats && n_tile != cur_n) {
         if (cur_n >= 0) flush_stats(cur_n);
         cur_n = n_tile;
       }
       if (FAST_TAIL && n_tile != cur_aff_n) {
         named_bar_sync(bar_id, 128);   // nobody still reads the previous tile's coefficients
-        for (int c = et; c < GW; c += 128) {
-          const int gc = n_tile * BLOCK_N + col_base + c;
+        for (int c = et; c < BLOCK_N; c += 128) {
+          const int gc = n0 + c;
           s_aff[c] = gc < p.n_total ? __ldg(ep_scale + gc) : 0.f;
-          s_aff[GW + c] = gc < p.n_total ? __ldg(ep_shift + gc) : 0.f;
+          s_aff[BLOCK_N + c] = gc < p.n_total ? __ldg(ep_shift + gc) : 0.f;
         }
         named_bar_sync(bar_id, 128);
         cur_aff_n = n_tile;
       }
 
-      mbar_wait(tfull_bar(tg), full_phase);
+      mbar_wait(tfull_bar(acc), full_phase);
       tc_fence_after();
 
 #pragma unroll 1
@@ -483,7 +456,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
         uint32_t v[2][32];
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
-          const uint32_t taddr = tmem_base + (static_cast<uint32_t>(wq * 32) << 16) + acc * BLOCK_N + col_base + ch * 64 + h * 32;
+          const uint32_t taddr = tmem_base + (static_cast<uint32_t>(wq * 32) << 16) + acc * BLOCK_N + ch * 64 + h * 32;
           tmem_ld_32x32(taddr, v[h]);
         }
         // Residual + statistics: the prefetch below refills the buffer the PREVIOUS chunk was staged in, and the statistics
@@ -499,7 +472,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
             // the residual tile of the next chunk (this buffer's residual is already in flight / landed)
             tma_store_wait_read<0>();
             const bool last_ch = (ch == kChunks - 1);
-            const int ntile = last_ch ? tile + kTileGroups * gridDim.x : tile;
+            const int ntile = last_ch ? tile + kEpiGroups * gridDim.x : tile;
             if (ntile < num_tiles) issue_residual(ntile, last_ch ? 0 : ch + 1, buf ^ 1);
           } else {
             // this buffer was handed to a TMA store two chunks ago (one chunk = one tile ago with a single buffer)
@@ -550,7 +523,7 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
           if constexpr (FAST_TAIL) {
             uint32_t ob = 0;
             const float4* sc4 = reinterpret_cast<const float4*>(s_aff + ch * 64 + h * 32);
-            const float4* sh4 = reinterpret_cast<const float4*>(s_aff + GW + ch * 64 + h * 32);
+            const float4* sh4 = reinterpret_cast<const float4*>(s_aff + BLOCK_N + ch * 64 + h * 32);
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
               const int phys = (h * 4 + q) ^ (r & 7);
@@ -716,8 +689,8 @@ conv_gemm_kernel(const __grid_constant__ ConvGemmParams p) {
           const int c = ch * 64 + lane * 2;
           s_mine[c] += s2.x;
           s_mine[c + 1] += s2.y;
-          s_mine[GW + c] += q2.x;
-          s_mine[GW + c + 1] += q2.y;
+          s_mine[BLOCK_N + c] += q2.x;
+          s_mine[BLOCK_N + c + 1] += q2.y;
         }
         if (NBUF == 2) buf ^= 1;
       }

@@ -355,7 +355,6 @@ ConvLaunch plan_conv_forward(const ConvShape& s, const __nv_bfloat16* x, const _
   p.log2_wo = ilog2(s.Wo());
   p.log2_howo = ilog2(s.Ho() * s.Wo());
   setup_halo(p, s, x, s.Cin, false, l.block_n);
-  l.epi = choose_epilogue_groups(p, l.block_n);
   return l;
 }
 
@@ -435,7 +434,6 @@ std::vector<ConvLaunch> plan_conv_dgrad(const ConvShape& s, const __nv_bfloat16*
     p.log2_wo = ilog2(Wo);
     p.log2_howo = ilog2(Ho * Wo);
     setup_halo(p, s, dy, s.Cout, true, block_n);
-    l.epi = choose_epilogue_groups(p, block_n);
     out.push_back(l);
   }
   return out;
@@ -468,7 +466,6 @@ ConvLaunch plan_dgrad_concat(const ConvShape& s, const __nv_bfloat16* dy, const 
     p.b_map = make_tmap_bf16(bstack, 2, dims, str, box);
   }
   p.k2_blocks = C1 / 64;
-  l.epi = choose_epilogue_groups(p, l.block_n);
   return l;
 }
 
@@ -578,9 +575,9 @@ WgradLaunch plan_gram(const ConvShape& s, const __nv_bfloat16* x, float* g) {
 // ------------------------------------------------------------------------------------------------
 // Final per-launch parameters of one kernel instance: the halo pipeline depth and the weights-resident choice depend
 // on the instance's shared-memory layout and on the grid.
-template <int BN, int BMN, int EPI, int OPT>
+template <int BN, int OPT>
 static ConvGemmParams finish_params(const ConvGemmParams& p) {
-  using L = ConvGemmSmem<BN, EPI, conv_staging_buffers<BN, OPT, EPI>()>;
+  using L = ConvGemmSmem<BN, conv_staging_buffers<BN, OPT>()>;
   const int tiles = p.num_m_tiles * p.num_n_tiles;
   const int grid = std::min(tiles, num_sms());
   // weights-resident mode (see ConvGemmParams::b_resident)
@@ -604,26 +601,21 @@ static ConvGemmParams finish_params(const ConvGemmParams& p) {
   return q;
 }
 
-template <int BN, int BMN, int EPI, int OPT>
+template <int BN, int BMN, int OPT>
 static void launch_conv_t(const ConvGemmParams& q, cudaStream_t stream) {
-  using L = ConvGemmSmem<BN, EPI, conv_staging_buffers<BN, OPT, EPI>()>;
+  using L = ConvGemmSmem<BN, conv_staging_buffers<BN, OPT>()>;
   static bool configured = false;
   if (!configured) {
-    ARGUS_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<BN, BMN, EPI, OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
+    ARGUS_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<BN, BMN, OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
     configured = true;
   }
   const int grid = std::min(q.num_m_tiles * q.num_n_tiles, num_sms());
-  launch_kernel(conv_gemm_kernel<BN, BMN, EPI, OPT>, grid, 64 + 128 * EPI, L::kTotal, stream, q);
+  launch_kernel(conv_gemm_kernel<BN, BMN, OPT>, grid, kNumThreads, L::kTotal, stream, q);
   ARGUS_CUDA(cudaGetLastError());
 }
 
-// Two epilogue groups (one per TMEM accumulator stage) everywhere. Round 1 also built three groups and a split-tile
-// mode with sixteen epilogue warps; neither helped (the wide shallow-K launches sit at the HBM write bandwidth, not at
-// the epilogue's instruction rate; DESIGN.md section 4) and both were removed in round 2.
-int choose_epilogue_groups(const ConvGemmParams&, int) { return 2; }
-
 namespace {
-// Every conv_gemm_kernel instance the library compiles, all with two epilogue groups.
+// Every conv_gemm_kernel instance the library compiles.
 struct ConvInstanceEntry {
   int block_n, b_mn, opt;
   ConvGemmParams (*finish)(const ConvGemmParams&);
@@ -631,7 +623,7 @@ struct ConvInstanceEntry {
 };
 template <int BN, int BMN, int OPT>
 constexpr ConvInstanceEntry conv_entry() {
-  return {BN, BMN, OPT, &finish_params<BN, BMN, 2, OPT>, &launch_conv_t<BN, BMN, 2, OPT>};
+  return {BN, BMN, OPT, &finish_params<BN, OPT>, &launch_conv_t<BN, BMN, OPT>};
 }
 constexpr int kTail = kOptAffine | kOptRes | kOptRelu;   // fused forward block tail: BN + identity + ReLU (+ bits)
 const ConvInstanceEntry kConvInstances[] = {
@@ -702,7 +694,6 @@ ConvGemmParams epilogue_params(const ConvLaunch& l, const Epilogue& e) {
 
 // Specialised epilogues for the option combinations the model launches; anything else runs the generic kernel.
 ConvInstance select_conv_instance(const ConvLaunch& l, const ConvGemmParams& p) {
-  ARGUS_CHECK(l.epi == 2, "two epilogue groups");
   int need = 0;
   if (p.scale || p.shift) need |= kOptAffine;
   if (p.has_res) need |= kOptRes;
@@ -790,7 +781,7 @@ void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream) {
 
 int stat_slots(const ConvLaunch& l) {
   const int tiles = l.p.num_m_tiles * l.p.num_n_tiles;
-  return l.epi * std::min(tiles, num_sms());
+  return kEpiGroups * std::min(tiles, num_sms());
 }
 
 int64_t wgrad_scratch_elems(const WgradLaunch& l) {

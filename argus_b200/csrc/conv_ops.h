@@ -62,7 +62,6 @@ struct ConvLaunch {
   ConvGemmParams p;
   int block_n = 64;
   int b_mn = 0;
-  int epi = 2;        // epilogue groups of the kernel variant (choose_epilogue_groups)
   TmapGeom out_geom;
 };
 
@@ -105,7 +104,7 @@ void stem_dgrad(const __nv_bfloat16* dy, const __nv_bfloat16* w, float* dx, int 
 
 void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream);
 
-// The conv_gemm_kernel<block_n, b_mn, 2, opt> instance a launch runs (opt = kOptAll for the generic kernel).
+// The conv_gemm_kernel<block_n, b_mn, opt> instance a launch runs (opt = kOptAll for the generic kernel).
 struct ConvInstance {
   int block_n = 0, b_mn = 0, opt = 0;
 };
@@ -127,7 +126,6 @@ void conv_instances_record(bool on);
 std::vector<std::array<int, 5>> conv_instances_recorded();
 // (block_n, b_mn, opt) of every kernel instance launch_conv can dispatch to
 std::vector<std::array<int, 3>> conv_instances_all();
-int choose_epilogue_groups(const ConvGemmParams& p, int block_n);
 // number of statistic slots launch_conv writes for this launch (one per epilogue group per CTA)
 int stat_slots(const ConvLaunch& l);
 // elements of split-K scratch this launch needs (0 when it does not split)

@@ -77,7 +77,7 @@ Model::~Model() {
   cudaFree(bn_scratch_);
   cudaFree(bn_stats_);
   cudaFree(bn_bwd_scratch_);
-  cudaFree(alg_h_); cudaFree(alg_s_); cudaFree(alg_k1k0_); cudaFree(alg_bias_); cudaFree(alg_gstats_);
+  cudaFree(alg_h_); cudaFree(alg_k1k0_); cudaFree(alg_bias_); cudaFree(alg_gstats_);
   cudaFree(alg_bstack_);
   cudaFree(alg_mpartial_);
   cudaFree(bnred_stats_);
@@ -208,21 +208,12 @@ void Model::bind(float* params, float* grads, float* buffers) {
     ARGUS_CUDA(cudaMalloc(&packed_, n_packed_ * sizeof(bf16)));
     ARGUS_CUDA(cudaMalloc(&gpacked_, std::max<int64_t>(n_gpacked_, 1) * sizeof(float)));
     ARGUS_CUDA(cudaMalloc(&bn_scratch_, n_bn_scratch_ * sizeof(float)));
-    max_stat_slots_ = 4 * num_sms();   // up to four epilogue groups per CTA
+    max_stat_slots_ = kEpiGroups * num_sms();   // one slot per epilogue group per CTA (stat_slots)
     ARGUS_CUDA(cudaMalloc(&bn_stats_, n_bn_stats_ * 2 * max_stat_slots_ * sizeof(float)));
     ARGUS_CUDA(cudaMalloc(&bn_bwd_scratch_, bn_bwd_scratch_elems() * sizeof(float)));
     {
       const char* e = getenv("ARGUS_BN_ALGEBRA");
       bn_algebra_ = !(e && e[0] == '0');
-      // Fused block tail in the training forward (default; ARGUS_FUSED_TAIL=0 selects the separate passes): bn3's batch
-      // statistics come from the Gram matrix of act2 (kept for the algebraic backward, which then only needs H = g^T act2),
-      // conv3 applies BN + identity + ReLU + the bit mask in its epilogue and raw3 is never written: 10 instead of 17
-      // narrow-tensor passes per block tail. Round 1 measured it SLOWER (45.2 vs 44.1 ms: 8 epilogue warps, ~1 000
-      // instructions per 64-column chunk, coefficient loads stalling every FMUL / FADD); with the packed-fp32 epilogue, the
-      // coefficients in shared memory and the group barrier removed from the residual path it is 1.0-1.2 ms per step
-      // FASTER (profiles/r2_fused_tail_ab.txt).
-      const char* ft = getenv("ARGUS_FUSED_TAIL");
-      fused_tail_ = !(ft && ft[0] == '0');
       // eligible: bottlenecks whose mid width is <= 256 (layers 1-3); layer4's small matrices would cost more than the
       // two passes over its (small) activations
       for (const auto& b : blocks_)
@@ -232,8 +223,7 @@ void Model::bind(float* params, float* grads, float* buffers) {
           if (b.has_ds && b.ds.shape.Cin <= 256) alg_max_c_ = std::max(alg_max_c_, b.ds.shape.Cin);
         }
       const size_t O = alg_max_o_, C = alg_max_c_;
-      ARGUS_CUDA(cudaMalloc(&alg_h_, (O + C) * C * sizeof(float)));   // H [O][C] followed by the Gram matrix [C][C]
-      ARGUS_CUDA(cudaMalloc(&alg_s_, C * sizeof(float)));
+      ARGUS_CUDA(cudaMalloc(&alg_h_, O * C * sizeof(float)));   // H [O][C]
       ARGUS_CUDA(cudaMalloc(&alg_k1k0_, 2 * O * sizeof(float)));
       ARGUS_CUDA(cudaMalloc(&alg_bias_, C * sizeof(float)));
       ARGUS_CUDA(cudaMalloc(&alg_gstats_, static_cast<size_t>(max_stat_slots_) * 2 * O * sizeof(float)));
@@ -242,9 +232,10 @@ void Model::bind(float* params, float* grads, float* buffers) {
     }
     {
       // BN-backward reduction in the epilogue of the dgrad that produces the gradient: OPT-IN (ARGUS_BN_REDUCE_FUSED=1
-      // fuses layers 1-2, =2 every eligible layer). It saves 0.3 ms per step, but with it and the separate block tail the
-      // bench trajectory stopped reproducing from run to run once the look-ahead staging started (0 of 7 runs; 9 of 9
-      // with the fused tail; every other mode 100 % -- profiles/r2_determinism.md), and the cause was not found.
+      // fuses layers 1-2, =2 every eligible layer). It saves 0.3 ms per step. The only configuration in which its bench
+      // trajectory did not reproduce from run to run, the separate-pass block tail of layers 1-3 (0 of 7 runs against
+      // 13 of 13 with the fused tail; profiles/r2_determinism.md), no longer exists; making it the default is left to its
+      // own measurement.
       const char* e = getenv("ARGUS_BN_REDUCE_FUSED");
       bn_reduce_fused_ = e ? atoi(e) : 0;
       ARGUS_CUDA(cudaMalloc(&bnred_stats_, static_cast<size_t>(max_stat_slots_) * 2 * 512 * sizeof(float)));
@@ -400,7 +391,7 @@ void Model::build_plan(Plan& p) {
     bp.act1 = arena_alloc<bf16>(e_in * wd);
     if (tr) bp.raw2 = arena_alloc<bf16>(e_out * wd);
     bp.act2 = arena_alloc<bf16>(e_out * wd);
-    bp.fused_tail = tr && bn_algebra_ && fused_tail_ && wd <= 256;
+    bp.fused_tail = tr && bn_algebra_ && wd <= 256;
     if (tr && !bp.fused_tail) bp.raw3 = arena_alloc<bf16>(e_out * oc);
     if (br.has_ds) bp.rawd = arena_alloc<bf16>(e_out * oc);  // eval / fused tail: holds the folded-BN identity branch
     bp.out = arena_alloc<bf16>(e_out * oc);
@@ -409,9 +400,8 @@ void Model::build_plan(Plan& p) {
       bp.act1_bits = arena_alloc<uint8_t>(e_in * wd / 8);
       bp.act2_bits = arena_alloc<uint8_t>(e_out * wd / 8);
     }
-    if (tr && bn_algebra_ && wd <= 256)
-      bp.act2_colsum = arena_alloc<float>(static_cast<size_t>(bn_apply_grid(static_cast<int64_t>(e_out), wd)) * wd);
     if (bp.fused_tail) {
+      bp.act2_colsum = arena_alloc<float>(static_cast<size_t>(bn_apply_grid(static_cast<int64_t>(e_out), wd)) * wd);
       // (C x C Gram matrix followed by the C column sums of the same activation)
       bp.gram_saved = arena_alloc<float>(static_cast<size_t>(wd) * wd + wd);
       if (br.has_ds && br.ds.shape.Cin <= 256)
@@ -511,20 +501,16 @@ void Model::build_plan(Plan& p) {
       // conv3: dy = Q (dRaw3), input act2, dx -> R
       bp.c3.wgrad = plan_conv_wgrad(br.c3.shape, Q, bp.act2, wg_dst(br.c3));
       bp.c3.dgrad = plan_conv_dgrad(br.c3.shape, Q, packed_ + br.c3.packed_off, R);
-      bp.algebraic = bn_algebra_ && br.c1.shape.Cout <= 256;
-      if (bp.algebraic) {
+      if (bp.fused_tail) {
         // algebraic bn3 backward: GEMMs on the masked gradient P itself (never on dRaw3)
         const int C = br.c3.shape.Cin;
-        bp.hg_wgrad = bp.gram_saved ? plan_conv_wgrad(br.c3.shape, P, bp.act2, alg_h_)
-                                    : plan_conv_wgrad_gram(br.c3.shape, P, bp.act2, alg_h_);
+        bp.hg_wgrad = plan_conv_wgrad(br.c3.shape, P, bp.act2, alg_h_);
         bp.c3_concat = plan_dgrad_concat(br.c3.shape, P, bp.act2, C, alg_bstack_, R);
         ensure_wgrad_scratch(bp.hg_wgrad);
       }
-      bp.ds_algebraic = bp.algebraic && br.has_ds && br.ds.shape.Cin <= 256;   // layer1.0, layer2.0
-      if (bp.ds_algebraic) {
+      if (bp.ds_gram_saved != nullptr) {   // layer1.0, layer2.0: the downsample branch the same way
         const int C = br.ds.shape.Cin;
-        bp.ds_hg_wgrad = bp.ds_gram_saved ? plan_conv_wgrad(br.ds.shape, P, bp.x, alg_h_)
-                                          : plan_conv_wgrad_gram(br.ds.shape, P, bp.x, alg_h_);
+        bp.ds_hg_wgrad = plan_conv_wgrad(br.ds.shape, P, bp.x, alg_h_);
         bp.ds_concat = plan_dgrad_concat(br.ds.shape, P, bp.x, C, alg_bstack_, Tb);
         ensure_wgrad_scratch(bp.ds_hg_wgrad);
       }
@@ -895,34 +881,27 @@ void Model::conv_backward(const ConvPlan& cp, const bf16* residual, const uint8_
 
 // Expanding 1x1 convolution + batch norm backward without touching the BN input or its gradient (see bn_algebra.cu
 // for the derivation): upstream masked gradient g and the saved conv input `act` go through three GEMMs.
-void Model::conv_bn_backward_algebraic(const ConvRef& c, const WgradLaunch& hg, const ConvLaunch& concat, const bf16* act,
-                                       const float* colsum_partial, int64_t rows, int N, cudaStream_t s,
-                                       const BnRed* red, const float* saved_gram) {
+void Model::conv_bn_backward_algebraic(const ConvRef& c, const WgradLaunch& hg, const ConvLaunch& concat,
+                                       const float* saved_gram, int64_t rows, cudaStream_t s, const BnRed* red) {
   const int O = c.shape.Cout, C = c.shape.Cin;
-  // fused tail: G is the matrix the forward statistics came from (kept per block) and hg computes H only; otherwise hg
-  // is the stacked launch that appends G below H
-  const float* alg_g = saved_gram != nullptr ? saved_gram : alg_h_ + static_cast<size_t>(O) * C;
+  // G and the column sums of `act` stored after it: what the fused block tail derived the forward statistics from
+  const float* colsum = saved_gram + static_cast<size_t>(C) * C;
   join_wgrad(s);   // one split-K scratch buffer: no weight-gradient GEMM may be in flight on the side stream
-  ARGUS_CUDA(cudaMemsetAsync(alg_h_, 0, static_cast<size_t>(saved_gram != nullptr ? O : O + C) * C * sizeof(float), s)); pdl_break(s, kPdlAfterMemop);
-  launch_wgrad(hg, wgrad_scratch_, s);     // H = g^T act (rows < O) [and G = act^T act (rows O..O+C), act tiles loaded once]
-  // column sums of `act`: the forward kept them next to its Gram matrix (fused tail); otherwise they are rebuilt here
-  const float* colsum = alg_s_;
-  if (saved_gram != nullptr) colsum = saved_gram + static_cast<size_t>(C) * C;
-  else if (colsum_partial != nullptr) colsum_finalize(colsum_partial, bn_apply_grid(rows, C), alg_s_, C, s);
-  else colsum_pixels_bf16(act, N, c.shape.H, c.shape.W, C, c.shape.stride, bn_bwd_scratch_, alg_s_, s);
+  ARGUS_CUDA(cudaMemsetAsync(alg_h_, 0, static_cast<size_t>(O) * C * sizeof(float), s)); pdl_break(s, kPdlAfterMemop);
+  launch_wgrad(hg, wgrad_scratch_, s);     // H = g^T act
   const float* sc = bn_scratch_ + c.bn.scratch_off;
   // the coefficient / B-stack kernels feed the dgrad below; the weight-gradient kernel feeds nothing in this chain and
   // runs on the weight-gradient side stream (joined before H, G, s or k1k0 are overwritten: every algebraic call and
   // every bn_backward joins first)
   const bool dw_aside = overlap_wgrad_;
-  bn_alg_backward_small(packed_ + c.packed_off, alg_h_, alg_g, colsum, alg_gstats_, alg_gstats_slots_, 2 * O, sc,
+  bn_alg_backward_small(packed_ + c.packed_off, alg_h_, saved_gram, colsum, alg_gstats_, alg_gstats_slots_, 2 * O, sc,
                         sc + 2 * O, sc + 3 * O, static_cast<double>(rows), grads_dev_ + c.bn.gamma_off,
                         grads_dev_ + c.bn.beta_off, dw_aside ? nullptr : grads_dev_ + c.w_off, alg_k1k0_, alg_bstack_, alg_bias_,
                         alg_mpartial_, O, C, s);
   if (dw_aside) {
     const bf16* Wp = packed_ + c.packed_off;
     float* dW = grads_dev_ + c.w_off;
-    run_on_side(s, [=](cudaStream_t ss) { bn_alg_backward_dw(Wp, alg_h_, alg_g, colsum, sc, alg_k1k0_, dW, O, C, ss); });
+    run_on_side(s, [=](cudaStream_t ss) { bn_alg_backward_dw(Wp, alg_h_, saved_gram, colsum, sc, alg_k1k0_, dW, O, C, ss); });
   }
   Epilogue e;
   e.shift = alg_bias_;
@@ -971,13 +950,12 @@ void Model::backward(const float* d_out, int stage_begin, int stage_end, cudaStr
       // avgpool_bwd that produced it applied the bit mask), so it is the BN3 / downsample-BN upstream gradient and the
       // identity-branch gradient at once.
       const uint8_t* prev_bits = (i > 0) ? p.blocks[i - 1].out_bits : nullptr;
-      float* prev_stats = (i > 0 && p.blocks[i - 1].algebraic) ? alg_gstats_ : nullptr;
+      float* prev_stats = (i > 0 && p.blocks[i - 1].fused_tail) ? alg_gstats_ : nullptr;
       const bf16* residual = P;
       if (br.has_ds) {
-        if (bp.ds_algebraic) {
+        if (bp.ds_gram_saved != nullptr) {
           zero_ds_gradient_once(bp, br, T, s);
-          conv_bn_backward_algebraic(br.ds, bp.ds_hg_wgrad, bp.ds_concat, bp.x, nullptr, bp.rows_out, N, s, nullptr,
-                                     bp.ds_gram_saved);
+          conv_bn_backward_algebraic(br.ds, bp.ds_hg_wgrad, bp.ds_concat, bp.ds_gram_saved, bp.rows_out, s);
         } else {
           bn_backward(br.ds, P, bp.rawd, nullptr, R, bp.rows_out, 0, s);
           zero_ds_gradient_once(bp, br, T, s);
@@ -994,10 +972,10 @@ void Model::backward(const float* d_out, int stage_begin, int stage_end, cudaStr
       const int cmax = bn_reduce_fused_ == 2 ? 512 : 128;
       const bool fuse2 = bn_reduce_fused_ && br.c2.bn.C <= cmax;
       const bool fuse1 = bn_reduce_fused_ && br.c1.bn.C <= cmax && br.c2.shape.stride == 1;
-      if (bp.algebraic) {
+      if (bp.fused_tail) {
         // P, act2 -> R (dAct2), dW3, dgamma3, dbeta3
-        conv_bn_backward_algebraic(br.c3, bp.hg_wgrad, bp.c3_concat, bp.act2, bp.act2_colsum, bp.rows_out, N, s,
-                                   fuse2 ? &red2 : nullptr, bp.gram_saved);
+        conv_bn_backward_algebraic(br.c3, bp.hg_wgrad, bp.c3_concat, bp.gram_saved, bp.rows_out, s,
+                                   fuse2 ? &red2 : nullptr);
       } else {
         bn_backward(br.c3, P, bp.raw3, nullptr, Q, bp.rows_out, 0, s);      // Q = dRaw3
         conv_backward(bp.c3, nullptr, nullptr, nullptr, s, fuse2 ? &red2 : nullptr);   // Q -> R (dAct2)

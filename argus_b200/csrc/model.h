@@ -63,19 +63,19 @@ struct BlockPlan {
   int64_t rows_in = 0, rows_mid = 0, rows_out = 0;
   // gradient scratch roles for this block
   bf16 *g_out = nullptr, *g_q = nullptr, *g_r = nullptr, *g_t = nullptr, *g_x = nullptr;
-  // algebraic bn3 backward (bn_algebra.cu): H = g^T act2, G = act2^T act2, concatenated-K dgrad of conv3
-  // Fused block tail in the training forward (same eligibility as `algebraic`): bn3's batch statistics come from the
-  // Gram matrix of act2, so conv3 applies BN + identity + ReLU (+ bit mask) in its epilogue: raw3 is never written
+  // Fused block tail (training plans, mid width <= 256, unless ARGUS_BN_ALGEBRA=0): bn3's batch statistics come from the
+  // Gram matrix of act2, so conv3 applies BN + identity + ReLU (+ bit mask) in its epilogue and raw3 is never written.
+  // The backward is then algebraic (bn_algebra.cu): H = g^T act2 with the saved G = act2^T act2, concatenated-K dgrad of
+  // conv3.
   bool fused_tail = false;
   WgradLaunch fwd_gram, ds_fwd_gram;
-  // fused tail: the Gram matrices of act2 / x the forward statistics were derived from, kept for the algebraic backward
-  // (which then only needs H = g^T act: the stacked [g | act]^T act launch loses a fifth of its rows)
+  // the Gram matrices of act2 / x the forward statistics were derived from, each followed by the column sums of the same
+  // activation; ds_gram_saved is set when the downsample branch (Cin <= 256) takes the same path, with act = the block
+  // input (its even pixels at stride 2)
   float *gram_saved = nullptr, *ds_gram_saved = nullptr;
-  bool algebraic = false;
   float* act2_colsum = nullptr;   // [bn_apply_grid][C] per-block column sums of act2, written by the forward bn_apply
-  WgradLaunch hg_wgrad;           // one launch: H (rows < O) and the Gram matrix (rows O..O+C) into alg_h_
+  WgradLaunch hg_wgrad;           // H = g^T act2 into alg_h_
   ConvLaunch c3_concat;
-  bool ds_algebraic = false;      // same for the downsample branch, with act = the block input (its even pixels at stride 2)
   WgradLaunch ds_hg_wgrad;
   ConvLaunch ds_concat;
   size_t x_bytes = 0;
@@ -196,11 +196,10 @@ class Model {
   void attach_bn_reduction(Epilogue& e, const ConvLaunch& l, const BnRed& red, cudaStream_t s);
   // BN backward of a layer whose gradient arrived masked and already reduced (bnred_stats_): finalize + apply
   void bn_backward_reduced(const ConvRef& c, bf16* dy, const bf16* raw, bf16* dx, int64_t rows, cudaStream_t s);
-  // conv (expanding 1x1) + BN backward on the masked upstream gradient (bn_algebra.cu); colsum_partial == nullptr:
-  // the column sums of `act` are computed here
-  void conv_bn_backward_algebraic(const ConvRef& c, const WgradLaunch& hg, const ConvLaunch& concat, const bf16* act,
-                                  const float* colsum_partial, int64_t rows, int N, cudaStream_t s,
-                                  const BnRed* red = nullptr, const float* saved_gram = nullptr);
+  // conv (expanding 1x1) + BN backward on the masked upstream gradient (bn_algebra.cu); saved_gram: the Gram matrix of
+  // the convolution input the forward kept, followed by its column sums
+  void conv_bn_backward_algebraic(const ConvRef& c, const WgradLaunch& hg, const ConvLaunch& concat,
+                                  const float* saved_gram, int64_t rows, cudaStream_t s, const BnRed* red = nullptr);
 
   template <typename T>
   T* arena_alloc(size_t count);
@@ -234,9 +233,8 @@ class Model {
   float* bn_bwd_scratch_ = nullptr;   // per-block partial sums of the BN-backward reductions
   // algebraic bn3 backward scratch (sized for the widest eligible block)
   bool bn_algebra_ = true;
-  bool fused_tail_ = true;
   int alg_max_o_ = 0, alg_max_c_ = 0;
-  float *alg_h_ = nullptr, *alg_s_ = nullptr, *alg_k1k0_ = nullptr, *alg_bias_ = nullptr;
+  float *alg_h_ = nullptr, *alg_k1k0_ = nullptr, *alg_bias_ = nullptr;
   float* alg_mpartial_ = nullptr;
   float* alg_gstats_ = nullptr;       // [max_stat_slots_][2][alg_max_o_] sums of the masked gradient, per dgrad CTA slot
   bf16* alg_bstack_ = nullptr;

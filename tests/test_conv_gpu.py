@@ -44,9 +44,9 @@ CASES = [
     (20, 32, 32, 128, 128, 3, 1),   # halo mode with BLOCK_N = 128 and two channel blocks (layer2 shape)
     (3, 16, 16, 64, 128, 3, 1),     # halo mode, eight image rows per tile
     (2, 8, 16, 128, 64, 3, 1),      # halo mode, tile = one whole (8 x 16) image
-    (8, 64, 64, 64, 256, 1, 1),     # >= 148 tiles of 256 columns: split-tile mode (four epilogue groups) in the forward
+    (8, 64, 64, 64, 256, 1, 1),     # >= 148 tiles of 256 columns in the forward
     (8, 64, 64, 256, 64, 1, 1),     # ... and in the dgrad (output = the 256 input channels)
-    (16, 32, 32, 128, 512, 1, 1),   # split-tile mode with two N tiles
+    (16, 32, 32, 128, 512, 1, 1),   # 256-column tiles, two N tiles
 ]
 
 

@@ -27,9 +27,7 @@ def test_without_programmatic_dependent_launch(cuda_device):
 
 
 def test_fused_bn_reduction_modes(cuda_device):
-    """ARGUS_BN_REDUCE_FUSED=2 (BN-backward sums in the dgrad epilogues, every eligible layer) and ARGUS_FUSED_TAIL=0
-    (separate bn_apply block tail): the gradient and reproducibility tests must hold in both."""
+    """ARGUS_BN_REDUCE_FUSED=2 (BN-backward sums in the dgrad epilogues, every eligible layer): the gradient and
+    reproducibility tests must hold."""
     _rerun({"ARGUS_BN_REDUCE_FUSED": "2"}, ["tests/test_model_gpu.py", "tests/test_train_gpu.py", "-k",
                                             "train_forward_backward or reproducible or prefetch"])
-    _rerun({"ARGUS_FUSED_TAIL": "0"}, ["tests/test_model_gpu.py", "tests/test_train_gpu.py", "-k",
-                                       "train_forward_backward or reproducible or prefetch"])
