@@ -741,6 +741,15 @@ int argus_model_stage_input_u8(argus_model* m, const void* images, const float* 
                          static_cast<cudaStream_t>(stream));
   ARGUS_API_END
 }
+int argus_model_stage_input_frozen_u8(argus_model* m, const void* images, const float* aug_params, const void* arc_mask,
+                                      void* plasma_ws, int B, int H, int W, int apply, void* stream) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(m != nullptr, "null model");
+  m->impl.stage_input_u8(static_cast<const uint8_t*>(images), aug_params, static_cast<const uint32_t*>(arc_mask),
+                         static_cast<uint32_t*>(plasma_ws), B, H, W, false, apply != 0,
+                         static_cast<cudaStream_t>(stream), true);
+  ARGUS_API_END
+}
 int argus_model_set_precision(argus_model* m, int mode) {
   ARGUS_API_BEGIN
   ARGUS_CHECK(m != nullptr, "null model");

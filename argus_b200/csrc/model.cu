@@ -293,7 +293,8 @@ void Model::reserve(int max_batch, int H, int W, bool training, bool frozen) {
   build_plan(tmp);
   const size_t need = arena_used_;
   arena_ = saved;
-  const size_t stem_need = training ? static_cast<size_t>(max_batch) * n_cams_ * (H / 2) * (W / 2 + 4) * 16 : 0;
+  const size_t stem_need =
+      (training || frozen) ? static_cast<size_t>(max_batch) * n_cams_ * (H / 2) * (W / 2 + 4) * 16 : 0;
   if (stem_need > stem_in_elems_) {
     // (plan-build time only) every stream of this model must be idle before the staging buffers move
     ARGUS_CUDA(cudaDeviceSynchronize());
@@ -355,19 +356,21 @@ void Model::build_plan(Plan& p) {
     cp.fwd = plan_conv_forward(c.shape, in, packed_ + c.packed_off, out_raw);
     cp.has_dgrad = want_dgrad;
   };
-  // ---- stem (training plans read the model-level double buffer; an eval plan owns a private input in the arena)
-  if (!tr) p.x_in = arena_alloc<bf16>(static_cast<size_t>(N) * (H / 2) * (W / 2 + 4) * 16);
+  // ---- stem (training and frozen plans read the model-level double buffer; an eval plan owns a private input in the
+  // arena)
+  const bool db = tr || fz;
+  if (!db) p.x_in = arena_alloc<bf16>(static_cast<size_t>(N) * (H / 2) * (W / 2 + 4) * 16);
   const int H1 = H / 2, W1 = W / 2;  // stem output
   const int H2 = H1 / 2, W2 = W1 / 2;  // after max pooling
   const size_t stem_elems = static_cast<size_t>(N) * H1 * W1 * 64;
   if (tr) p.raw0 = arena_alloc<bf16>(stem_elems); else p.act0 = arena_alloc<bf16>(stem_elems);
   p.pooled0 = arena_alloc<bf16>(stem_elems / 4);
   if (tr || fz) p.idx0 = arena_alloc<uint8_t>(stem_elems / 4);
-  plan_conv(p.stem, stem_, N, H, W, tr ? stem_in_[0] : p.x_in, tr ? p.raw0 : p.act0, false);
+  plan_conv(p.stem, stem_, N, H, W, db ? stem_in_[0] : p.x_in, tr ? p.raw0 : p.act0, false);
   if (real) {
-    ARGUS_CHECK(!tr || static_cast<size_t>(N) * (H / 2) * (W / 2 + 4) * 16 <= stem_in_elems_, "stem input buffers too small");
+    ARGUS_CHECK(!db || static_cast<size_t>(N) * (H / 2) * (W / 2 + 4) * 16 <= stem_in_elems_, "stem input buffers too small");
     for (int b = 0; b < 2; ++b)
-      p.stem_fwd_buf[b] = plan_conv_forward(stem_.shape, tr ? stem_in_[b] : p.x_in, packed_ + stem_.packed_off,
+      p.stem_fwd_buf[b] = plan_conv_forward(stem_.shape, db ? stem_in_[b] : p.x_in, packed_ + stem_.packed_off,
                                             tr ? p.raw0 : p.act0);
   }
 
@@ -483,7 +486,9 @@ void Model::build_plan(Plan& p) {
     p.g_stem_in = P;
     p.g_raw0 = Q;   // g0
     if (real) {
-      p.stem.wgrad = plan_conv_wgrad(stem_.shape, Q, p.x_in, gpacked_ + stem_.gpacked_off);
+      for (int b = 0; b < 2; ++b)
+        p.stem_wgrad_buf[b] = plan_conv_wgrad(stem_.shape, Q, stem_in_[b], gpacked_ + stem_.gpacked_off);
+      p.stem.wgrad = p.stem_wgrad_buf[0];
       ensure_wgrad_scratch(p.stem.wgrad);
     }
     return;
@@ -697,7 +702,6 @@ void Model::forward(const void* x, bool is_u8, int B, int H, int W, bool trainin
   ARGUS_CHECK(!training || B * n_cams_ * (H / 32) * (W / 32) > 1,
               "train-mode batch norm needs more than one value per channel");
   ARGUS_CHECK(!(training && frozen), "a frozen-statistics forward is an eval-mode forward");
-  ARGUS_CHECK(!frozen || x != nullptr, "the frozen-statistics forward needs the image tensor (no staged input)");
   stem_grad_ready_ = false;
   if (training || frozen) train_input_f32_ = (x != nullptr && !is_u8);
   // which forward backward() differentiates (set after get_plan(), whose arena growth forgets the previous plans)
@@ -713,16 +717,17 @@ void Model::forward(const void* x, bool is_u8, int B, int H, int W, bool trainin
   }
   Plan& p = get_plan(B, H, W, training, frozen);
   note_kind();
-  // every input is written to the alternate stem buffer, which then becomes the current one: a batch staged ahead of
-  // time (stage_input_u8 on another stream) never touches the buffer the in-flight pass still reads
+  // every training or frozen input is written to the alternate stem buffer, which then becomes the current one: a batch
+  // staged ahead of time (stage_input_u8 on another stream) never touches the buffer the in-flight pass still reads
+  const bool db = training || frozen;
   if (x == nullptr) {
     ARGUS_CHECK(staged_plan_ == &p, "forward(x = NULL) needs a preceding stage_input_u8() for the same batch shape");
   } else if (is_u8) {
-    pack_input_u8(static_cast<const uint8_t*>(x), training ? stem_in_[cur_in_ ^ 1] : p.x_in, p.N, H, W, s);
+    pack_input_u8(static_cast<const uint8_t*>(x), db ? stem_in_[cur_in_ ^ 1] : p.x_in, p.N, H, W, s);
   } else {
-    pack_input_f32(static_cast<const float*>(x), training ? stem_in_[cur_in_ ^ 1] : p.x_in, p.N, H, W, s);
+    pack_input_f32(static_cast<const float*>(x), db ? stem_in_[cur_in_ ^ 1] : p.x_in, p.N, H, W, s);
   }
-  if (training) {
+  if (db) {
     cur_in_ ^= 1;
     p.stem.fwd = p.stem_fwd_buf[cur_in_];
     p.stem.wgrad = p.stem_wgrad_buf[cur_in_];
@@ -741,14 +746,15 @@ void Model::forward(const void* x, bool is_u8, int B, int H, int W, bool trainin
 }
 
 void Model::stage_input_u8(const uint8_t* images, const float* aug_params, const uint32_t* arc_mask, uint32_t* plasma_ws,
-                           int B, int H, int W, bool training, bool apply, cudaStream_t s) {
+                           int B, int H, int W, bool training, bool apply, cudaStream_t s, bool frozen) {
   ARGUS_CHECK(B > 0, "empty batch");
   ARGUS_CHECK(!apply || aug_params != nullptr, "augmentation needs a parameter table");
   ARGUS_CHECK(precision_ == 0, "the fused augmentation + staging path exists in bf16 mode only");
-  Plan& p = get_plan(B, H, W, training);
+  ARGUS_CHECK(!(training && frozen), "a frozen-statistics forward is an eval-mode forward");
+  Plan& p = get_plan(B, H, W, training, frozen);
   fuzz_delay(2, s);
-  augment_images(images, true, training ? stem_in_[cur_in_ ^ 1] : p.x_in, true, aug_params, arc_mask, plasma_ws, p.N, H, W,
-                 apply, s);
+  augment_images(images, true, (training || frozen) ? stem_in_[cur_in_ ^ 1] : p.x_in, true, aug_params, arc_mask,
+                 plasma_ws, p.N, H, W, apply, s);
   staged_plan_ = &p;
 }
 

@@ -93,11 +93,12 @@ struct Plan {
   bool frozen = false;
   ConvPlan stem;
   bf16 *raw0 = nullptr, *act0 = nullptr, *pooled0 = nullptr;
-  // The stem input is double buffered so that the NEXT batch can be augmented / staged (on another stream) while the
-  // current one trains. The two buffers belong to the MODEL (Model::stem_in_, sized for the largest reserved batch,
-  // outside the per-plan arena layout), so that staging a batch of a different size -- the short last batch of an epoch --
-  // can never alias the buffer the in-flight step still reads. stem_fwd_buf / stem_wgrad_buf are the launches reading
-  // buffer 0 / 1; forward() copies the pair of the buffer it consumes into stem.fwd / stem.wgrad.
+  // The stem input of training and frozen plans is double buffered so that the NEXT batch can be augmented / staged (on
+  // another stream) while the current one trains. The two buffers belong to the MODEL (Model::stem_in_, sized for the
+  // largest reserved batch, outside the per-plan arena layout), so that staging a batch of a different size -- the short
+  // last batch of an epoch -- can never alias the buffer the in-flight step still reads. Training and frozen forwards
+  // alternate through the same pair. stem_fwd_buf / stem_wgrad_buf are the launches reading buffer 0 / 1; forward()
+  // copies the pair of the buffer it consumes into stem.fwd / stem.wgrad.
   bf16* x_in = nullptr;   // eval plans: private stem input inside the arena (staging + forward run on one stream)
   ConvLaunch stem_fwd_buf[2];
   WgradLaunch stem_wgrad_buf[2];
@@ -139,10 +140,10 @@ class Model {
   void forward(const void* x, bool is_u8, int B, int H, int W, bool training, float* out, cudaStream_t s,
                bool frozen = false);
   // Augmentation fused with input staging: uint8 (B*n_cams, H, W, 3) images -> augmented bf16 stem input of the plan
-  // for (B, H, W, training). A following forward() with x == nullptr consumes it.
+  // for (B, H, W, training, frozen). A following forward() of the same kind with x == nullptr consumes it.
   // arc_mask (nullable): spaghetti arcs as 1 bit per pixel; plasma_ws: workspace of B * n_cams * H * W / 8 bytes
   void stage_input_u8(const uint8_t* images, const float* aug_params, const uint32_t* arc_mask, uint32_t* plasma_ws, int B,
-                      int H, int W, bool training, bool apply, cudaStream_t s);
+                      int H, int W, bool training, bool apply, cudaStream_t s, bool frozen = false);
   // d_out: (B, 6) gradient of the loss wrt forward()'s output. Accumulates parameter gradients (+=) into the bound
   // gradient arena for stages [stage_begin, stage_end); stages must be run in increasing order 0..3. Differentiates the
   // last training or frozen forward, whichever ran last; a frozen one must still be the last forward of all.

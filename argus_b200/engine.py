@@ -92,6 +92,10 @@ class TrainEngine:
         process_group: torch.distributed group for data parallelism (None = single process).
         augmentation: optional argus_b200.data.Augmentation applied on device to uint8 image batches.
         scaler: optional GradScaler (the reference's amp mode, train.py:234,298-300,316-320).
+        frozen_bn: not in the reference -- fine-tuning with frozen batch norm. Every forward is the frozen-statistics
+            forward (argus_model_forward_frozen): batch norm uses the running statistics as constants, and neither the
+            running statistics nor num_batches_tracked change. `model.training` is left as it is. Loss, backward,
+            all-reduce buckets and the optimizer are those of a training step.
 
     It also stands in the reference's `optimizer` slot of `initialize_training` (train.py:245-255): `param_groups`,
     `zero_grad()`, `state_dict()` / `load_state_dict()` follow torch.optim.Adam's surface.
@@ -100,7 +104,7 @@ class TrainEngine:
     def __init__(self, model: NCameraCNN, lr: float = 1e-4, max_grad_norm: float = 1.0,
                  betas: tuple[float, float] = (0.9, 0.999), eps: float = 1e-8,
                  process_group: Optional["dist.ProcessGroup"] = None, distributed: Optional[bool] = None,
-                 augmentation=None, scaler: Optional[GradScaler] = None) -> None:
+                 augmentation=None, scaler: Optional[GradScaler] = None, frozen_bn: bool = False) -> None:
         if not model.flat_params.is_cuda:
             raise _lib.ArgusError("TrainEngine needs the model on a CUDA device (no CPU fallback)")
         self.model = model
@@ -110,6 +114,7 @@ class TrainEngine:
         self.eps = float(eps)
         self.augmentation = augmentation
         self.scaler = scaler
+        self.frozen_bn = bool(frozen_bn)
         self.step_count = 0
         self.device = model.flat_params.device
         if distributed is None:
@@ -128,13 +133,13 @@ class TrainEngine:
         self._loss_mean = torch.zeros(1, dtype=torch.float32, device=self.device)
         self._stage_ranges = model.stage_ranges()
         self.last_grad_norm = self._grad_norm
-        # look-ahead staging (prefetch): side stream + events, see prefetch()
+        # look-ahead staging (prefetch): side stream + event, see prefetch()
         self._side = torch.cuda.Stream(device=self.device)
-        self._prev_done = torch.cuda.Event()
         self._staged_event = torch.cuda.Event()
         self._staged = None            # (data_ptr, shape) of the uint8 batch already augmented into the model
         if self.distributed:
-            # DDP's constructor broadcasts rank 0's parameters and buffers (train.py:199)
+            # DDP's constructor broadcasts rank 0's parameters and buffers (train.py:199); with frozen_bn the running
+            # statistics never change afterwards, so the ranks keep identical buffers
             dist.broadcast(model.flat_params, src=0, group=process_group)
             dist.broadcast(model._flat_buffers, src=0, group=process_group)
             model.sync_weights(force=True)
@@ -154,8 +159,10 @@ class TrainEngine:
         aug = self.augmentation
         apply = aug is not None and aug.train and aug.enabled
         key = (images.data_ptr(), tuple(images.shape))
-        # the buffer being written was last read by the step BEFORE the one in flight: wait for that step only
-        self._side.wait_event(self._prev_done)
+        # the buffer being written was last read by the forward BEFORE the one in flight (this engine's previous step, or
+        # whatever training / frozen forward ran in between): wait for that one only
+        if model._stem_free is not None:
+            self._side.wait_event(model._stem_free)
         if after is not None:
             self._side.wait_event(after)
         with torch.cuda.stream(self._side):
@@ -168,9 +175,15 @@ class TrainEngine:
             ws = aug.workspace(B * n_cams, H, W, self.device, tag="plasma_side") if apply else None
             model._ensure_bound()
             with torch.cuda.device(self.device):
-                _lib.call("argus_model_stage_input_u8", model._handle.ptr, images, params, arc_mask, ws, int(B), int(H),
-                          int(W), 1, int(apply), _lib.stream_ptr())
+                if self.frozen_bn:
+                    _lib.call("argus_model_stage_input_frozen_u8", model._handle.ptr, images, params, arc_mask, ws,
+                              int(B), int(H), int(W), int(apply), _lib.stream_ptr())
+                else:
+                    _lib.call("argus_model_stage_input_u8", model._handle.ptr, images, params, arc_mask, ws, int(B),
+                              int(H), int(W), 1, int(apply), _lib.stream_ptr())
             self._staged_event.record(self._side)
+        # the next forward into the stem buffers, whichever it is, waits for this write
+        model._staging = self._staged_event
         images.record_stream(self._side)
         if params is not None:
             params.record_stream(self._side)
@@ -197,28 +210,28 @@ class TrainEngine:
         """
         model = self.model
         lib_stream = _lib.stream_ptr()
-        model.train()
-        # everything enqueued so far (the previous step) precedes this event: a prefetch() issued after this call may
-        # overwrite the stem buffer of the previous step as soon as it fires
-        self._prev_done.record(torch.cuda.current_stream(self.device))
+        frozen = self.frozen_bn
+        training = not frozen
+        if training:
+            model.train()
+        # The model orders its stem buffers (NCameraCNN._stem_input_turn): the forward below waits for a staged batch
+        # (also when it is not the one given now: its write into the alternate buffer must be over before anything else
+        # is written there) and marks when everything enqueued before it, the previous step included, is done. A
+        # prefetch() issued after this call may overwrite the stem buffer of the previous step from then on.
         staged, self._staged = self._staged, None
-        if staged is not None:
-            # (also when the staged batch is not the one given now: its write into the alternate buffer must be over
-            # before anything else is staged there)
-            torch.cuda.current_stream(self.device).wait_event(self._staged_event)
         if staged is not None and images.dtype == torch.uint8 and staged == (images.data_ptr(), tuple(images.shape)):
-            out = model._forward_staged(images.shape[0], images.shape[2], images.shape[3])
+            out = model._forward_staged(images.shape[0], images.shape[2], images.shape[3], frozen=frozen)
         elif images.dtype == torch.uint8 and model.precision == "fp32":
             # fp32 parity mode: the same augmentation kernel with fp32 NCHW output, then the fp32 network
             aug = self.augmentation
             B_, n_cams, H, W, _ = images.shape
             if aug is not None and aug.train and aug.enabled:
                 arc_mask = aug.arc_mask(B_ * n_cams, H, W, self.device) if aug.gpu_spaghetti else None
-                out = model._forward_impl(aug.augment_batch(images, arc_mask=arc_mask), True)
+                out = model._forward_impl(aug.augment_batch(images, arc_mask=arc_mask), training, frozen=frozen)
             elif aug is not None and aug.gpu_spaghetti:
-                out = model._forward_impl(aug.spaghetti_batch(images), True)
+                out = model._forward_impl(aug.spaghetti_batch(images), training, frozen=frozen)
             else:
-                out = model._forward_impl(images, True)
+                out = model._forward_impl(images, training, frozen=frozen)
         elif images.dtype == torch.uint8:
             # fused augmentation + staging: uint8 pairs -> augmented bf16 stem input inside the model's staging buffer
             aug = self.augmentation
@@ -227,9 +240,10 @@ class TrainEngine:
             apply = aug is not None and aug.train and aug.enabled
             params = aug.sample_params(B_, n_cams, self.device, H=H, W=W) if apply else None
             ws = aug.workspace(B_ * n_cams, H, W, self.device) if apply else None
-            out = model._forward_impl(images, True, aug_params=params, augment=apply, arc_mask=arc_mask, plasma_ws=ws)
+            out = model._forward_impl(images, training, aug_params=params, augment=apply, arc_mask=arc_mask, plasma_ws=ws,
+                                      frozen=frozen)
         else:
-            out = model._forward_impl(images, True)
+            out = model._forward_impl(images, training, frozen=frozen)
         B = out.shape[0]
         targets = targets.to(device=self.device, dtype=torch.float32).contiguous()
         grad = torch.empty_like(out)

@@ -150,6 +150,9 @@ class NCameraCNN(nn.Module):
         self._bound_key = None
         self._flat_grads = None
         self._precision = "bf16"
+        # stream order of the two stem input buffers that training and frozen forwards share (see _stem_input_turn)
+        self._stem_free = None
+        self._staging = None
 
     def set_precision(self, precision: str) -> "NCameraCNN":
         """"bf16" (default): tcgen05 tensor-core path. "fp32": the fp32 parity mode of the C library (same weights,
@@ -327,17 +330,25 @@ class NCameraCNN(nn.Module):
         x = x.contiguous()
         self.sync_weights()
         out = torch.empty((B, 6), dtype=torch.float32, device=x.device)
+        if training or frozen:
+            self._stem_input_turn()
         with torch.cuda.device(x.device):
-            if frozen:
-                _lib.call("argus_model_forward_frozen", self._handle.ptr, x, int(is_u8), int(B), int(H), int(W), out,
-                          _lib.stream_ptr())
-            elif is_u8 and (augment or arc_mask is not None):
+            if is_u8 and (augment or arc_mask is not None):
                 # fused staging: arcs (bit mask) + augmentation (when `augment`) + /255 + bf16 space-to-depth packing
                 if augment and plasma_ws is None:
                     plasma_ws = torch.empty((B * self.n_cams, H, W // 32), dtype=torch.int32, device=x.device)
-                _lib.call("argus_model_stage_input_u8", self._handle.ptr, x, aug_params, arc_mask, plasma_ws, int(B),
-                          int(H), int(W), int(training), int(augment), _lib.stream_ptr())
-                _lib.call("argus_model_forward", self._handle.ptr, None, 0, int(B), int(H), int(W), int(training), out,
+                if frozen:
+                    _lib.call("argus_model_stage_input_frozen_u8", self._handle.ptr, x, aug_params, arc_mask, plasma_ws,
+                              int(B), int(H), int(W), int(augment), _lib.stream_ptr())
+                    _lib.call("argus_model_forward_frozen", self._handle.ptr, None, 0, int(B), int(H), int(W), out,
+                              _lib.stream_ptr())
+                else:
+                    _lib.call("argus_model_stage_input_u8", self._handle.ptr, x, aug_params, arc_mask, plasma_ws, int(B),
+                              int(H), int(W), int(training), int(augment), _lib.stream_ptr())
+                    _lib.call("argus_model_forward", self._handle.ptr, None, 0, int(B), int(H), int(W), int(training),
+                              out, _lib.stream_ptr())
+            elif frozen:
+                _lib.call("argus_model_forward_frozen", self._handle.ptr, x, int(is_u8), int(B), int(H), int(W), out,
                           _lib.stream_ptr())
             else:
                 _lib.call("argus_model_forward", self._handle.ptr, x, int(is_u8), int(B), int(H), int(W), int(training),
@@ -346,16 +357,38 @@ class NCameraCNN(nn.Module):
             self._flat_nbt += 1
         return out
 
-    def _forward_staged(self, B: int, H: int, W: int) -> torch.Tensor:
-        """Training forward over a batch already staged by argus_model_stage_input_u8 (TrainEngine.prefetch)."""
+    def _forward_staged(self, B: int, H: int, W: int, frozen: bool = False) -> torch.Tensor:
+        """Training forward (frozen: the frozen-statistics forward, which leaves num_batches_tracked alone) over a batch
+        already staged by argus_model_stage_input_u8 / argus_model_stage_input_frozen_u8 (TrainEngine.prefetch)."""
         self._ensure_bound()
         self.sync_weights()
         dev = self._flat_params.device
         out = torch.empty((B, 6), dtype=torch.float32, device=dev)
+        self._stem_input_turn()
         with torch.cuda.device(dev):
-            _lib.call("argus_model_forward", self._handle.ptr, None, 0, int(B), int(H), int(W), 1, out, _lib.stream_ptr())
-        self._flat_nbt += 1
+            if frozen:
+                _lib.call("argus_model_forward_frozen", self._handle.ptr, None, 0, int(B), int(H), int(W), out,
+                          _lib.stream_ptr())
+            else:
+                _lib.call("argus_model_forward", self._handle.ptr, None, 0, int(B), int(H), int(W), 1, out,
+                          _lib.stream_ptr())
+                self._flat_nbt += 1
         return out
+
+    def _stem_input_turn(self) -> None:
+        """Stream order for a forward that writes the model's pair of stem input buffers (training and frozen forwards
+        alternate through them; an eval forward has its own). The forward first waits for a batch being staged on
+        another stream (`_staging`, set by TrainEngine.prefetch). Then `_stem_free` is recorded: once it fires, the
+        buffer the next staging writes (the one the previous forward read, and its backward) is no longer in use."""
+        if self._precision != "bf16":
+            return
+        stream = torch.cuda.current_stream(self._flat_params.device)
+        if self._staging is not None:
+            stream.wait_event(self._staging)
+            self._staging = None
+        if self._stem_free is None:
+            self._stem_free = torch.cuda.Event()
+        self._stem_free.record(stream)
 
     def _backward_impl(self, grad_out: torch.Tensor, needs_grad=None) -> list[Optional[torch.Tensor]]:
         """Parameter gradients of the last training or frozen forward; None for parameters whose `needs_grad` entry is

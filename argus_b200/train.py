@@ -56,6 +56,12 @@ class TrainConfig:
     # not in the reference: "bf16" = tcgen05 tensor-core path (default), "fp32" = the fp32 parity mode (what the
     # reference computes with amp=False), see argus_model_set_precision in include/argus_b200.h
     precision: str = "bf16"
+    # not in the reference: fine-tuning with frozen batch norm -- every training forward uses the running statistics as
+    # constants and leaves them unchanged (TrainEngine(frozen_bn=True), argus_model_forward_frozen)
+    freeze_bn: bool = False
+    # not in the reference: a .pth (model.state_dict(), with or without DDP's `module.` prefix) loaded with strict=True
+    # before training starts; what freeze_bn fine-tunes from, since the running statistics of a fresh network are 0 / 1
+    init_model_path: Optional[str] = None
 
     # validation, printing, and saving
     val_epochs: int = 1
@@ -114,6 +120,15 @@ def _collate_u8(samples: list[dict]) -> dict:
             "cube_pose": torch.stack([s["cube_pose"] for s in samples])}
 
 
+def load_state_dict_for_init(path: str) -> dict:
+    """A saved `.pth` as `model.load_state_dict` takes it: the `module.` prefix of a checkpoint saved under multigpu
+    (state_dict_for_save) is removed."""
+    sd = torch.load(path, map_location="cpu", weights_only=True)
+    if sd and all(k.startswith("module.") for k in sd):
+        sd = {k[len("module."):]: v for k, v in sd.items()}
+    return sd
+
+
 def initialize_training(cfg: TrainConfig, rank: int = 0):
     """Sets up the training (reference: train.py:122-255). Returns the reference's 10-tuple
     `(train_dataloader, val_dataloader, model, optimizer, scheduler, loss_fn, wandb_id, train_sampler, val_sampler,
@@ -151,11 +166,13 @@ def initialize_training(cfg: TrainConfig, rank: int = 0):
     val_dataloader = DataLoader(val_dataset, shuffle=False, sampler=val_sampler, **common)
 
     model = NCameraCNN(cfg.model_config).to(device).set_precision(cfg.precision)
+    if cfg.init_model_path is not None:
+        model.load_state_dict(load_state_dict_for_init(cfg.init_model_path), strict=True)
     augmentation = Augmentation(cfg.augmentation_config, train=True, seed=cfg.random_seed + 7919 * rank,
                                 gpu_spaghetti=cfg.gpu_spaghetti) if cfg.use_augmentation else None
     scaler = GradScaler(enabled=cfg.amp)
     engine = TrainEngine(model, lr=cfg.learning_rate, max_grad_norm=cfg.max_grad_norm, augmentation=augmentation,
-                         scaler=scaler)
+                         scaler=scaler, frozen_bn=cfg.freeze_bn)
     scheduler = ReduceLROnPlateau(engine, patience=5, factor=0.5)
     loss_fn = geometric_loss_fn
 

@@ -296,9 +296,12 @@ int argus_stem_unpool_relu(const void* dpool, const void* idx, const void* poole
 int argus_pack_weight_scaled(const float* w, const float* scale, void* packed, int Cout, int Cin, int k, int kind,
                              void* stream);
 /* Eval-mode forward that can be differentiated: the running statistics are constants, the output is bit for bit that of
- * argus_model_forward(training = 0), and the running statistics, num_batches_tracked and the training input buffers
- * are left as they are. argus_model_backward and argus_model_input_grad (fp32 x only) then differentiate it, as long as
- * no other forward has run since. x as for argus_model_forward (no staged input). */
+ * argus_model_forward(training = 0), and the running statistics and num_batches_tracked are left as they are.
+ * argus_model_backward and argus_model_input_grad (fp32 x only) then differentiate it, as long as no other forward has
+ * run since. x as for argus_model_forward; the input goes to the same pair of model-owned stem buffers a training
+ * forward uses, so training and frozen forwards can alternate. x = NULL consumes the batch staged by
+ * argus_model_stage_input_frozen_u8 for the same (B, H, W); any other forward in between drops that batch (then this
+ * call fails). */
 int argus_model_forward_frozen(argus_model* m, const void* x, int is_u8, int B, int H, int W, float* out, void* stream);
 /* Fused augmentation + input staging: u8 (B*n_cams, H, W, 3) -> augmented stem input inside the model (training: one
  * of two model-owned staging buffers, so the NEXT batch -- of any size -- can be staged on another stream while the
@@ -306,6 +309,12 @@ int argus_model_forward_frozen(argus_model* m, const void* x, int is_u8, int B, 
  * arc_mask / plasma_ws: as for argus_augment. */
 int argus_model_stage_input_u8(argus_model* m, const void* images, const float* aug_params, const void* arc_mask,
                                void* plasma_ws, int B, int H, int W, int training, int apply, void* stream);
+/* argus_model_stage_input_u8 for a frozen-statistics forward: the same arguments (no training flag) and the same work,
+ * into the stem buffer the next argus_model_forward_frozen(x = NULL) call for the same (B, H, W) consumes. Fine-tuning
+ * with frozen batch norm can thus stage batch k+1 on another stream while step k runs. The staged input is bf16 and
+ * augmented, so it has no input gradient: argus_model_input_grad returns an error after such a forward. */
+int argus_model_stage_input_frozen_u8(argus_model* m, const void* images, const float* aug_params, const void* arc_mask,
+                                      void* plasma_ws, int B, int H, int W, int apply, void* stream);
 /* Precision mode. 0 (default): bf16 activations / weights on the tcgen05 tensor cores, fp32 accumulate.
  * 1: fp32 parity mode -- every tensor fp32, SIMT implicit-GEMM convolutions with fp32 FMA accumulation, reductions in
  * fp64; same parameter / gradient / buffer arenas and the same entry points. It exists to compare forward outputs,
