@@ -442,6 +442,17 @@ int argus_bn_apply_bits(const void* x, const float* scale, const float* shift, c
            static_cast<bf16*>(y), static_cast<uint8_t*>(relu_bits), nullptr, rows, C, static_cast<cudaStream_t>(stream));
   ARGUS_API_END
 }
+int argus_bn_apply_colsum(const void* x, const float* scale, const float* shift, int relu, void* y, void* relu_bits,
+                          float* colsum_partial, int64_t rows, int C, int* partials, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(partials != nullptr, "null argument");
+  *partials = bn_apply_grid(rows, C);
+  if (colsum_partial != nullptr)
+    bn_apply(static_cast<const bf16*>(x), scale, shift, nullptr, nullptr, nullptr, relu, static_cast<bf16*>(y),
+             static_cast<uint8_t*>(relu_bits), colsum_partial, rows, C, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
 int argus_bn_backward(void* dy, const void* x, const void* out, const float* scale, const float* shift,
                       const float* mean, const float* invstd, float* dgamma, float* dbeta, void* dx, int64_t rows,
                       int C, int mask_mode, void* stream) {
@@ -449,10 +460,11 @@ int argus_bn_backward(void* dy, const void* x, const void* out, const float* sca
   require_sm100();
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   bn_check_aligned(dy, x, out, dx);   // dx too: the reduce pass below already adds to dgamma / dbeta
+  float* scratch = lib_scratch(bn_bwd_scratch_elems());
   bn_bwd_reduce(static_cast<const bf16*>(dy), static_cast<const bf16*>(x), static_cast<const bf16*>(out), scale, shift,
-                mean, invstd, dgamma, dbeta, rows, C, mask_mode, lib_scratch(bn_bwd_scratch_elems()), s);
+                mean, invstd, dgamma, dbeta, rows, C, mask_mode, scratch, s);
   bn_bwd_apply(static_cast<bf16*>(dy), static_cast<const bf16*>(x), static_cast<const bf16*>(out), scale, shift, mean,
-               invstd, dgamma, dbeta, static_cast<bf16*>(dx), rows, C, mask_mode, s);
+               invstd, bn_bwd_sums(scratch), static_cast<bf16*>(dx), rows, C, mask_mode, s);
   ARGUS_API_END
 }
 int argus_maxpool_forward(const void* x, const float* scale, const float* shift, void* y, void* idx, int N, int H,
@@ -491,6 +503,14 @@ int argus_avgpool_backward(const void* dy, void* dx, int N, int HW, int C, void*
   ARGUS_API_BEGIN
   require_sm100();
   avgpool_bwd(static_cast<const bf16*>(dy), static_cast<bf16*>(dx), nullptr, N, HW, C, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+int argus_avgpool_backward_bits(const void* dy, void* dx, const void* relu_bits, int N, int HW, int C, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(relu_bits != nullptr, "null argument");
+  avgpool_bwd(static_cast<const bf16*>(dy), static_cast<bf16*>(dx), static_cast<const uint8_t*>(relu_bits), N, HW, C,
+              static_cast<cudaStream_t>(stream));
   ARGUS_API_END
 }
 

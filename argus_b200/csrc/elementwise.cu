@@ -380,9 +380,12 @@ void bn_fold_eval(const float* gamma, const float* beta, const float* running_me
   ARGUS_CUDA(cudaGetLastError());
 }
 
+// sums[0][c] = sum g, sums[1][c] = sum g * xhat of this call alone: the dx pass reads these, never dgamma / dbeta, which
+// may already hold other contributions (gradients accumulated over several backward calls)
 __global__ void __launch_bounds__(256)
-bn_bwd_finalize_kernel(const float* __restrict__ partial, int blocks, float* dgamma, float* dbeta, int C,
-                       const float* __restrict__ mean, const float* __restrict__ invstd) {
+bn_bwd_finalize_kernel(const float* __restrict__ partial, int blocks, float* dgamma, float* dbeta,
+                       float* __restrict__ sums, int C, const float* __restrict__ mean,
+                       const float* __restrict__ invstd) {
   pdl_prologue();
   double s[2];   // sum g, sum g * xhat
   if (!ordered_slot_sum<2>(partial, blocks, C, s)) return;
@@ -390,8 +393,11 @@ bn_bwd_finalize_kernel(const float* __restrict__ partial, int blocks, float* dga
   // mean != nullptr: the second sums are sum(g * x) of the RAW layer output (statistics slots of a dgrad epilogue,
   // bn_bwd_finalize_slots); centred and scaled here, once, in double
   if (mean != nullptr) s[1] = (s[1] - static_cast<double>(mean[c]) * s[0]) * static_cast<double>(invstd[c]);
-  dbeta[c] += static_cast<float>(s[0]);
-  dgamma[c] += static_cast<float>(s[1]);
+  const float db = static_cast<float>(s[0]), dg = static_cast<float>(s[1]);
+  sums[c] = db;
+  sums[C + c] = dg;
+  dbeta[c] += db;
+  dgamma[c] += dg;
 }
 
 __global__ void __launch_bounds__(256)
@@ -498,6 +504,9 @@ __device__ __forceinline__ void ring_consume(const uint8_t* smem, uint32_t sbase
     const uint4 a0 = ring_elem<R::kBytes0>(s0, t), a1 = ring_elem<R::kBytes0>(s0, t + 256);
     const uint4 b0 = ring_elem<R::kBytes1>(s1, t), b1 = ring_elem<R::kBytes1>(s1, t + 256);
     const uint4 e0 = ring_elem<R::kBytes2>(s2, t), e1 = ring_elem<R::kBytes2>(s2, t + 256);
+    // The stage is refilled by the async proxy (bulk copy) once every warp has arrived: order this thread's shared-memory
+    // reads before that write, or a read still in flight when the warp arrives can return the next lap's data.
+    fence_proxy_async_smem();
     __syncwarp();
     if ((t & 31) == 0) mbar_arrive(sbase + R::kOffBars + 8u * (R::kStages + s));   // stage free: data is in registers
     const int64_t i0 = c * kRingVec + t;
@@ -565,7 +574,8 @@ __device__ __forceinline__ F8 bn_masked_grad(const F8& d, const F8& xv, const ui
   }
   return g;
 }
-// dx = sc * (g - db/M - xhat * dg/M) with xhat = (x - mu) * is   ==   sc*g + k1*x + k0 (per-channel pointers at c0)
+// dx = sc * (g - db/M - xhat * dg/M) with xhat = (x - mu) * is   ==   sc*g + k1*x + k0 (per-channel pointers at c0;
+// db = sum g and dg = sum g * xhat of this pass: the [2][C] sums of bn_bwd_finalize_kernel)
 __device__ __forceinline__ void bn_dx_coeffs(const F8& sc, const float* mean, const float* invstd, const float* dgamma,
                                              const float* dbeta, float inv_rows, F8& k0, F8& k1) {
   const F8 mu = load8f(mean), is = load8f(invstd), dg = load8f(dgamma), db = load8f(dbeta);
@@ -687,8 +697,8 @@ __global__ void __launch_bounds__(kRingThreads, 2)
 bn_bwd_apply_ring_kernel(uint4* __restrict__ dy, const uint4* __restrict__ x, const uint4* __restrict__ out,
                          const float* __restrict__ scale, const float* __restrict__ shift,
                          const float* __restrict__ mean, const float* __restrict__ invstd,
-                         const float* __restrict__ dgamma, const float* __restrict__ dbeta, uint4* __restrict__ dx,
-                         int64_t nvec, int cvec, float inv_rows) {
+                         const float* __restrict__ sums, uint4* __restrict__ dx, int64_t nvec, int cvec,
+                         float inv_rows) {
   pdl_prologue();
   using R = BnRing<MASK>;
   extern __shared__ __align__(128) uint8_t ring_smem[];
@@ -704,7 +714,7 @@ bn_bwd_apply_ring_kernel(uint4* __restrict__ dy, const uint4* __restrict__ x, co
   F8 sh;
   if (MASK == 1) sh = load8f(shift + c0);
   F8 k0, k1;
-  bn_dx_coeffs(sc, mean + c0, invstd + c0, dgamma + c0, dbeta + c0, inv_rows, k0, k1);
+  bn_dx_coeffs(sc, mean + c0, invstd + c0, sums + cvec * 8 + c0, sums + c0, inv_rows, k0, k1);
   auto body = [&](int64_t i, const uint4& dyv, const uint4& xv4, const uint4& ov4) {
     const F8 xv = unpack8(xv4);
     const F8 g = bn_masked_grad<MASK>(unpack8(dyv), xv, ov4, sc, sh);
@@ -757,7 +767,10 @@ void bn_apply(const bf16* x, const float* scale, const float* shift, const bf16*
     launch_ring<bn_apply_ring_kernel<2, false>, ApplyRing<2>>(grid, s, X, scale, shift, R, rscale, rshift, relu, Y, relu_bits, colsum_partial, nvec, cvec);
 }
 
-int64_t bn_bwd_scratch_elems() { return 4LL * num_sms() * 2 * 2048; }
+// per-block partials (up to 4 x SMs blocks of [2][2048]), then the [2][C] sums of the last finalize
+static int64_t bn_bwd_partial_elems() { return 4LL * num_sms() * 2 * 2048; }
+int64_t bn_bwd_scratch_elems() { return bn_bwd_partial_elems() + 2 * 2048; }
+float* bn_bwd_sums(float* scratch) { return scratch + bn_bwd_partial_elems(); }
 
 void bn_bwd_reduce(const bf16* dy, const bf16* x, const bf16* out, const float* scale, const float* shift,
                    const float* mean, const float* invstd, float* dgamma, float* dbeta, int64_t rows, int C,
@@ -787,20 +800,21 @@ void bn_bwd_reduce(const bf16* dy, const bf16* x, const bf16* out, const float* 
       break;
     default: throw Error("bad mask_mode");
   }
-  launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, scratch, grid, dgamma, dbeta, C, nullptr, nullptr);
+  launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, scratch, grid, dgamma, dbeta, bn_bwd_sums(scratch), C,
+                nullptr, nullptr);
   ARGUS_CUDA(cudaGetLastError());
 }
 
 void bn_bwd_finalize_slots(const float* partial, int slots, const float* mean, const float* invstd, float* dgamma,
-                           float* dbeta, int C, cudaStream_t s) {
+                           float* dbeta, float* sums, int C, cudaStream_t s) {
   ProfileScope prof("bn_bwd_reduce", s, 0, static_cast<double>(slots) * 2 * C * 4);
-  launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, partial, slots, dgamma, dbeta, C, mean, invstd);
+  launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, partial, slots, dgamma, dbeta, sums, C, mean, invstd);
   ARGUS_CUDA(cudaGetLastError());
 }
 
 void bn_bwd_apply(bf16* dy, const bf16* x, const bf16* out, const float* scale, const float* shift,
-                  const float* mean, const float* invstd, const float* dgamma, const float* dbeta, bf16* dx,
-                  int64_t rows, int C, int mask_mode, cudaStream_t s) {
+                  const float* mean, const float* invstd, const float* sums, bf16* dx, int64_t rows, int C,
+                  int mask_mode, cudaStream_t s) {
   bn_check_aligned(dy, x, out, dx);
   ProfileScope prof("bn_bwd_apply", s, 0, static_cast<double>(rows) * C * (mask_mode == 2 ? 10.0 : (mask_mode == 3 ? 6.125 : 6.0)));
   ARGUS_CHECK(C % 8 == 0 && is_pow2(C / 8) && C <= 2048, "bn_bwd_apply: C/8 must be a power of two <= 256");
@@ -813,10 +827,10 @@ void bn_bwd_apply(bf16* dy, const bf16* x, const bf16* out, const float* scale, 
   auto O = reinterpret_cast<const uint4*>(out);
   auto DX = reinterpret_cast<uint4*>(dx);
   switch (mask_mode) {
-    case 0: launch_ring<bn_bwd_apply_ring_kernel<0>, BnRing<0>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
-    case 1: launch_ring<bn_bwd_apply_ring_kernel<1>, BnRing<1>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
-    case 2: launch_ring<bn_bwd_apply_ring_kernel<2>, BnRing<2>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
-    case 3: launch_ring<bn_bwd_apply_ring_kernel<3>, BnRing<3>>(grid, s, DY, X, O, scale, shift, mean, invstd, dgamma, dbeta, DX, nvec, cvec, inv_rows); break;
+    case 0: launch_ring<bn_bwd_apply_ring_kernel<0>, BnRing<0>>(grid, s, DY, X, O, scale, shift, mean, invstd, sums, DX, nvec, cvec, inv_rows); break;
+    case 1: launch_ring<bn_bwd_apply_ring_kernel<1>, BnRing<1>>(grid, s, DY, X, O, scale, shift, mean, invstd, sums, DX, nvec, cvec, inv_rows); break;
+    case 2: launch_ring<bn_bwd_apply_ring_kernel<2>, BnRing<2>>(grid, s, DY, X, O, scale, shift, mean, invstd, sums, DX, nvec, cvec, inv_rows); break;
+    case 3: launch_ring<bn_bwd_apply_ring_kernel<3>, BnRing<3>>(grid, s, DY, X, O, scale, shift, mean, invstd, sums, DX, nvec, cvec, inv_rows); break;
     default: throw Error("bad mask_mode");
   }
 }
@@ -1003,8 +1017,8 @@ __global__ void __launch_bounds__(256)   // (256, 3) forces 80 registers and spi
 stem_pool_bn_bwd_kernel(const uint4* __restrict__ dpool, const uint2* __restrict__ idx, const uint4* __restrict__ raw,
                         const float* __restrict__ scale, const float* __restrict__ shift,
                         const float* __restrict__ mean, const float* __restrict__ invstd,
-                        const float* __restrict__ dgamma, const float* __restrict__ dbeta, float* __restrict__ partial,
-                        uint4* __restrict__ dx, int N, int H, int W, float inv_rows, int lg_wo, int lg_ho) {
+                        const float* __restrict__ sums, float* __restrict__ partial, uint4* __restrict__ dx, int N,
+                        int H, int W, float inv_rows, int lg_wo, int lg_ho) {
   pdl_prologue();
   constexpr int cvec = 8;   // C = 64
   __shared__ float red[16][256];
@@ -1013,7 +1027,7 @@ stem_pool_bn_bwd_kernel(const uint4* __restrict__ dpool, const uint2* __restrict
   const int c0 = cv * 8;
   const F8 sc = load8f(scale + c0), sh = load8f(shift + c0);
   F8 k0, k1;
-  if (APPLY) bn_dx_coeffs(sc, mean + c0, invstd + c0, dgamma + c0, dbeta + c0, inv_rows, k0, k1);
+  if (APPLY) bn_dx_coeffs(sc, mean + c0, invstd + c0, sums + 64 + c0, sums + c0, inv_rows, k0, k1);
   float a_dy[8], a_dyx[8];
 #pragma unroll
   for (int k = 0; k < 8; ++k) a_dy[k] = a_dyx[k] = 0.f;
@@ -1125,17 +1139,18 @@ void stem_pool_bn_backward(const bf16* dpool, const uint8_t* idx, const bf16* ra
   {
     ProfileScope prof("bn_bwd_reduce", s, 0, static_cast<double>(rows) * C * (2.0 + 0.75));
     const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((threads + 255) / 256, 4LL * num_sms())));
-    launch_kernel(stem_pool_bn_bwd_kernel<0>, grid, 256, 0, s, DP, ID, RW, scale, shift, mean, invstd, nullptr, nullptr, scratch,
+    launch_kernel(stem_pool_bn_bwd_kernel<0>, grid, 256, 0, s, DP, ID, RW, scale, shift, mean, invstd, nullptr, scratch,
                                                     nullptr, N, H, W, inv_rows, lg_wo, lg_ho);
     ARGUS_CUDA(cudaGetLastError());
-    launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, scratch, grid, dgamma, dbeta, C, nullptr, nullptr);
+    launch_kernel(bn_bwd_finalize_kernel, (C + 7) / 8, 256, 0, s, scratch, grid, dgamma, dbeta, bn_bwd_sums(scratch), C,
+                  nullptr, nullptr);
     ARGUS_CUDA(cudaGetLastError());
   }
   {
     ProfileScope prof("bn_bwd_apply", s, 0, static_cast<double>(rows) * C * (4.0 + 0.75));
     const int grid = grid_for(threads, 256);
-    launch_kernel(stem_pool_bn_bwd_kernel<1>, grid, 256, 0, s, DP, ID, RW, scale, shift, mean, invstd, dgamma, dbeta, nullptr,
-                                                    reinterpret_cast<uint4*>(dx), N, H, W, inv_rows, lg_wo, lg_ho);
+    launch_kernel(stem_pool_bn_bwd_kernel<1>, grid, 256, 0, s, DP, ID, RW, scale, shift, mean, invstd,
+                  bn_bwd_sums(scratch), nullptr, reinterpret_cast<uint4*>(dx), N, H, W, inv_rows, lg_wo, lg_ho);
     ARGUS_CUDA(cudaGetLastError());
   }
 }

@@ -87,20 +87,23 @@ void colsum_finalize(const float* partial, int blocks, float* out, int C, cudaSt
 // mask_mode: 0 = no ReLU after this BN, 1 = ReLU directly after (mask recomputed from x), 2 = ReLU after a residual
 // add (mask = out > 0), 3 = like 2 but `out` points to the relu_bits written by bn_apply. Accumulates dgamma += sum(g * xhat), dbeta += sum(g) with g = masked dy.
 // Deterministic: every block writes its partial sums to `scratch` (>= bn_bwd_scratch_elems() floats), a second tiny
-// kernel adds them in block order.
+// kernel adds them in block order. This call's sums alone also go to bn_bwd_sums(scratch), [2][C]: sum(g), sum(g * xhat).
 void bn_bwd_reduce(const bf16* dy, const bf16* x, const bf16* out, const float* scale, const float* shift,
                    const float* mean, const float* invstd, float* dgamma, float* dbeta, int64_t rows, int C,
                    int mask_mode, float* scratch, cudaStream_t s);
 int64_t bn_bwd_scratch_elems();
+float* bn_bwd_sums(float* scratch);
 // The same sums when a dgrad epilogue already reduced them (Epilogue::bn_raw): partial = [slots][2][C] with sum(g) and
-// sum(g * x) of the raw layer output x per slot; dbeta += sum(g), dgamma += (sum(g * x) - mean * sum(g)) * invstd.
+// sum(g * x) of the raw layer output x per slot; dbeta += sum(g), dgamma += (sum(g * x) - mean * sum(g)) * invstd, and
+// sums [2][C] = those two terms alone.
 void bn_bwd_finalize_slots(const float* partial, int slots, const float* mean, const float* invstd, float* dgamma,
-                           float* dbeta, int C, cudaStream_t s);
-// dx = scale * (g - dbeta/rows - xhat * dgamma/rows); mask_mode 2 also overwrites dy with g (mask_mode 3 leaves dy
-// untouched: the consumers of the identity-branch gradient apply the bit mask themselves).
+                           float* dbeta, float* sums, int C, cudaStream_t s);
+// dx = scale * (g - sum(g)/rows - xhat * sum(g * xhat)/rows) with sums = [2][C] (sum g, sum g * xhat) of THIS layer's
+// reduction (never the dgamma / dbeta accumulators, which may hold earlier gradients); mask_mode 2 also overwrites dy
+// with g (mask_mode 3 leaves dy untouched: the consumers of the identity-branch gradient apply the bit mask themselves).
 void bn_bwd_apply(bf16* dy, const bf16* x, const bf16* out, const float* scale, const float* shift,
-                  const float* mean, const float* invstd, const float* dgamma, const float* dbeta, bf16* dx,
-                  int64_t rows, int C, int mask_mode, cudaStream_t s);
+                  const float* mean, const float* invstd, const float* sums, bf16* dx, int64_t rows, int C,
+                  int mask_mode, cudaStream_t s);
 
 // ---- pooling ----------------------------------------------------------------------------------------------
 // 3x3 stride-2 pad-1 max pooling of relu(x*scale+shift) (scale == nullptr: x is already activated).
@@ -110,7 +113,8 @@ void maxpool_fwd(const bf16* x, const float* scale, const float* shift, bf16* y,
 void maxpool_bwd(const bf16* dy, const uint8_t* idx, bf16* dx, int N, int H, int W, int C, cudaStream_t s);
 // Stem tail backward in two passes over the stem convolution output `raw` (N, H, W, 64): max-pool backward (from the
 // pooled gradient dpool (N, H/2, W/2, 64) and the arg-max bytes), ReLU mask and batch-norm backward fused, the
-// un-pooled gradient is never written. dgamma / dbeta are accumulated (+=); dx = gradient wrt `raw`.
+// un-pooled gradient is never written. dgamma / dbeta are accumulated (+=); dx = gradient wrt `raw`, formed from this
+// call's sums alone (bn_bwd_sums(scratch); scratch: >= bn_bwd_scratch_elems() floats).
 void stem_pool_bn_backward(const bf16* dpool, const uint8_t* idx, const bf16* raw, const float* scale,
                            const float* shift, const float* mean, const float* invstd, float* dgamma, float* dbeta,
                            bf16* dx, int N, int H, int W, int C, float* scratch, cudaStream_t s);

@@ -838,7 +838,7 @@ void Model::bn_backward(const ConvRef& c, bf16* dy, const bf16* raw, const bf16*
   bn_bwd_reduce(dy, raw, out, sc, sc + C, sc + 2 * C, sc + 3 * C, dgamma, dbeta, rows, C, mask, bn_bwd_scratch_, s);
   // the apply pass overwrites a gradient buffer that an in-flight weight-gradient GEMM may still be reading
   join_wgrad(s);
-  bn_bwd_apply(dy, raw, out, sc, sc + C, sc + 2 * C, sc + 3 * C, dgamma, dbeta, dx, rows, C, mask, s);
+  bn_bwd_apply(dy, raw, out, sc, sc + C, sc + 2 * C, sc + 3 * C, bn_bwd_sums(bn_bwd_scratch_), dx, rows, C, mask, s);
 }
 
 void Model::attach_bn_reduction(Epilogue& e, const ConvLaunch& l, const BnRed& red, cudaStream_t s) {
@@ -858,10 +858,11 @@ void Model::bn_backward_reduced(const ConvRef& c, bf16* dy, const bf16* raw, bf1
   float* dgamma = grads_dev_ + c.bn.gamma_off;
   float* dbeta = grads_dev_ + c.bn.beta_off;
   const int C = c.bn.C;
-  bn_bwd_finalize_slots(bnred_stats_, bnred_slots_, sc + 2 * C, sc + 3 * C, dgamma, dbeta, C, s);
+  float* sums = bn_bwd_sums(bn_bwd_scratch_);
+  bn_bwd_finalize_slots(bnred_stats_, bnred_slots_, sc + 2 * C, sc + 3 * C, dgamma, dbeta, sums, C, s);
   // the apply pass overwrites a gradient buffer that an in-flight weight-gradient GEMM may still be reading
   join_wgrad(s);
-  bn_bwd_apply(dy, raw, nullptr, sc, sc + C, sc + 2 * C, sc + 3 * C, dgamma, dbeta, dx, rows, C, 0, s);   // dy is masked
+  bn_bwd_apply(dy, raw, nullptr, sc, sc + C, sc + 2 * C, sc + 3 * C, sums, dx, rows, C, 0, s);   // dy is masked
 }
 
 void Model::conv_backward(const ConvPlan& cp, const bf16* residual, const uint8_t* out_bits, float* out_stats,

@@ -158,10 +158,16 @@ int argus_bn_apply(const void* x, const float* scale, const float* shift, const 
  * relu_bits must be 16-byte aligned too. */
 int argus_bn_apply_bits(const void* x, const float* scale, const float* shift, const void* res, const float* rscale,
                         const float* rshift, int relu, void* y, void* relu_bits, int64_t rows, int C, void* stream);
+/* The plain variant (no residual) that also writes per-block column sums of the stored y: colsum_partial
+ * [*partials][C] fp32, block b's sums in row b (their sum in row order is colsum(y)). relu_bits nullable, as for
+ * argus_bn_apply_bits. *partials is always set; with colsum_partial NULL nothing runs (sizing query). */
+int argus_bn_apply_colsum(const void* x, const float* scale, const float* shift, int relu, void* y, void* relu_bits,
+                          float* colsum_partial, int64_t rows, int C, int* partials, void* stream);
 /* BN (+ReLU) backward. mask_mode 0: no ReLU; 1: ReLU right after the BN; 2: ReLU after a residual add (mask = out > 0,
  * dy is overwritten with the masked gradient); 3: like 2 but `out` is the relu_bits mask of argus_bn_apply_bits and dy
- * is left untouched. dgamma / dbeta are ADDED to (caller zeroes); dx = d loss / d x. dy, x, out and dx must be 16-byte
- * aligned: a misaligned pointer is an error, reported before dgamma / dbeta are touched. */
+ * is left untouched. This call's dgamma / dbeta are ADDED to the accumulators; dx = d loss / d x depends only on this
+ * call's inputs, whatever the accumulators held. dy, x, out and dx must be 16-byte aligned: a misaligned pointer is an
+ * error, reported before dgamma / dbeta are touched. */
 int argus_bn_backward(void* dy, const void* x, const void* out, const float* scale, const float* shift,
                       const float* mean, const float* invstd, float* dgamma, float* dbeta, void* dx, int64_t rows,
                       int C, int mask_mode, void* stream);
@@ -171,12 +177,15 @@ int argus_maxpool_forward(const void* x, const float* scale, const float* shift,
 int argus_maxpool_backward(const void* dy, const void* idx, void* dx, int N, int H, int W, int C, void* stream);
 /* Stem tail backward, fused: max-pool backward (pooled gradient dpool (N,H/2,W/2,64) + arg-max bytes idx) -> ReLU mask
  * -> batch-norm backward over the stem convolution output raw (N,H,W,64). Equivalent to argus_maxpool_backward followed
- * by argus_bn_backward(mask_mode 1) without materialising the un-pooled gradient. dgamma / dbeta are ADDED to. */
+ * by argus_bn_backward(mask_mode 1) without materialising the un-pooled gradient. dgamma / dbeta are ADDED to; dx depends
+ * only on this call's inputs. */
 int argus_stem_pool_bn_backward(const void* dpool, const void* idx, const void* raw, const float* scale,
                                 const float* shift, const float* mean, const float* invstd, float* dgamma,
                                 float* dbeta, void* dx, int N, int H, int W, int C, void* stream);
 int argus_avgpool_forward(const void* x, void* y, int N, int HW, int C, void* stream);
 int argus_avgpool_backward(const void* dy, void* dx, int N, int HW, int C, void* stream);
+/* dx = dy / HW masked by the ReLU bit mask relu_bits [N*HW][C/8] of the pooled tensor (the last block's output). */
+int argus_avgpool_backward_bits(const void* dy, void* dx, const void* relu_bits, int N, int HW, int C, void* stream);
 
 /* ---- fp32 parity-mode primitives (argus_model_set_precision(m, 1) runs the network on these) ---------------------
  * All tensors fp32; activations NHWC; weights and weight gradients in PyTorch's [Cout][Cin][k][k] layout; padding k/2.
