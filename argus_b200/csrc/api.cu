@@ -262,6 +262,67 @@ int argus_conv_instances_all(int* keys, int cap, int* n) {
   ARGUS_API_END
 }
 
+int argus_conv2d_wgrad_launch_info(int mode, int N, int H, int W, int Cin, int Cout, int k, int stride, int kind,
+                                   int* out, int cap) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(out != nullptr && cap >= ARGUS_WGRAD_INFO_INTS, "launch info buffer too small");
+  ARGUS_CUDA(cudaFree(nullptr));   // tensor-map encoding needs a current context
+  // as in argus_conv2d_launch_info: planning encodes tensor maps against a dummy address and reads no memory
+  static __align__(1024) char dummy[1024];
+  const bf16* d = reinterpret_cast<const bf16*>(dummy);
+  float* f = reinterpret_cast<float*>(dummy);
+  WgradLaunch l;
+  if (mode == 0) {
+    ConvShape s = make_shape(N, H, W, Cin, Cout, k, stride, kind);
+    l = plan_conv_wgrad(s, d, d, f);
+  } else if (mode == 1) {
+    l = plan_conv_wgrad_gram(make_shape(N, H, W, Cin, Cout, 1, stride, 0), d, d, f);
+  } else if (mode == 2) {
+    ConvShape s = make_shape(N, H, W, Cin, Cout, 1, stride, 0);
+    validate_shape(s);
+    l = plan_gram(s, d, f);
+  } else {
+    throw Error("unknown weight-gradient mode");
+  }
+  const WgradLaunchInfo li = wgrad_launch_info(l);
+  ARGUS_CHECK(li.scratch_elems <= INT32_MAX, "scratch size does not fit the launch info record");
+  const int v[ARGUS_WGRAD_INFO_INTS] = {li.xpose, li.n, li.stacked, li.co_split, li.num_taps, li.num_co_tiles,
+                                        li.num_ci_tiles, li.num_ksplits, li.kblocks_total, li.grid,
+                                        static_cast<int>(li.scratch_elems)};
+  std::memcpy(out, v, sizeof(v));
+  ARGUS_API_END
+}
+
+int argus_wgrad_instances_get(int* keys, int cap, int* n) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(n != nullptr && (keys != nullptr || cap == 0), "null argument");
+  const auto rec = wgrad_instances_recorded();
+  *n = static_cast<int>(rec.size());
+  for (int i = 0; i < *n && 5 * (i + 1) <= cap; ++i) std::memcpy(keys + 5 * i, rec[i].data(), 5 * sizeof(int));
+  ARGUS_API_END
+}
+
+int argus_wgrad_instances_all(int* keys, int cap, int* n) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(n != nullptr && (keys != nullptr || cap == 0), "null argument");
+  const auto all = wgrad_instances_all();
+  *n = static_cast<int>(all.size());
+  for (int i = 0; i < *n && 2 * (i + 1) <= cap; ++i) std::memcpy(keys + 2 * i, all[i].data(), 2 * sizeof(int));
+  ARGUS_API_END
+}
+
+int argus_lib_scratch_fill(int64_t elems, int byte_value, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(elems >= 0, "negative size");
+  if (elems == 0) return 0;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  ARGUS_CUDA(cudaMemsetAsync(lib_scratch(elems), byte_value & 0xff, elems * sizeof(float), st));
+  pdl_break(st, kPdlAfterMemop);
+  ARGUS_API_END
+}
+
 int argus_conv2d_gram(const void* x, float* g, int N, int H, int W, int Cin, int Cout, int stride, void* stream) {
   ARGUS_API_BEGIN
   require_sm100();

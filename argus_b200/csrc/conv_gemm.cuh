@@ -948,7 +948,7 @@ struct WgradXposeParams {
   float* partial;         // [num_splits][64][dw_row_stride]
 };
 
-template <int NBOX>   // padded to an even number: 2, 4 or 10
+template <int NBOX>   // padded to an even number: 4 (stem) or 10 (3x3, Cin = 64)
 struct WgradXposeSmem {
   static constexpr int kStageBytes = 8192 + NBOX * 8192;
   static constexpr int kStagesRaw = 196608 / kStageBytes;

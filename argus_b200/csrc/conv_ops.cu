@@ -523,7 +523,7 @@ WgradLaunch plan_conv_wgrad(const ConvShape& s, const __nv_bfloat16* dy, const _
         b.out_off = static_cast<int16_t>(p.taps[t].b_off + cb * 64);
         x.boxes[nb++] = b;
       }
-    const int padded = nb <= 2 ? 2 : (nb <= 4 ? 4 : 10);
+    const int padded = nb <= 4 ? 4 : 10;
     l.xpose_nbox = padded;
     x.kblocks_total = p.kblocks_total;
     x.num_splits = std::max(1, std::min(num_sms(), p.kblocks_total / 4));
@@ -656,6 +656,7 @@ const ConvInstanceEntry& find_instance(const ConvInstance& c) {
 std::mutex g_record_mu;
 std::atomic<bool> g_recording{false};
 std::set<std::array<int, 5>> g_recorded;
+std::set<std::array<int, 5>> g_recorded_wgrad;
 }  // namespace
 
 ConvGemmParams epilogue_params(const ConvLaunch& l, const Epilogue& e) {
@@ -736,7 +737,7 @@ ConvLaunchInfo conv_launch_info(const ConvLaunch& l, const Epilogue& e) {
 
 void conv_instances_record(bool on) {
   std::lock_guard<std::mutex> lk(g_record_mu);
-  if (on) g_recorded.clear();
+  if (on) { g_recorded.clear(); g_recorded_wgrad.clear(); }
   g_recording = on;
 }
 std::vector<std::array<int, 3>> conv_instances_all() {
@@ -747,6 +748,10 @@ std::vector<std::array<int, 3>> conv_instances_all() {
 std::vector<std::array<int, 5>> conv_instances_recorded() {
   std::lock_guard<std::mutex> lk(g_record_mu);
   return std::vector<std::array<int, 5>>(g_recorded.begin(), g_recorded.end());
+}
+std::vector<std::array<int, 5>> wgrad_instances_recorded() {
+  std::lock_guard<std::mutex> lk(g_record_mu);
+  return std::vector<std::array<int, 5>>(g_recorded_wgrad.begin(), g_recorded_wgrad.end());
 }
 
 void launch_conv(const ConvLaunch& l, const Epilogue& e, cudaStream_t stream) {
@@ -827,34 +832,69 @@ wgrad_reduce_kernel(const float4* __restrict__ partial, float4* __restrict__ dw,
 }
 
 template <int NBOX>
-static void launch_wgrad_xpose_t(const WgradXposeParams& p, cudaStream_t stream) {
+static void launch_wgrad_xpose_t(const WgradLaunch& l, int grid, cudaStream_t stream) {
   using L = WgradXposeSmem<NBOX>;
   static bool configured = false;
   if (!configured) {
     ARGUS_CUDA(cudaFuncSetAttribute(wgrad_xpose_kernel<NBOX>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
     configured = true;
   }
-  launch_kernel(wgrad_xpose_kernel<NBOX>, p.num_splits, kWgradThreads, L::kTotal, stream, p);
+  launch_kernel(wgrad_xpose_kernel<NBOX>, grid, kWgradThreads, L::kTotal, stream, l.xp);
   ARGUS_CUDA(cudaGetLastError());
 }
 
 template <int BN>
-static void launch_wgrad_t(const WgradParams& p, cudaStream_t stream) {
+static void launch_wgrad_t(const WgradLaunch& l, int grid, cudaStream_t stream) {
   using L = WgradSmem<BN>;
   static bool configured = false;
   if (!configured) {
     ARGUS_CUDA(cudaFuncSetAttribute(wgrad_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kTotal));
     configured = true;
   }
-  const int items = p.num_co_tiles * p.num_ci_tiles * p.num_ksplits * p.num_taps;
-  const int grid = std::min(items, num_sms());
-  launch_kernel(wgrad_kernel<BN>, grid, kWgradThreads, L::kTotal, stream, p);
+  launch_kernel(wgrad_kernel<BN>, grid, kWgradThreads, L::kTotal, stream, l.p);
   ARGUS_CUDA(cudaGetLastError());
+}
+
+namespace {
+// Every weight-gradient kernel instance the library compiles: (transposed, BLOCK_N or padded box count).
+struct WgradInstanceEntry {
+  int xpose, n;
+  void (*launch)(const WgradLaunch&, int, cudaStream_t);
+};
+const WgradInstanceEntry kWgradInstances[] = {
+    {0, 64, &launch_wgrad_t<64>}, {0, 128, &launch_wgrad_t<128>}, {0, 256, &launch_wgrad_t<256>},
+    {1, 4, &launch_wgrad_xpose_t<4>}, {1, 10, &launch_wgrad_xpose_t<10>},
+};
+}  // namespace
+
+std::vector<std::array<int, 2>> wgrad_instances_all() {
+  std::vector<std::array<int, 2>> v;
+  for (const auto& e : kWgradInstances) v.push_back({e.xpose, e.n});
+  return v;
+}
+
+WgradLaunchInfo wgrad_launch_info(const WgradLaunch& l) {
+  WgradLaunchInfo info;
+  const WgradParams& p = l.p;
+  info.xpose = l.xpose_nbox > 0 ? 1 : 0;
+  info.n = info.xpose ? l.xpose_nbox : l.block_n;
+  info.stacked = p.stacked;
+  info.co_split = p.co_split;
+  info.num_taps = p.num_taps;
+  info.num_co_tiles = p.num_co_tiles;
+  info.num_ci_tiles = p.num_ci_tiles;
+  info.num_ksplits = p.num_ksplits;
+  info.kblocks_total = p.kblocks_total;
+  info.grid = info.xpose ? l.xp.num_splits
+                         : std::min(p.num_co_tiles * p.num_ci_tiles * p.num_ksplits * p.num_taps, num_sms());
+  info.scratch_elems = wgrad_scratch_elems(l);
+  return info;
 }
 
 void launch_wgrad(const WgradLaunch& l0, float* scratch, cudaStream_t stream) {
   WgradLaunch l = l0;
-  const int64_t need = wgrad_scratch_elems(l);
+  const WgradLaunchInfo info = wgrad_launch_info(l);
+  const int64_t need = info.scratch_elems;
   ARGUS_CHECK(need == 0 || scratch != nullptr, "split-K weight gradient needs a scratch buffer");
   l.p.partial = scratch;
   l.p.partial_stride = static_cast<long long>(l.p.cout) * l.p.dw_row_stride;
@@ -869,20 +909,16 @@ void launch_wgrad(const WgradLaunch& l0, float* scratch, cudaStream_t stream) {
   if (l.xpose_nbox > 0) {
     ARGUS_CHECK(scratch != nullptr, "transposed weight gradient needs a scratch buffer");
     l.xp.partial = scratch;
-    switch (l.xpose_nbox) {
-      case 2: launch_wgrad_xpose_t<2>(l.xp, stream); break;
-      case 4: launch_wgrad_xpose_t<4>(l.xp, stream); break;
-      case 10: launch_wgrad_xpose_t<10>(l.xp, stream); break;
-      default: throw Error("unsupported transposed wgrad configuration");
-    }
-  } else {
-    switch (l.block_n) {
-      case 64: launch_wgrad_t<64>(l.p, stream); break;
-      case 128: launch_wgrad_t<128>(l.p, stream); break;
-      case 256: launch_wgrad_t<256>(l.p, stream); break;
-      default: throw Error("unsupported wgrad tile configuration");
-    }
   }
+  const WgradInstanceEntry* entry = nullptr;
+  for (const auto& e : kWgradInstances)
+    if (e.xpose == info.xpose && e.n == info.n) entry = &e;
+  if (entry == nullptr) throw Error("unsupported wgrad configuration");
+  if (g_recording) {
+    std::lock_guard<std::mutex> lk(g_record_mu);
+    g_recorded_wgrad.insert({info.xpose, info.n, info.stacked, info.co_split > 0 ? 1 : 0, info.num_ksplits > 1 ? 1 : 0});
+  }
+  entry->launch(l, info.grid, stream);
   if (need > 0) {
     // every (split, cout, tap, ci) word of the scratch was written by exactly one work item
     const int64_t n4 = l.p.partial_stride / 4;

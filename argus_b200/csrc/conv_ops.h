@@ -130,6 +130,19 @@ std::vector<std::array<int, 3>> conv_instances_all();
 int stat_slots(const ConvLaunch& l);
 // elements of split-K scratch this launch needs (0 when it does not split)
 int64_t wgrad_scratch_elems(const WgradLaunch& l);
+// Everything launch_wgrad decides for l without launching: the kernel instance (tile kernel with BLOCK_N = n, or the
+// transposed kernel with n padded boxes), the stacked operand, the split-K geometry, the grid and the scratch size.
+struct WgradLaunchInfo {
+  int xpose = 0, n = 0, stacked = 0, co_split = 0, num_taps = 0, num_co_tiles = 0, num_ci_tiles = 0;
+  int num_ksplits = 0, kblocks_total = 0, grid = 0;
+  int64_t scratch_elems = 0;
+};
+WgradLaunchInfo wgrad_launch_info(const WgradLaunch& l);
+// While conv_instances_record is on, launch_wgrad adds the key (xpose, n, stacked, co_split > 0, num_ksplits > 1) of
+// every launch to a second host-side set.
+std::vector<std::array<int, 5>> wgrad_instances_recorded();
+// (xpose, n) of every kernel instance launch_wgrad can dispatch to
+std::vector<std::array<int, 2>> wgrad_instances_all();
 // scratch: at least wgrad_scratch_elems(l) floats (may be null when that is 0)
 void launch_wgrad(const WgradLaunch& l, float* scratch, cudaStream_t stream);
 

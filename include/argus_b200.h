@@ -107,6 +107,22 @@ int argus_conv_instances_record(int on);
 int argus_conv_instances_get(int* keys, int cap, int* n);
 /* Every kernel instance a convolution launch can run: up to cap keys of three ints (block_n, b_mn, opt); *n = count. */
 int argus_conv_instances_all(int* keys, int cap, int* n);
+/* Plans a weight-gradient launch the way the calls below do and reports, without launching, what it would run.
+ * mode: 0 argus_conv2d_wgrad (k, stride, kind), 1 argus_conv2d_wgrad_gram, 2 argus_conv2d_gram (k and kind ignored
+ * for 1 and 2). ARGUS_WGRAD_INFO_INTS ints go to out: xpose (0 = tile kernel, 1 = transposed all-taps kernel), n
+ * (BLOCK_N, or the padded box count of the transposed kernel), stacked, co_split, num_taps, co tiles, ci tiles,
+ * num_ksplits, kblocks_total (64-pixel k-blocks), grid, scratch elements (floats of split-K scratch). */
+#define ARGUS_WGRAD_INFO_INTS 11
+int argus_conv2d_wgrad_launch_info(int mode, int N, int H, int W, int Cin, int Cout, int k, int stride, int kind,
+                                   int* out, int cap);
+/* While argus_conv_instances_record is on, every weight-gradient launch is recorded as well: get copies up to cap
+ * keys of five ints (xpose, n, stacked, co_split > 0, num_ksplits > 1) and sets *n to the number recorded. */
+int argus_wgrad_instances_get(int* keys, int cap, int* n);
+/* Every weight-gradient kernel instance: up to cap keys of two ints (xpose, n); *n = count. */
+int argus_wgrad_instances_all(int* keys, int cap, int* n);
+/* Fills the first `elems` floats of the scratch buffer the standalone entry points share (growing it as they do) with
+ * the byte byte_value, on stream: tests make stale scratch visible this way (0xff reads as NaN). */
+int argus_lib_scratch_fill(int64_t elems, int byte_value, void* stream);
 /* g[Cin][Cin] (fp32, +=; the caller zero-fills) = x_s^T x_s over the pixels a 1x1 convolution of this shape reads (its
  * even pixels at stride 2): the Gram matrix from which the statistics of the convolution's output follow. */
 int argus_conv2d_gram(const void* x, float* g, int N, int H, int W, int Cin, int Cout, int stride, void* stream);
@@ -132,7 +148,8 @@ int argus_conv_bn_backward_algebraic(const void* g, const void* act, const void*
                                      const float* scale, const float* mean, const float* invstd, float* dgamma,
                                      float* dbeta, float* dw, void* dact, int N, int H, int W, int C, int O, int stride,
                                      void* stream);
-/* dw[Cout][k*k*Cin] (fp32) += dy^T * im2col(x); the caller zero-fills dw. */
+/* dw[Cout][k*k*Cin] (fp32) += dy^T * im2col(x): each element receives its sum with one rounding. kind 1 (stem):
+ * dw[64][256] in the packed [64][p 4][q 4][16] layout of the forward's weight, x the s2d input of argus_conv2d_forward. */
 int argus_conv2d_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int k,
                        int stride, int kind, void* stream);
 /* Input gradient of the stem (resnet.conv1: 7x7, stride 2, pad 3, 3 -> 64; argus/models.py:84).
