@@ -416,6 +416,49 @@ int argus_conv_bn_backward_algebraic(const void* g, const void* act, const void*
   ARGUS_API_END
 }
 
+int argus_bn_alg_backward_small(const void* W, const float* H, const float* G, const float* s, const float* stat_partial,
+                                int slots, int stat_stride, const float* scale, const float* mean, const float* invstd,
+                                double rows, float* dgamma, float* dbeta, float* dW, float* k1k0, void* bstack,
+                                float* bias, float* mpartial, int O, int C, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(O > 0 && C > 0 && O % 256 == 0 && C % 32 == 0, "algebraic BN backward: O % 256 == 0 and C % 32 == 0 required");
+  ARGUS_CHECK(slots > 0 && stat_stride >= O && rows > 0, "algebraic BN backward: bad statistics layout or row count");
+  ARGUS_CHECK(W && H && stat_partial && scale && mean && invstd && dgamma && dbeta && k1k0 && bstack && bias && mpartial &&
+                  (dW == nullptr || (G && s)),
+              "null argument");
+  bn_alg_backward_small(static_cast<const bf16*>(W), H, G, s, stat_partial, slots, stat_stride, scale, mean, invstd, rows,
+                        dgamma, dbeta, dW, k1k0, static_cast<bf16*>(bstack), bias, mpartial, O, C,
+                        static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
+int argus_bn_alg_backward_dw(const void* W, const float* H, const float* G, const float* s, const float* scale,
+                             const float* k1k0, float* dW, int O, int C, void* stream) {
+  ARGUS_API_BEGIN
+  require_sm100();
+  ARGUS_CHECK(O > 0 && C > 0 && O % 256 == 0 && C % 32 == 0, "algebraic BN backward: O % 256 == 0 and C % 32 == 0 required");
+  ARGUS_CHECK(W && H && G && s && scale && k1k0 && dW, "null argument");
+  bn_alg_backward_dw(static_cast<const bf16*>(W), H, G, s, scale, k1k0, dW, O, C, static_cast<cudaStream_t>(stream));
+  ARGUS_API_END
+}
+
+int argus_bn_alg_matrix_scratch_elems(int C, int64_t* elems) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(elems != nullptr && C > 0, "bad argument");
+  *elems = bn_alg_matrix_scratch_elems(C);
+  ARGUS_API_END
+}
+
+int argus_bn_alg_calls_get(int* keys, int cap, int* n) {
+  ARGUS_API_BEGIN
+  ARGUS_CHECK(n != nullptr && (keys != nullptr || cap == 0), "null argument");
+  const auto rec = bn_alg_calls_recorded();
+  *n = static_cast<int>(rec.size());
+  for (int i = 0; i < *n && 5 * (i + 1) <= cap; ++i) std::memcpy(keys + 5 * i, rec[i].data(), 5 * sizeof(int));
+  ARGUS_API_END
+}
+
 int argus_conv2d_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int k,
                        int stride, int kind, void* stream) {
   ARGUS_API_BEGIN

@@ -657,6 +657,7 @@ std::mutex g_record_mu;
 std::atomic<bool> g_recording{false};
 std::set<std::array<int, 5>> g_recorded;
 std::set<std::array<int, 5>> g_recorded_wgrad;
+std::set<std::array<int, 5>> g_recorded_bn_alg;
 }  // namespace
 
 ConvGemmParams epilogue_params(const ConvLaunch& l, const Epilogue& e) {
@@ -737,8 +738,17 @@ ConvLaunchInfo conv_launch_info(const ConvLaunch& l, const Epilogue& e) {
 
 void conv_instances_record(bool on) {
   std::lock_guard<std::mutex> lk(g_record_mu);
-  if (on) { g_recorded.clear(); g_recorded_wgrad.clear(); }
+  if (on) { g_recorded.clear(); g_recorded_wgrad.clear(); g_recorded_bn_alg.clear(); }
   g_recording = on;
+}
+void bn_alg_call_record(int O, int C, int stride, bool dw_aside, bool multi_slot) {
+  if (!g_recording) return;
+  std::lock_guard<std::mutex> lk(g_record_mu);
+  g_recorded_bn_alg.insert({O, C, stride, dw_aside ? 1 : 0, multi_slot ? 1 : 0});
+}
+std::vector<std::array<int, 5>> bn_alg_calls_recorded() {
+  std::lock_guard<std::mutex> lk(g_record_mu);
+  return std::vector<std::array<int, 5>>(g_recorded_bn_alg.begin(), g_recorded_bn_alg.end());
 }
 std::vector<std::array<int, 3>> conv_instances_all() {
   std::vector<std::array<int, 3>> v;

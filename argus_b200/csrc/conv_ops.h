@@ -141,6 +141,10 @@ WgradLaunchInfo wgrad_launch_info(const WgradLaunch& l);
 // While conv_instances_record is on, launch_wgrad adds the key (xpose, n, stacked, co_split > 0, num_ksplits > 1) of
 // every launch to a second host-side set.
 std::vector<std::array<int, 5>> wgrad_instances_recorded();
+// While conv_instances_record is on, Model::conv_bn_backward_algebraic adds the key (O, C, stride, dW on the side stream,
+// more than one statistics slot) of every call to a third host-side set.
+void bn_alg_call_record(int O, int C, int stride, bool dw_aside, bool multi_slot);
+std::vector<std::array<int, 5>> bn_alg_calls_recorded();
 // (xpose, n) of every kernel instance launch_wgrad can dispatch to
 std::vector<std::array<int, 2>> wgrad_instances_all();
 // scratch: at least wgrad_scratch_elems(l) floats (may be null when that is 0)

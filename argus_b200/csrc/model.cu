@@ -901,6 +901,7 @@ void Model::conv_bn_backward_algebraic(const ConvRef& c, const WgradLaunch& hg, 
   // runs on the weight-gradient side stream (joined before H, G, s or k1k0 are overwritten: every algebraic call and
   // every bn_backward joins first)
   const bool dw_aside = overlap_wgrad_;
+  bn_alg_call_record(O, C, c.shape.stride, dw_aside, alg_gstats_slots_ > 1);
   bn_alg_backward_small(packed_ + c.packed_off, alg_h_, saved_gram, colsum, alg_gstats_, alg_gstats_slots_, 2 * O, sc,
                         sc + 2 * O, sc + 3 * O, static_cast<double>(rows), grads_dev_ + c.bn.gamma_off,
                         grads_dev_ + c.bn.beta_off, dw_aside ? nullptr : grads_dev_ + c.w_off, alg_k1k0_, alg_bstack_, alg_bias_,

@@ -148,6 +148,28 @@ int argus_conv_bn_backward_algebraic(const void* g, const void* act, const void*
                                      const float* scale, const float* mean, const float* invstd, float* dgamma,
                                      float* dbeta, float* dw, void* dact, int N, int H, int W, int C, int O, int stride,
                                      void* stream);
+/* The small fp32 kernels of the algebraic backward above, as the model launches them (csrc/bn_algebra.cu). Inputs:
+ * W bf16 [O][C]; H = g^T act [O][C]; G = act^T act [C][C]; s = colsum(act) [C]; stat_partial: `slots` statistics slots,
+ * slot k's column sums of g at stat_partial + k * stat_stride (the dgrad slot layout [slots][2][O] has stride 2 * O);
+ * scale / mean / invstd [O]: the forward's batch-norm constants; rows: pixels of g.
+ * ADDED TO: dgamma [O], dbeta [O] and (when dW is not null) dW [O][C] += diag(scale) H + diag(k1) W G + k0 (x) s.
+ * OVERWRITTEN: k1k0 [2][O] (k1, then k0); bstack bf16 [(O + C)][C] (rows < O: diag(scale) W, rows O + j: row j of
+ * W^T diag(k1) W), the B operand of the K-concatenated dgrad (argus_conv2d_dgrad_ex); bias [C] = k0^T W; mpartial:
+ * argus_bn_alg_matrix_scratch_elems(C) floats of o-split partial sums. O % 256 == 0, C % 32 == 0; G and s may be null
+ * when dW is. */
+int argus_bn_alg_backward_small(const void* W, const float* H, const float* G, const float* s, const float* stat_partial,
+                                int slots, int stat_stride, const float* scale, const float* mean, const float* invstd,
+                                double rows, float* dgamma, float* dbeta, float* dW, float* k1k0, void* bstack,
+                                float* bias, float* mpartial, int O, int C, void* stream);
+/* The dW half alone (argus_bn_alg_backward_small with dW null, then this: the model runs it on the weight-gradient side
+ * stream): dW [O][C] += diag(scale) H + diag(k1) W G + k0 (x) s, from the k1k0 that call wrote. */
+int argus_bn_alg_backward_dw(const void* W, const float* H, const float* G, const float* s, const float* scale,
+                             const float* k1k0, float* dW, int O, int C, void* stream);
+/* *elems = floats of the mpartial scratch argus_bn_alg_backward_small needs for C. */
+int argus_bn_alg_matrix_scratch_elems(int C, int64_t* elems);
+/* While argus_conv_instances_record is on, every algebraic conv + BN backward of a model is recorded as well: get copies
+ * up to cap keys of five ints (O, C, stride, dW on the side stream, more than one statistics slot); *n = count. */
+int argus_bn_alg_calls_get(int* keys, int cap, int* n);
 /* dw[Cout][k*k*Cin] (fp32) += dy^T * im2col(x): each element receives its sum with one rounding. kind 1 (stem):
  * dw[64][256] in the packed [64][p 4][q 4][16] layout of the forward's weight, x the s2d input of argus_conv2d_forward. */
 int argus_conv2d_wgrad(const void* dy, const void* x, float* dw, int N, int H, int W, int Cin, int Cout, int k,
